@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- rollout-steps/s and optimize() latency of the MPPI hot path.
 
-  python bench.py --gpus N --steps K --warmup W [--workload NAME] [--impl reference]
+  python bench.py --gpus N --steps K --warmup W [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one Optimizer::optimize() (nav2_sortham_controller/src/optimizer.cpp:157-164) over one batch of
 synthetic input: iteration_count x {noised rollout, critics, softmax update}.  Protocol = the reference's own
@@ -20,7 +20,7 @@ workloads (BASELINE.json configs):
   robots_256          configs[4]: 256 robots x (2000 x 56), 256/N per rank, one bound group per rank, no exchange.
 
 Without --workload the ONE line printed is the omni_1000x56 line and it carries three nested records measured in the
-same process at the same N: "obstacles_16384x56" and "obstacles_dense_16384x56" (N = 1 only), "sharded_262144x100" and "robots_256", each with
+same process at the same N and with the same --steps / --warmup: "obstacles_16384x56" and "obstacles_dense_16384x56" (N = 1 only), "sharded_262144x100" and "robots_256", each with
 ms_per_step, e2e, per-kernel ms, roofline and a "parity" object produced in the same run (every rank's result against
 the CPU oracle; "MISMATCH" makes the process exit non-zero after the line is printed).
 
@@ -33,6 +33,11 @@ roofline = the bound that binds the dominant kernel: "hbm" (algorithmic bytes / 
          or "issue" (warp instructions of that launch, from the ncu capture recorded in profiles/ncu_kernel_counters.json,
          / duration against the issue-slot peak measured by scripts/peak_microbench.cu, profiles/measured_sm_peaks.json);
          whichever fraction is larger is reported as frac, the other one beside it.
+
+--dump-outputs DIR writes what the caller of the timed path received in its LAST timed step, for every workload of the
+line, as DIR/<workload>.<array>.npy (float32 / float64): the control sequence vx, vy, wz ([T], or [robots, T] for
+robots_256), fail_flag and furthest_reached_path_point (-1: none).  The inputs are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 import argparse
 import json
@@ -53,6 +58,7 @@ METRIC = "rollout_steps_per_sec"
 UNIT = "rollout-steps/s"
 RTOL, ATOL = 1e-4, 1e-6          # north_star's parity bar on the control sequence
 ZERO_COPY_MAX = 96 * 1024        # costmaps above this are handed over in place (registered caller memory)
+DEFAULT_STEPS, DEFAULT_WARMUP = 1000, 20
 
 
 def algorithmic_bytes(B, T, N, cells, iterations=1):
@@ -160,6 +166,21 @@ def pct(a, q):
     return float(np.percentile(np.asarray(a, np.float64), q))
 
 
+def result_outputs(r):
+    """what a caller of optimize() receives (api.Result), as the arrays of --dump-outputs"""
+    f = r.furthest_reached_path_point
+    return {"vx": r.vx, "vy": r.vy, "wz": r.wz, "fail_flag": np.array([float(r.fail_flag)]),
+            "furthest_reached_path_point": np.array([-1.0 if f is None else float(f)])}
+
+
+def dump_outputs(directory, outputs):
+    """--dump-outputs: DIR/<workload>.<array>.npy for every workload of the line"""
+    os.makedirs(directory, exist_ok=True)
+    for workload, arrays in outputs.items():
+        for name, a in arrays.items():
+            np.save(os.path.join(directory, f"{workload}.{name}.npy"), a)
+
+
 # ----------------------------------------------------------------------------------------------------------------
 # CPU side: the reference arm and the cpu_baseline object
 # ----------------------------------------------------------------------------------------------------------------
@@ -211,19 +232,22 @@ def run_reference(args, rank, world):
     sc, noise_kind = pick_scenario(args.workload, 0, 1)
     B, T = sc.cfg["batch_size"], sc.cfg["time_steps"]
     e = oracle_engine(sc, noise_kind)
-    # bound the sample: a step of the big configs takes seconds on one core
+    # without --steps / --warmup the sample is bounded: a step of the big configs takes seconds on one core
     est = B * T * 1.0e-7
-    steps = max(1, min(args.steps, int(60.0 / max(est, 1e-6))))
-    warm = args.warmup if est * args.warmup < 20.0 else max(1, int(20.0 / est))
+    steps = args.steps if args.steps is not None else max(1, min(DEFAULT_STEPS, int(60.0 / max(est, 1e-6))))
+    warm = args.warmup if args.warmup is not None else (DEFAULT_WARMUP if est * DEFAULT_WARMUP < 20.0
+                                                        else max(1, int(20.0 / est)))
     for _ in range(warm):
         e.optimize(sc.cycle)
     lat = []
     t_all = time.perf_counter()
     for _ in range(steps):
         t0 = time.perf_counter()
-        e.optimize(sc.cycle)
+        r = e.optimize(sc.cycle)
         lat.append((time.perf_counter() - t0) * 1e3)
     wall = time.perf_counter() - t_all
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {sc.name: result_outputs(r)})
     iters = sc.cfg.get("iteration_count", 1)
     value = B * T * iters * steps / wall
     line = {
@@ -375,6 +399,7 @@ class Ctx:
         self.torch, self.dist, self.fns = torch, dist, fns
         self.flush = None if args.no_flush else torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
         self.peaks = load_peaks()
+        self.outputs = {}   # workload -> {array name: what the last timed step returned}, for --dump-outputs
 
     def barrier(self):
         self.torch.cuda.synchronize()
@@ -576,6 +601,7 @@ def run_workload(ctx, workload, steps, warmup, with_cpu_baseline, parity=None):
     ctx.barrier()
     region_s = time.perf_counter() - t_region
     launches = e.get_profile()["kernel_launches"] - launches0
+    ctx.outputs[workload] = result_outputs(r)
 
     # ---- leg 2: end to end through mppi_optimize() with host buffers ---------------------------
     # (the ctypes argument struct is marshalled once: the caller's buffers are plain host memory that does not change
@@ -749,6 +775,12 @@ def run_robots(ctx, steps, warmup, with_cpu_baseline, check_parity):
     ctx.barrier()
     region_s = time.perf_counter() - t_region
     launches = sum(e.get_profile()["kernel_launches"] for e in engines) - launches0
+    # copied now: the e2e leg below writes into the same output buffers
+    ctx.outputs["robots_256"] = {
+        **{name: np.stack([arrs[p] for _, arrs in keep]) for p, name in enumerate(("vx", "vy", "wz"))},
+        "fail_flag": np.array([float(bool(o.fail_flag)) for o in outs]),
+        "furthest_reached_path_point": np.array([-1.0 if o.furthest_reached_path_point == abi.UINT32_MAX
+                                                 else float(o.furthest_reached_path_point) for o in outs])}
     for e in engines:
         e.set_timing(False)
     for _ in range(warmup):
@@ -826,8 +858,10 @@ def main():
     _claim_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=1000)
-    ap.add_argument("--warmup", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=None,
+                    help=f"timed steps of every workload (default {DEFAULT_STEPS}; the reference arm: at most about a minute's worth)")
+    ap.add_argument("--warmup", type=int, default=None,
+                    help=f"untimed steps first (default {DEFAULT_WARMUP}, at least 3; the reference arm: at most about 20 s' worth)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default=None)
     ap.add_argument("--no-flush", action="store_true", help="do not flush L2 between timed steps (steady-state number)")
@@ -835,8 +869,13 @@ def main():
     ap.add_argument("--no-nested", action="store_true", help="default line only: skip the nested sharded / robots records")
     ap.add_argument("--exchange", default="peer", choices=["peer", "nccl"],
                     help="sharded workload: exchanges fused into the kernels over peer memory (default) or NCCL collectives")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of every workload returned as DIR/<workload>.<array>.npy")
     args = ap.parse_args()
-    args.warmup = max(args.warmup, 3)
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup is not None:
+        args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -847,6 +886,8 @@ def main():
     if args.impl == "reference":
         run_reference(args, rank, world)
         return
+    args.steps = DEFAULT_STEPS if args.steps is None else args.steps
+    args.warmup = DEFAULT_WARMUP if args.warmup is None else args.warmup
 
     import torch
     import torch.distributed as dist
@@ -871,7 +912,7 @@ def main():
             return {"error": repr(exc)} if rank == 0 else None
 
     if args.workload == "robots_256":
-        line = run_robots(ctx, max(1, min(args.steps, 200)), args.warmup, False, True)
+        line = run_robots(ctx, args.steps, args.warmup, False, True)
     elif args.workload == "sharded_262144x100":
         line = run_workload(ctx, args.workload, args.steps, args.warmup, False, parity=sharded_parity(ctx))
     elif args.workload.startswith("obstacles_"):
@@ -880,13 +921,12 @@ def main():
         line = run_workload(ctx, args.workload, args.steps, args.warmup, False)
     extra = {}
     if nested:
-        n_steps, n_warm = max(1, min(args.steps, 50)), max(3, min(args.warmup, 10))
         if world == 1:
             for wl in ("obstacles_16384x56", "obstacles_dense_16384x56"):
-                extra[wl] = guarded(wl, lambda wl=wl: run_workload(ctx, wl, n_steps, n_warm, False, parity=single_parity(ctx, wl)))
+                extra[wl] = guarded(wl, lambda wl=wl: run_workload(ctx, wl, args.steps, args.warmup, False, parity=single_parity(ctx, wl)))
         extra["sharded_262144x100"] = guarded("sharded_262144x100", lambda: run_workload(
-            ctx, "sharded_262144x100", n_steps, n_warm, False, parity=sharded_parity(ctx)))
-        extra["robots_256"] = guarded("robots_256", lambda: run_robots(ctx, min(n_steps, 30), n_warm, False, True))
+            ctx, "sharded_262144x100", args.steps, args.warmup, False, parity=sharded_parity(ctx)))
+        extra["robots_256"] = guarded("robots_256", lambda: run_robots(ctx, args.steps, args.warmup, False, True))
 
     # the ranks part BEFORE rank 0 starts the CPU baselines: nobody spins in a collective while one host thread works
     if world > 1:
@@ -894,6 +934,8 @@ def main():
         dist.destroy_process_group()
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ctx.outputs)
     for name, rec in extra.items():
         line[name] = rec
         if isinstance(rec, dict) and (rec.get("error") or rec.get("parity", {}).get("status") == "MISMATCH"):

@@ -814,6 +814,7 @@ mppi_status enqueue_uploads(mppi_handle * h)
 // the exact set of features this cycle's record asks of the stream kernel (StreamFeature bits)
 unsigned stream_feature_need(const DevParams & p)
 {
+  if (p.scan_mode != 0) {return SF_ALL;}   // the warp-scan experiment is compiled into the generic instance only
   unsigned need = 0;
   if (p.holonomic) {need |= SF_HOL;}
   if (p.model == MPPI_MODEL_ACKERMANN) {need |= SF_ACKER;}

@@ -479,8 +479,10 @@ __device__ __forceinline__ void rollout_tile_body(
   // ---- P2 (experiment, MPPI_SCAN=warp): the same cumsum as a warp-shuffle inclusive scan ALONG THE HORIZON (lane = time
   //      step, 32 steps per pass, carry between passes), trajectories dealt to the warps.  This is what north_star item (2)
   //      names; it re-associates the fp32 sums, so poses - and with them costmap cells - can differ from the reference's
-  //      sequential order.  Measured and rejected for the parity path (profiles/r02_scan_experiment.json).
-  const bool warp_scan = mode == 0 && p.scan_mode != 0;
+  //      sequential order.  Measured and rejected for the parity path (profiles/r02_scan_experiment.json).  Compiled into
+  //      the generic instance only: the host runs that one while the switch is set (stream_feature_need), so the exact
+  //      instances carry none of its code.
+  const bool warp_scan = !kExact && mode == 0 && p.scan_mode != 0;
   if (warp_scan) {
     const float yaw0 = p.yaw0;
     for (int r = seg; r < kTile && b0 + r < B; r += S) {
@@ -2362,9 +2364,22 @@ __device__ __forceinline__ float path_align_finish(
   return term;
 }
 
+// The two per-warp path critics below are out of line, and they take the shared-memory planes and path tables by value:
+// a FusedCtx passed by reference to a call would pin the whole record in local memory, and the tail would reload its
+// pointers from there (an L1 round trip each, on the default path).
+struct WarpCtx
+{
+  const float * s_x, * s_y, * s_yaw;   // time-major tile planes [T][33]
+  const float * px, * py;              // path points
+  const uint8_t * valid;
+};
+__device__ __forceinline__ WarpCtx warp_ctx(const FusedCtx & fx)
+{
+  return {fx.s_x, fx.s_y, fx.s_yaw, fx.fs.px, fx.fs.py, fx.fs.valid};
+}
+
 // PathAlignLegacyCritic::score (path_align_legacy_critic.cpp:97-128) for trajectory r, by one warp; lane = sampled pose
-__device__ __noinline__ float path_align_legacy_warp(
-  const DevParams * P, const FusedCtx & fx, int r, const float * path_yaw, int lane)
+__device__ __noinline__ float path_align_legacy_warp(const DevParams * P, const WarpCtx fx, int r, const float * path_yaw, int lane)
 {
   const int T = P->T, step = P->legacy_step, segs = P->N - 1;
   float summed = 0.0f;
@@ -2378,8 +2393,8 @@ __device__ __noinline__ float path_align_legacy_warp(
       float min_d = 3.402823466e+38f;
       int min_s = 0;
       for (int sgm = 0; sgm < segs - 1; ++sgm) {
-        const float dx = __fsub_rn(fx.fs.px[sgm], Tx);
-        const float dy = __fsub_rn(fx.fs.py[sgm], Ty);
+        const float dx = __fsub_rn(fx.px[sgm], Tx);
+        const float dy = __fsub_rn(fx.py[sgm], Ty);
         float d = __fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy));
         if (P->legacy_use_yaw) {
           const float dyaw = static_cast<float>(normalize_angle_d(static_cast<double>(Tyaw) - static_cast<double>(path_yaw[sgm])));
@@ -2387,7 +2402,7 @@ __device__ __noinline__ float path_align_legacy_warp(
         }
         if (d < min_d) {min_d = d; min_s = sgm;}
       }
-      if (min_s != 0 && fx.fs.valid[min_s]) {contrib = __fsqrt_rn(min_d);}
+      if (min_s != 0 && fx.valid[min_s]) {contrib = __fsqrt_rn(min_d);}
     }
     summed += warp_sum(contrib);
   }
@@ -2396,10 +2411,10 @@ __device__ __noinline__ float path_align_legacy_warp(
 }
 
 // PathAngleCritic::score (path_angle_critic.cpp:85-100) for trajectory r, by one warp; lane = time step
-__device__ __noinline__ float path_angle_warp(const DevParams * P, const FusedCtx & fx, int r, int angle_idx, int lane)
+__device__ __noinline__ float path_angle_warp(const DevParams * P, const WarpCtx fx, int r, int angle_idx, int lane)
 {
   const int T = P->T;
-  const float gx = fx.fs.px[angle_idx], gy = fx.fs.py[angle_idx];
+  const float gx = fx.px[angle_idx], gy = fx.py[angle_idx];
   float sum = 0.0f;
   for (int t = lane; t < T; t += 32) {
     const int o = t * kPad + r;
@@ -2538,11 +2553,11 @@ __device__ __forceinline__ void tile_fused_body(
   if (dec.legacy_go || dec.angle_go) {
     for (int r = seg; r < rows_here; r += S) {
       if (dec.legacy_go) {
-        const float v = path_align_legacy_warp(P, fx, r, path_yaw, lane);
+        const float v = path_align_legacy_warp(P, warp_ctx(fx), r, path_yaw, lane);
         if (lane == 0) {fs.term[2 * kTile + r] = v;}
       }
       if (dec.angle_go) {
-        const float v = path_angle_warp(P, fx, r, dec.angle_idx, lane);
+        const float v = path_angle_warp(P, warp_ctx(fx), r, dec.angle_idx, lane);
         if (lane == 0) {fs.term[3 * kTile + r] = v;}
       }
     }

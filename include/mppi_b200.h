@@ -221,12 +221,12 @@ mppi_status mppi_get_control_history(mppi_handle * h, float hist12[12]);
 /* batched multi-robot form: n independent handles (possibly on several devices) launched back to back
  * and then joined, so their kernels overlap */
 mppi_status mppi_optimize_batch(mppi_handle ** hs, const mppi_cycle_in * ins, mppi_cycle_out * outs, int32_t n);
-/* Multi-robot server (BASELINE configs[4]): bind n handles of ONE device with the same batch_size / time_steps (tile
- * layout, unsharded, regenerate_noises off) into a group.  The members share the first handle's stream from then on, and
- * mppi_optimize_batch[_resident] over exactly this group, in this order, is ONE kernel launch for all robots (blocks draw
- * tickets, so the robots' tiles need not be co-resident).  Every other call keeps working on a bound handle; a cycle whose
- * members do not all qualify (different critic sets, evalControl tail, ...) runs them one by one.  Destroying a member
- * dissolves the group. */
+/* Multi-robot server (BASELINE configs[4]): bind n handles of ONE device with the same batch_size / time_steps
+ * (unsharded, regenerate_noises off) into a group.  The members move to the stream layout and share the first handle's
+ * stream from then on, and mppi_optimize_batch[_resident] over exactly this group, in this order, runs in chunks of up to
+ * 64 robots: each chunk is one strided upload plus four kernel launches.  Every other call keeps working on a bound
+ * handle; a cycle whose members do not all qualify (evalControl tail, iteration_count > 1, profiling, ...) runs them one
+ * by one.  Destroying a member dissolves the group. */
 mppi_status mppi_batch_bind(mppi_handle ** handles, int32_t n);
 mppi_status mppi_batch_unbind(mppi_handle * any_member);
 /* The same over inputs already resident on the device (mppi_upload_cycle on every handle).  Measurement hook. */

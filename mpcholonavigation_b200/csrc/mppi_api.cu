@@ -100,9 +100,6 @@ struct mppi_handle
   float * d_partials{nullptr};
   unsigned * d_ws_done{nullptr};         // per row group of the weighted-sums kernel: blocks finished (last one merges)
   CUtensorMap noise_map[3];           // TMA descriptors of the time-major noise planes (stream layout, weighted_sums_tma_kernel)
-  bool pdl_enabled{true};             // MPPI_PDL=0: ordinary (fully serialised) launches of the stream layout's post-rollout kernels
-  int scan_mode{0};                   // MPPI_SCAN=warp: experiment, warp-shuffle prefix scans in the tile kernels (not the parity path)
-  bool ws_tma_enabled{true};             // MPPI_WS_TMA=0: the register-staged weighted-sums kernel (always used when B % 4 != 0)
   bool ws_tma_ok{false};                 // the TMA-fed weighted-sums kernel can run (B % 4 == 0, descriptors made)
   float * d_rank_partial{nullptr};
   float * d_gathered{nullptr};
@@ -123,8 +120,6 @@ struct mppi_handle
   bool cycle_uploaded{false};
   bool spilled_traj{false}, spilled_cells{false}, have_rows{false};
   DevParams last;   // host copy of the last uploaded record
-  int segments_override{0};
-  int stream_threads_override{0};
   // fused small-batch kernel: packet buffers of the in-GPU exchanges, launch epoch (device + host mirror), result packets
   uint2 * d_pk{nullptr};                  // [G] exchange-1 packets, then [G][3T + 2] record packets
   unsigned * d_fepoch{nullptr};           // completed fused launches (never reset: tags do not repeat)
@@ -132,25 +127,22 @@ struct mppi_handle
   uint2 * h_res{nullptr};                 // pinned + mapped: [3T + 8] result packets written by the kernels
   bool zero_copy_now{false};              // this cycle's fused kernel pulls the upload out of pinned host memory itself
   bool wait_packets{false};               // the cycle in flight delivers its result as packets (no D2H copy, no stream sync)
-  // multi-robot batch (mppi_batch_bind): the bound handles share the leader's stream, so that ONE launch can serve all
-  // of them (tile_fused_batch_kernel) and every later operation on any of them is still ordered behind it
+  // multi-robot batch (mppi_batch_bind): the bound handles share the leader's stream, so that the group's four launches
+  // serve all of them and every later operation on any of them is still ordered behind them
   mppi_handle * batch_leader{nullptr};    // non-null for every bound handle (the leader points to itself)
   cudaStream_t own_stream{nullptr};       // a follower's own stream while it borrows the leader's
   mppi_handle * ev_src{nullptr};          // whose ev0 / ev1 bracket the cycle in flight (the leader's after a batched launch)
   std::vector<mppi_handle *> batch_group; // leader only, in bind order
-  cudaStream_t copy_stream{nullptr};      // leader only (stream-layout group): the chunk uploads ride here, beside the previous chunk's kernels
+  cudaStream_t copy_stream{nullptr};      // leader only: the chunk uploads ride here, beside the previous chunk's kernels
   cudaEvent_t ev_upload[8]{};             // leader only: upload of chunk c done (c modulo 8)
   FusedJob * h_jobs{nullptr};             // leader only: job table, pinned ...
   FusedJob * d_jobs{nullptr};             // ... and its device copy (re-sent only when an entry changes)
   std::vector<char> jobs_sent;            // what the device copy holds
-  unsigned * d_ticket{nullptr};           // leader only: ticket counter of the batch kernel (never reset)
-  uint32_t ticket_base{0};                // tickets drawn by all earlier batched launches
-  int batch_mode{0};                      // leader: 1 = tile layout, ticketed fused kernel; 2 = stream layout, four batched kernels
-  char * arena_h{nullptr};                // leader, mode 2: the [record | costmap] buffers of all members, one slice each,
+  char * arena_h{nullptr};                // leader: the [record | costmap] buffers of all members, one slice each,
   char * arena_d{nullptr};                //   so that the whole group uploads with ONE strided copy
   size_t arena_slice{0};
   bool params_in_arena{false};            // member: h_params / d_params point into the leader's arena
-  uint32_t batch_tag{0};                  // leader, mode 2: counter behind the tag of the group's result packets
+  uint32_t batch_tag{0};                  // leader: counter behind the tag of the group's result packets
   uint32_t result_tag{0};                 // tag the cycle in flight delivers its result packets with
   // caller memory registered as pinned (mppi_register_costmap_memory): a costmap inside such a range is copied to the
   // device straight from the caller's buffer, without the staging memcpy
@@ -158,8 +150,6 @@ struct mppi_handle
   const uint8_t * costmap_direct{nullptr};   // this cycle's costmap source when it is copied directly
   uint64_t host_ns[8]{0, 0, 0, 0, 0, 0, 0, 0};   // host-side time of the steady-state call by phase (mppi_debug_get_host_ns)
   bool zero_copy_enabled{true};   // MPPI_ZERO_COPY=0 disables
-  bool coop_launch{true};
-  bool packets_enabled{true};     // MPPI_STREAM_PACKETS=0: the stream layout copies its result back and synchronises
   bool fused_enabled{true};    // small batches: one cooperative launch per iteration (tile_fused_kernel); MPPI_FUSED=0 disables
   int fused_key_N{-1};         // path size the cached decision below was taken for (the shared-memory size depends on it)
   bool fused_fits{false};      // the whole grid is co-resident (a cooperative launch needs that)
@@ -174,6 +164,7 @@ struct mppi_handle
   size_t gkey_params[12]{}, gkey_costmap[12]{};
   unsigned gkey_inst[12]{};
   int gkey_fused[12]{};   // fused kernel: shared-memory key (path capacity, PathAlign samples); -1 = two-kernel path
+  uint64_t glaunches[12]{};   // kernel launches in the captured graph (counted while it was captured)
   int tail_mode{0};            // 0: optimize only, 1: + evalControl tail, 2: + tail with shiftControlSequence
   // peer-memory exchange (one process per GPU; mppi_comm_get_mailbox_handle / mppi_comm_connect_peers)
   uint2 * d_mailbox{nullptr};             // this rank's mailbox (kBoxPackets packets)
@@ -649,7 +640,6 @@ mppi_status build_params(mppi_handle * h, const mppi_cycle_in * in, int mode, un
   }
   p.spill_traj = ((h->want_mask & MPPI_WANT_TRAJECTORIES) || any_gate_open || mode == 1) ? 1 : 0;
   p.noise_tm = (h->stream_layout && mode == 0) ? 1 : 0;
-  p.scan_mode = h->scan_mode;
   p.need_furthest = (p.follow.idx >= 0 || p.angle.idx >= 0 || p.align.idx >= 0 || p.legacy.idx >= 0) ? 1 : 0;
   h->last = p;
   return MPPI_OK;
@@ -665,7 +655,6 @@ int weighted_sums_row_groups(int T, int chunks)
 
 int pick_segments(const mppi_handle * h)
 {
-  if (h->segments_override > 0) {return h->segments_override;}
   const int tiles = (h->B + kTile - 1) / kTile;
   int S = 8;
   if (tiles > 148 * 4) {S = 4;}
@@ -733,8 +722,6 @@ DevBuffers make_bufs(mppi_handle * h, int mode)
   b.epoch = h->d_fepoch;
   // sticky "a bounded poll gave up" word in pinned host memory, behind the result packets (raise_comm_error)
   b.host_err = h->h_res ? reinterpret_cast<unsigned *>(h->h_res + 3 * static_cast<size_t>(h->T) + 9) : nullptr;
-  static const int k3_fast = std::getenv("MPPI_K3_FAST") ? std::atoi(std::getenv("MPPI_K3_FAST")) : 1;   // measurement switch
-  b.k3_fast = k3_fast;
   return b;
 }
 
@@ -814,7 +801,6 @@ mppi_status enqueue_uploads(mppi_handle * h)
 // the exact set of features this cycle's record asks of the stream kernel (StreamFeature bits)
 unsigned stream_feature_need(const DevParams & p)
 {
-  if (p.scan_mode != 0) {return SF_ALL;}   // the warp-scan experiment is compiled into the generic instance only
   unsigned need = 0;
   if (p.holonomic) {need |= SF_HOL;}
   if (p.model == MPPI_MODEL_ACKERMANN) {need |= SF_ACKER;}
@@ -846,7 +832,6 @@ unsigned pick_stream_instance(unsigned need)
 
 int stream_block_threads(const mppi_handle * h)
 {
-  if (h->stream_threads_override > 0) {return h->stream_threads_override;}
   // fewer threads per block below ~4 full blocks per SM: same number of warps, spread evenly over the 148 SMs
   return h->B >= 148 * 4 * kStreamThreads ? kStreamThreads : 64;
 }
@@ -874,7 +859,7 @@ cudaError_t fused_occupancy(int threads, size_t smem, int * blocks_per_sm)
 // tagged with the epoch the path-cost kernel advanced (no D2H copy node, no stream synchronisation).
 bool stream_packets(const mppi_handle * h)
 {
-  return h->stream_layout && h->nranks == 1 && h->tail_mode == 0 && h->d_fepoch != nullptr && h->packets_enabled;
+  return h->stream_layout && h->nranks == 1 && h->tail_mode == 0 && h->d_fepoch != nullptr;
 }
 
 // path capacity of the fused kernel's shared memory: rounded up to 64 points like the record copy (build_params), so that
@@ -929,9 +914,6 @@ cudaError_t launch_fused_instance(mppi_handle * h, int iteration, uint2 * host_r
   int up_vecs = zero_copy ? static_cast<int>((upload_bytes(h) + 15) / 16) : 0;
   float * hist = h->d_hist;
   void * args[] = {&dp, &cm, &bufs, &B, &T, &N, &iteration, &host_res, &up_host, &up_vecs, &tail_mode, &hist};
-  if (!h->coop_launch) {   // experiment switch (MPPI_COOP=0): plain launch, no co-residency guarantee
-    return cudaLaunchKernel(reinterpret_cast<const void *>(&tile_fused_kernel<F, kExact>), grid, block, args, smem, h->stream);
-  }
   return cudaLaunchCooperativeKernel(reinterpret_cast<const void *>(&tile_fused_kernel<F, kExact>), grid, block, args, smem, h->stream);
 }
 
@@ -1016,8 +998,7 @@ int weighted_sums_chunks(const mppi_handle * h)
 // step at 2 GPUs - the exposed part is the last row group's merge plus the rank skew either way - and left out.
 bool merge_in_weighted_sums(const mppi_handle * h)
 {
-  static const int enabled = std::getenv("MPPI_WS_MERGE") ? std::atoi(std::getenv("MPPI_WS_MERGE")) : 1;   // measurement switch
-  return enabled && h->stream_layout && h->ws_tma_ok && h->nranks == 1 && h->cfg.motion_model != MPPI_MODEL_ACKERMANN && h->d_ws_done;
+  return h->stream_layout && h->ws_tma_ok && h->nranks == 1 && h->cfg.motion_model != MPPI_MODEL_ACKERMANN && h->d_ws_done;
 }
 
 // host_res: the result leaves as packets (only looked at when the kernel merges itself)
@@ -1032,12 +1013,12 @@ mppi_status launch_weighted_sums(mppi_handle * h, uint2 * host_res = nullptr, bo
     const int stages = (holonomic(h) ? 3 : 2) * ((h->T + kPsRows - 1) / kPsRows);
     const int target = (5 * h->num_sms) / 2;
     const int gy = std::max(1, std::min(stages / 2, std::max(4, (target + chunks - 1) / chunks)));
-    CUDA_TRY(h, launch_kernel(weighted_sums_tma_kernel, dim3(chunks, gy), dim3(kPsThreads), ps_smem_bytes(), h->stream, h->pdl_enabled,
+    CUDA_TRY(h, launch_kernel(weighted_sums_tma_kernel, dim3(chunks, gy), dim3(kPsThreads), ps_smem_bytes(), h->stream, true,
       h->noise_map[0], h->noise_map[1], h->noise_map[2], dp, make_bufs(h, 0), h->T, h->B, holonomic(h) ? 1 : 0,
       (allow_merge && merge_in_weighted_sums(h)) ? h->d_ws_done : nullptr, host_res));
   } else {
     const int gy = weighted_sums_row_groups(h->T, chunks);
-    CUDA_TRY(h, launch_kernel(weighted_sums_tm_kernel, dim3(chunks, gy), dim3(kWsThreads), 0, h->stream, h->pdl_enabled, dp, make_bufs(h, 0)));
+    CUDA_TRY(h, launch_kernel(weighted_sums_tm_kernel, dim3(chunks, gy), dim3(kWsThreads), 0, h->stream, true, dp, make_bufs(h, 0)));
   }
   CUDA_TRY(h, cudaGetLastError());
   h->launches++;
@@ -1052,16 +1033,9 @@ mppi_status launch_update(mppi_handle * h, int mode, int iteration)
     // the iteration that completes the result advances the packet epoch when the result leaves as packets
     const int bump = (stream_packets(h) && iteration + 1 == h->cfg.iteration_count) ? 1 : 0;
     // programmatic dependent launch behind the rollout kernel (not behind an NCCL all-reduce: that is a library launch)
-    const bool pdl = h->pdl_enabled && !(h->nranks > 1 && !h->peer_mode);
+    const bool pdl = !(h->nranks > 1 && !h->peer_mode);
     const DevParams * dp = reinterpret_cast<const DevParams *>(h->d_params);
-    static const int k3a_blocks = std::getenv("MPPI_K3A_BLOCKS") ? std::atoi(std::getenv("MPPI_K3A_BLOCKS")) : 0;   // experiment
-    if (k3a_blocks == 6) {
-      CUDA_TRY(h, launch_kernel(path_costs_tm_kernel<6>, dim3(std::min(grid, 148 * 6)), dim3(kUpdThreads), k3_common_smem_bytes(), h->stream, pdl,
-        dp, make_bufs(h, mode), iteration, bump));
-    } else if (k3a_blocks == 4) {
-      CUDA_TRY(h, launch_kernel(path_costs_tm_kernel<4>, dim3(std::min(grid, 148 * 4)), dim3(kUpdThreads), k3_common_smem_bytes(), h->stream, pdl,
-        dp, make_bufs(h, mode), iteration, bump));
-    } else if (h->B >= 131072 && k3a_blocks != 5) {
+    if (h->B >= 131072) {
       CUDA_TRY(h, launch_kernel(path_costs_tm_kernel<8>, dim3(grid), dim3(kUpdThreads), k3_common_smem_bytes(), h->stream, pdl,
         dp, make_bufs(h, mode), iteration, bump));
     } else {
@@ -1126,7 +1100,7 @@ mppi_status enqueue_kernels(mppi_handle * h, bool prof)
       if (prof) {CUDA_TRY(h, cudaEventRecord(h->pev[2], h->stream));}
       const bool merged_in_k3 = !h->stream_layout && !many;   // K3's last block already merged into rank_partial
       CUDA_TRY(h, launch_kernel(merge_exchange_finalize_kernel, dim3(merge_grid), dim3(kUpdThreads), 0, h->stream,
-        h->pdl_enabled && h->stream_layout, dp, merged_in_k3 ? h->d_rank_partial : h->d_partials,
+        h->stream_layout, dp, merged_in_k3 ? h->d_rank_partial : h->d_partials,
         merged_in_k3 ? 1 : (h->stream_layout ? chunks : h->upd_blocks), stride, make_bufs(h, 0)));
       CUDA_TRY(h, cudaGetLastError());
       h->launches++;
@@ -1135,7 +1109,7 @@ mppi_status enqueue_kernels(mppi_handle * h, bool prof)
         // nothing to launch: the weighted-sums kernel's last block per row group merged, clipped and delivered
       } else if (h->stream_layout || many) {
         // too many partial records for a serial merge in K3's last block (or the stream layout): merge in parallel
-        CUDA_TRY(h, launch_kernel(merge_finalize_kernel, dim3(merge_grid), dim3(kUpdThreads), 0, h->stream, h->pdl_enabled && h->stream_layout,
+        CUDA_TRY(h, launch_kernel(merge_finalize_kernel, dim3(merge_grid), dim3(kUpdThreads), 0, h->stream, h->stream_layout,
           dp, h->d_partials, h->stream_layout ? chunks : h->upd_blocks, stride, make_bufs(h, 0), h->nranks > 1 ? 0 : 1, h->d_rank_partial,
           (stream_packets(h) && it + 1 == h->cfg.iteration_count) ? h->h_res : nullptr));
         CUDA_TRY(h, cudaGetLastError());
@@ -1258,7 +1232,8 @@ mppi_status enqueue_optimize_impl(mppi_handle * h, bool with_upload)
       if (s == MPPI_OK && h->timing && cudaEventRecordWithFlags(h->ev1, h->stream, cudaEventRecordExternal) != cudaSuccess) {s = MPPI_E_CUDA;}
       h->capturing = false;
       const cudaError_t ce = cudaStreamEndCapture(h->stream, &graph);
-      h->launches = launches_before;   // capture launched nothing
+      h->glaunches[slot] = h->launches - launches_before;
+      h->launches = launches_before;   // capture launched nothing: the graph's launches count when it is replayed
       if (s != MPPI_OK || ce != cudaSuccess || !graph) {
         if (graph) {cudaGraphDestroy(graph);}
         cudaGetLastError();
@@ -1277,8 +1252,7 @@ mppi_status enqueue_optimize_impl(mppi_handle * h, bool with_upload)
       CUDA_TRY(h, cudaGraphLaunch(h->gexec[slot], h->stream));
       const uint64_t t_c = now_ns();
       h->host_ns[3] += t_c - t_b;
-      h->launches += (use_fused(h) ? 1ull : (h->stream_layout ? 4ull : (h->upd_blocks > kLastBlockMergeMax ? 3ull : 2ull))) *
-        h->cfg.iteration_count + (h->tail_mode && !use_fused(h) ? 1ull : 0ull);
+      h->launches += h->glaunches[slot];
       h->host_ns[4] += now_ns() - t_c;
       return MPPI_OK;
     }
@@ -1515,13 +1489,10 @@ void batch_unbind_group(mppi_handle * leader)
   if (leader->arena_h) {cudaFreeHost(leader->arena_h); leader->arena_h = nullptr;}
   if (leader->arena_d) {cudaFree(leader->arena_d); leader->arena_d = nullptr;}
   leader->arena_slice = 0;
-  leader->batch_mode = 0;
   leader->batch_group.clear();
   leader->jobs_sent.clear();
   if (leader->h_jobs) {cudaFreeHost(leader->h_jobs); leader->h_jobs = nullptr;}
   if (leader->d_jobs) {cudaFree(leader->d_jobs); leader->d_jobs = nullptr;}
-  if (leader->d_ticket) {cudaFree(leader->d_ticket); leader->d_ticket = nullptr;}
-  leader->ticket_base = 0;
 }
 
 // is hs[0..n) exactly a bound group, in bind order?
@@ -1534,91 +1505,7 @@ bool batch_is_group(mppi_handle ** hs, int n)
   return true;
 }
 
-constexpr int kBatchChunk = 16;   // robots per launch: the host prepares the next chunk's records while this one runs
-
-template<unsigned F, bool kExact>
-cudaError_t launch_batch_instance(mppi_handle * leader, int c0, int n, int G, dim3 block, size_t smem)
-{
-  tile_fused_batch_kernel<F, kExact><<<dim3(static_cast<unsigned>(n) * G), block, smem, leader->stream>>>(
-    leader->d_jobs + c0, G, leader->d_ticket, leader->ticket_base);
-  return cudaGetLastError();
-}
-
-// One launch for the members [c0, c0 + n) of a bound group (their records are built, uploads staged).  Returns
-// MPPI_E_STATE without having launched anything when they do not qualify this cycle: the caller then runs them one by
-// one (they share a stream, so that is correct, only slower).  `first` / `last`: this is the first / last chunk of the
-// call (the leader's events bracket the whole call).
-mppi_status batch_launch(mppi_handle * L, mppi_handle ** hs, int c0, int n, bool with_upload, bool first, bool last)
-{
-  // the exact instance when every member asks for the same one, else the generic instance (it tests the per-cycle flags)
-  unsigned inst = pick_stream_instance(stream_feature_need(hs[0]->last));
-  for (int i = 1; i < n; ++i) {
-    if (pick_stream_instance(stream_feature_need(hs[i]->last)) != inst) {inst = SF_ALL; break;}
-  }
-  const int S = pick_segments(L);
-  const int G = (L->B + kTile - 1) / kTile;
-  const int n_cap = fused_path_capacity(hs[0]), n_s = fused_align_samples(hs[0]);
-  for (int i = 0; i < n; ++i) {
-    mppi_handle * h = hs[i];
-    const char * why = nullptr;
-    if (!use_fused(h)) {why = "fused kernel not applicable";}
-    else if (h->tail_mode != 0 || h->cfg.iteration_count != 1 || h->profiling) {why = "tail / iteration_count / profiling";}
-    else if (fused_path_capacity(h) != n_cap || fused_align_samples(h) != n_s) {why = "different path capacity / PathAlign samples";}
-    if (why) {
-      L->err = std::string("batched launch not used: member ") + std::to_string(c0 + i) + ": " + why;
-      return MPPI_E_STATE;
-    }
-  }
-  const size_t smem = fused_smem_bytes(L->T, S, n_cap, G, n_s);
-  for (int i = 0; i < n; ++i) {
-    mppi_handle * h = hs[i];
-    h->wait_packets = true;
-    h->ev_src = L;
-    h->zero_copy_now = with_upload && h->zero_copy_enabled && upload_bytes(h) <= kZeroCopyMaxBytes;
-    if (with_upload && !h->zero_copy_now) {
-      const mppi_status us = enqueue_uploads(h);
-      if (us != MPPI_OK) {return us;}
-    }
-    FusedJob & j = L->h_jobs[c0 + i];
-    std::memset(&j, 0, sizeof(j));
-    j.Pg = reinterpret_cast<const DevParams *>(h->d_params);
-    j.cm = h->d_costmap;
-    j.bufs = make_bufs(h, 0);
-    j.B = h->B; j.T = h->T; j.n_cap = n_cap; j.iteration = 0;
-    j.host_res = h->h_res;
-    j.up_host = h->zero_copy_now ? reinterpret_cast<const uint4 *>(h->h_params) : nullptr;
-    j.up_vecs = h->zero_copy_now ? static_cast<int>((upload_bytes(h) + 15) / 16) : 0;
-  }
-  // the device copy of the job table is re-sent only where it changed (pointers and sizes are the same every cycle)
-  const size_t off = sizeof(FusedJob) * static_cast<size_t>(c0), bytes = sizeof(FusedJob) * static_cast<size_t>(n);
-  if (std::memcmp(L->jobs_sent.data() + off, L->h_jobs + c0, bytes) != 0) {
-    CUDA_TRY(L, cudaMemcpyAsync(L->d_jobs + c0, L->h_jobs + c0, bytes, cudaMemcpyHostToDevice, L->stream));
-    std::memcpy(L->jobs_sent.data() + off, L->h_jobs + c0, bytes);
-  }
-  if (first && L->timing) {CUDA_TRY(L, cudaEventRecord(L->ev0, L->stream));}
-  const dim3 block(kTile, S);
-  cudaError_t e;
-  switch (inst) {
-    case kSfOmniDefault: e = launch_batch_instance<kSfOmniDefault, true>(L, c0, n, G, block, smem); break;
-    case kSfOmniDefaultFp: e = launch_batch_instance<kSfOmniDefaultFp, true>(L, c0, n, G, block, smem); break;
-    case kSfObstaclesFp: e = launch_batch_instance<kSfObstaclesFp, true>(L, c0, n, G, block, smem); break;
-    default: e = launch_batch_instance<SF_ALL, false>(L, c0, n, G, block, smem); break;
-  }
-  CUDA_TRY(L, e);
-  if (last && L->timing) {CUDA_TRY(L, cudaEventRecord(L->ev1, L->stream));}
-  L->ticket_base += static_cast<uint32_t>(n) * static_cast<uint32_t>(G);
-  L->launches++;
-  for (int i = 0; i < n; ++i) {
-    mppi_handle * h = hs[i];
-    h->fepoch_host += 1u;
-    h->result_tag = h->fepoch_host;
-    h->d2h_bytes = sizeof(uint2) * (3 * h->T + 2);
-    h->h2d_bytes = with_upload ? upload_bytes(h) + (h->zero_copy_now ? static_cast<size_t>(h->upd_blocks) * kHotBytes : 0) : 0;
-  }
-  return MPPI_OK;
-}
-
-// ---- mode 2: the group in the stream layout, four batched kernels for all robots -------------------------------
+// ---- the group in the stream layout, four batched kernels for all robots ---------------------------------------
 // [B][T] -> [T][B] for the three noise planes of a handle that was created in the tile layout
 mppi_status to_stream_layout(mppi_handle * h)
 {
@@ -1696,7 +1583,6 @@ mppi_status batch_stream_launch(mppi_handle * L, mppi_handle ** hs, int c0, int 
     j.Pg = reinterpret_cast<const DevParams *>(h->d_params);
     j.cm = h->d_costmap;
     j.bufs = make_bufs(h, 0);
-    j.B = h->B; j.T = h->T;
     j.host_res = h->h_res;
     h->wait_packets = true;
     h->zero_copy_now = false;
@@ -1746,46 +1632,15 @@ mppi_status batch_stream_launch(mppi_handle * L, mppi_handle ** hs, int c0, int 
   return MPPI_OK;
 }
 
-// The whole group, in chunks of kBatchChunk robots: records of a chunk are built (ins != nullptr) and the chunk is
-// launched while the device still works on the previous ones.  Members of a chunk that does not qualify run one by one.
+// The whole group, in chunks of kStreamBatchChunk robots: the records of a chunk are built (ins != nullptr), then the
+// chunk is uploaded with one strided copy and launched (four kernels) while the host builds the next chunk.  When a member
+// does not qualify this cycle, the members run one by one on the shared stream.
 mppi_status batch_run_group(mppi_handle ** hs, const mppi_cycle_in * ins, mppi_cycle_out * outs, int n)
 {
   mppi_handle * L = hs[0];
   CUDA_TRY(L, cudaSetDevice(L->device));
   mppi_status first = MPPI_OK;
-  std::vector<char> pending(n, 0);
-  if (L->batch_mode == 2) {
-    // stream-layout group, in chunks: the records of a chunk are built, then the chunk is uploaded with one strided copy
-    // and launched (four kernels) while the host builds the next chunk
-    if (batch_stream_ok(hs, n)) {
-      const uint32_t tag = 0x80000000u | (++L->batch_tag);   // never a tag of the fused kernel's epochs
-      const int chunk = ins ? kStreamBatchChunk : n;
-      for (int c0 = 0; c0 < n; c0 += chunk) {
-        const int cn = std::min(chunk, n - c0);
-        mppi_status s = MPPI_OK;
-        for (int i = c0; i < c0 + cn && s == MPPI_OK; ++i) {
-          if (ins) {
-            s = build_params(hs[i], &ins[i], 0, kUnset, true);
-            if (s == MPPI_OK) {s = stage_costmap(hs[i], ins[i].costmap);}
-            if (s == MPPI_OK) {hs[i]->cycle_uploaded = true;}
-          } else if (!hs[i]->cycle_uploaded) {
-            s = fail(hs[i], MPPI_E_STATE, "mppi_optimize_batch_resident before mppi_upload_cycle");
-          }
-        }
-        if (s == MPPI_OK) {s = batch_stream_launch(L, hs + c0, c0, cn, ins != nullptr, tag, c0 == 0, c0 + cn == n);}
-        if (s == MPPI_OK) {
-          for (int i = c0; i < c0 + cn; ++i) {pending[i] = 1;}
-        } else if (first == MPPI_OK) {
-          first = s;
-        }
-      }
-      for (int i = 0; i < n; ++i) {
-        if (!pending[i]) {continue;}
-        const mppi_status f = finish_optimize(hs[i], outs ? &outs[i] : nullptr);
-        if (f != MPPI_OK && first == MPPI_OK) {first = f;}
-      }
-      return first;
-    }
+  if (!batch_stream_ok(hs, n)) {
     if (L->timing) {cudaEventRecord(L->ev0, L->stream);}
     for (int i = 0; i < n; ++i) {   // one by one on the shared stream
       mppi_status f = MPPI_OK;
@@ -1802,8 +1657,9 @@ mppi_status batch_run_group(mppi_handle ** hs, const mppi_cycle_in * ins, mppi_c
     }
     return first;
   }
-  // resident inputs: nothing to prepare on the host, one launch for the whole group
-  const int chunk = ins ? kBatchChunk : n;
+  std::vector<char> pending(n, 0);
+  const uint32_t tag = 0x80000000u | (++L->batch_tag);   // never a tag of the fused kernel's epochs
+  const int chunk = ins ? kStreamBatchChunk : n;
   for (int c0 = 0; c0 < n; c0 += chunk) {
     const int cn = std::min(chunk, n - c0);
     mppi_status s = MPPI_OK;
@@ -1816,17 +1672,9 @@ mppi_status batch_run_group(mppi_handle ** hs, const mppi_cycle_in * ins, mppi_c
         s = fail(hs[i], MPPI_E_STATE, "mppi_optimize_batch_resident before mppi_upload_cycle");
       }
     }
-    if (s == MPPI_OK) {s = batch_launch(L, hs + c0, c0, cn, ins != nullptr, c0 == 0, c0 + cn == n);}
+    if (s == MPPI_OK) {s = batch_stream_launch(L, hs + c0, c0, cn, ins != nullptr, tag, c0 == 0, c0 + cn == n);}
     if (s == MPPI_OK) {
       for (int i = c0; i < c0 + cn; ++i) {pending[i] = 1;}
-    } else if (s == MPPI_E_STATE) {
-      // this chunk does not qualify: one by one on the shared stream (records are built already)
-      if (c0 == 0 && L->timing) {cudaEventRecord(L->ev0, L->stream);}
-      for (int i = c0; i < c0 + cn; ++i) {
-        mppi_status f = hs[i]->cycle_uploaded ? enqueue_optimize(hs[i], ins != nullptr) : MPPI_E_STATE;
-        if (f == MPPI_OK) {pending[i] = 1;} else if (first == MPPI_OK) {first = f;}
-      }
-      if (c0 + cn == n && L->timing) {cudaEventRecord(L->ev1, L->stream);}
     } else if (first == MPPI_OK) {
       first = s;
     }
@@ -1951,18 +1799,10 @@ mppi_status mppi_create(const mppi_config * cfg, mppi_handle ** out)
   h->base = {cfg->vx_max, cfg->vx_min, cfg->vy_max, cfg->wz_max};
   h->cur = h->base;
   std::memset(&h->robot, 0, sizeof(h->robot));
-  if (const char * e = std::getenv("MPPI_SEGMENTS")) {h->segments_override = std::atoi(e);}
-  if (const char * e = std::getenv("MPPI_STREAM_THREADS")) {
-    h->stream_threads_override = std::max(32, std::min(kStreamThreads, (std::atoi(e) / 32) * 32));
-  }
-  if (const char * e = std::getenv("MPPI_NO_GRAPH")) {h->use_graph = std::atoi(e) == 0;}
+  // test hooks: each forces a path the library also picks by itself for other inputs (the two-kernel tile path, the
+  // copy-engine upload, the stream layout), so that tests can compare the paths on the same input
   if (const char * e = std::getenv("MPPI_FUSED")) {h->fused_enabled = std::atoi(e) != 0;}
   if (const char * e = std::getenv("MPPI_ZERO_COPY")) {h->zero_copy_enabled = std::atoi(e) != 0;}
-  if (const char * e = std::getenv("MPPI_COOP")) {h->coop_launch = std::atoi(e) != 0;}
-  if (const char * e = std::getenv("MPPI_STREAM_PACKETS")) {h->packets_enabled = std::atoi(e) != 0;}
-  if (const char * e = std::getenv("MPPI_PDL")) {h->pdl_enabled = std::atoi(e) != 0;}
-  if (const char * e = std::getenv("MPPI_SCAN")) {h->scan_mode = std::strcmp(e, "warp") == 0 ? 1 : 0;}
-  if (const char * e = std::getenv("MPPI_WS_TMA")) {h->ws_tma_enabled = std::atoi(e) != 0;}
   {
     // batches too small to fill the GPU with one thread per trajectory keep the latency-oriented tile kernel
     long long stream_min = 8192;    // measured cross-over on B200 (profiles/): below it the tile kernel wins
@@ -1990,10 +1830,6 @@ mppi_status mppi_create(const mppi_config * cfg, mppi_handle ** out)
     CUDA_TRY(h, cudaFuncSetAttribute(tile_fused_kernel<kSfOmniDefault, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
     CUDA_TRY(h, cudaFuncSetAttribute(tile_fused_kernel<kSfOmniDefaultFp, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
     CUDA_TRY(h, cudaFuncSetAttribute(tile_fused_kernel<kSfObstaclesFp, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CUDA_TRY(h, cudaFuncSetAttribute(tile_fused_batch_kernel<SF_ALL, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CUDA_TRY(h, cudaFuncSetAttribute(tile_fused_batch_kernel<kSfOmniDefault, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CUDA_TRY(h, cudaFuncSetAttribute(tile_fused_batch_kernel<kSfOmniDefaultFp, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CUDA_TRY(h, cudaFuncSetAttribute(tile_fused_batch_kernel<kSfObstaclesFp, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
     int coop = 0;
     CUDA_TRY(h, cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, h->device));
     CUDA_TRY(h, cudaDeviceGetAttribute(&h->num_sms, cudaDevAttrMultiProcessorCount, h->device));
@@ -2019,7 +1855,7 @@ mppi_status mppi_create(const mppi_config * cfg, mppi_handle ** out)
     CUDA_TRY(h, cudaMalloc(&h->d_spill[i], plane));
     CUDA_TRY(h, cudaMemsetAsync(h->d_noise[i], 0, noise_plane, h->stream));
   }
-  if (h->stream_layout && h->ws_tma_enabled) {h->ws_tma_ok = make_noise_maps(h);}
+  if (h->stream_layout) {h->ws_tma_ok = make_noise_maps(h);}
   CUDA_TRY(h, cudaMalloc(&h->d_cells, B * T * sizeof(int)));
   CUDA_TRY(h, cudaMalloc(&h->d_params, kParamsCapacity + 256));
   CUDA_TRY(h, cudaMalloc(&h->d_cs, 3 * T * sizeof(float)));
@@ -2294,22 +2130,19 @@ mppi_status mppi_get_control_history(mppi_handle * h, float hist12[12])
   return MPPI_OK;
 }
 
-// Multi-robot server: bind n handles of one device (same batch_size / time_steps, tile layout, not sharded) into a
-// group.  They share the first handle's stream from here on, and mppi_optimize_batch[_resident] over exactly this group
-// (same order) becomes ONE kernel launch for all robots.  Everything else keeps working on bound handles.
+// Multi-robot server: bind n handles of one device (same batch_size / time_steps, not sharded) into a group.  They
+// move to the stream layout and share the first handle's stream from here on, and mppi_optimize_batch[_resident] over
+// exactly this group (same order) runs as four kernel launches per chunk of up to 64 robots.  Everything else keeps
+// working on bound handles.
 mppi_status mppi_batch_bind(mppi_handle ** hs, int32_t n)
 {
   if (!hs || n < 1 || !hs[0]) {return MPPI_E_CONFIG;}
   mppi_handle * L = hs[0];
-  // mode 2 (default): the members move to the stream layout and the group runs as four batched kernels; mode 1
-  // (MPPI_BATCH_MODE=tile): the members stay in the tile layout, one ticketed fused kernel per 16 robots
-  int mode = 2;
-  if (const char * e = std::getenv("MPPI_BATCH_MODE")) {mode = std::strcmp(e, "tile") == 0 ? 1 : 2;}
   for (int i = 0; i < n; ++i) {
     mppi_handle * h = hs[i];
     if (!h) {return MPPI_E_CONFIG;}
     if (h->device != L->device || h->B != L->B || h->T != L->T) {return fail(L, MPPI_E_CONFIG, "mppi_batch_bind: handles must share device, batch_size and time_steps");}
-    if ((mode == 1 && h->stream_layout) || h->nranks > 1 || h->cfg.regenerate_noises) {return fail(L, MPPI_E_CONFIG, "mppi_batch_bind: unsharded handles without regenerate_noises only (tile mode: tile layout only)");}
+    if (h->nranks > 1 || h->cfg.regenerate_noises) {return fail(L, MPPI_E_CONFIG, "mppi_batch_bind: unsharded handles without regenerate_noises only");}
     for (int k = 0; k < i; ++k) {if (hs[k] == h) {return fail(L, MPPI_E_CONFIG, "mppi_batch_bind: duplicate handle");}}
   }
   for (int i = 0; i < n; ++i) {
@@ -2318,39 +2151,31 @@ mppi_status mppi_batch_bind(mppi_handle ** hs, int32_t n)
   CUDA_TRY(L, cudaSetDevice(L->device));
   CUDA_TRY(L, cudaHostAlloc(&L->h_jobs, sizeof(FusedJob) * static_cast<size_t>(n), cudaHostAllocDefault));
   CUDA_TRY(L, cudaMalloc(&L->d_jobs, sizeof(FusedJob) * static_cast<size_t>(n)));
-  CUDA_TRY(L, cudaMalloc(&L->d_ticket, sizeof(unsigned)));
-  CUDA_TRY(L, cudaMemsetAsync(L->d_ticket, 0, sizeof(unsigned), L->stream));
-  L->ticket_base = 0;
   L->jobs_sent.assign(sizeof(FusedJob) * static_cast<size_t>(n), 0);
   std::memset(L->h_jobs, 0, sizeof(FusedJob) * static_cast<size_t>(n));
   L->batch_group.assign(hs, hs + n);
-  L->batch_mode = mode;
   L->batch_tag = 0;
-  if (mode == 2) {
-    size_t cap = 64 * 1024;
-    for (int i = 0; i < n; ++i) {cap = std::max(cap, hs[i]->costmap_capacity);}
-    L->arena_slice = (kParamsCapacity + 256 + cap + 255) & ~static_cast<size_t>(255);
-    CUDA_TRY(L, cudaHostAlloc(&L->arena_h, L->arena_slice * n, cudaHostAllocMapped | cudaHostAllocPortable));
-    CUDA_TRY(L, cudaMalloc(&L->arena_d, L->arena_slice * n));
-    CUDA_TRY(L, cudaStreamCreateWithFlags(&L->copy_stream, cudaStreamNonBlocking));
-    for (auto & e : L->ev_upload) {CUDA_TRY(L, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));}
-  }
+  size_t cap = 64 * 1024;
+  for (int i = 0; i < n; ++i) {cap = std::max(cap, hs[i]->costmap_capacity);}
+  L->arena_slice = (kParamsCapacity + 256 + cap + 255) & ~static_cast<size_t>(255);
+  CUDA_TRY(L, cudaHostAlloc(&L->arena_h, L->arena_slice * n, cudaHostAllocMapped | cudaHostAllocPortable));
+  CUDA_TRY(L, cudaMalloc(&L->arena_d, L->arena_slice * n));
+  CUDA_TRY(L, cudaStreamCreateWithFlags(&L->copy_stream, cudaStreamNonBlocking));
+  for (auto & e : L->ev_upload) {CUDA_TRY(L, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));}
   for (int i = 0; i < n; ++i) {
     mppi_handle * h = hs[i];
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     drop_graphs(h);
-    if (mode == 2) {
-      const mppi_status s = to_stream_layout(h);
-      if (s != MPPI_OK) {batch_unbind_group(L); return s;}
-      cudaFreeHost(h->h_params); cudaFree(h->d_params);
-      h->h_params = L->arena_h + L->arena_slice * i;
-      h->d_params = L->arena_d + L->arena_slice * i;
-      h->h_costmap = nullptr; h->d_costmap = nullptr;
-      h->costmap_capacity = L->arena_slice - kParamsCapacity - 256;
-      h->params_in_arena = true;
-      h->cycle_uploaded = false;
-      std::memset(h->h_res, 0, (3 * static_cast<size_t>(h->T) + 10) * sizeof(uint2));
-    }
+    const mppi_status s = to_stream_layout(h);
+    if (s != MPPI_OK) {batch_unbind_group(L); return s;}
+    cudaFreeHost(h->h_params); cudaFree(h->d_params);
+    h->h_params = L->arena_h + L->arena_slice * i;
+    h->d_params = L->arena_d + L->arena_slice * i;
+    h->h_costmap = nullptr; h->d_costmap = nullptr;
+    h->costmap_capacity = L->arena_slice - kParamsCapacity - 256;
+    h->params_in_arena = true;
+    h->cycle_uploaded = false;
+    std::memset(h->h_res, 0, (3 * static_cast<size_t>(h->T) + 10) * sizeof(uint2));
     h->batch_leader = L;
     if (h != L) {h->own_stream = h->stream; h->stream = L->stream;}
   }

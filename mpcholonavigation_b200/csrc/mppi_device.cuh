@@ -92,8 +92,6 @@ struct DevParams
   int vis_b_step, vis_t_step, vis_nb;        // visualiser feed: every vis_b_step-th trajectory x every vis_t_step-th step (0: off)
   int need_furthest;                         // some path critic may ask for the furthest reached path point
   int noise_tm;                              // noise planes are stored time-major [T][B] (stream layout) instead of [B][T]
-  int scan_mode;                             // 1: EXPERIMENT (MPPI_SCAN=warp) - the three cumsums as warp-shuffle prefix scans along the horizon
-                                             // (re-associated fp32 sums: NOT the reference's order, see profiles/r02_scan_experiment.json)
   // offsets (in floats) of the path arrays that follow this struct in the same buffer
   int off_path_x, off_path_y, off_path_yaw, off_path_D;
   // host-made tables behind the path arrays (build_params): valid[n16] (utils::findPathCosts, utils.hpp:361-394),

@@ -14,8 +14,7 @@
 //  KF tile_fused_kernel            small batches, one rank: K2's body, both grid-wide exchanges (as packets), the path critics,
 //                                  the update, the merge and the evalControl tail in ONE cooperative launch; zero-copy upload
 //                                  in, result packets out (the default 1000 x 56 path)
-//     tile_fused_batch_kernel      the same for several robots per launch (blocks draw tickets)
-//     *_batch_kernel (stream)      K2 / K3a / K3c / K4 of the stream layout with the robot as the last grid dimension
+//     *_batch_kernel (stream)     K2 / K3a / K3c / K4 of the stream layout with the robot as the last grid dimension
 //
 // Work shape of K2: one CTA owns a tile of 32 trajectories (lane == trajectory) and S warps split the
 // horizon into S contiguous segments.  The tile lives in shared memory time-major, [T][33] floats per
@@ -79,7 +78,6 @@ struct DevBuffers
   uint2 * pk_out;       // [3T]           evalControl tail: the new sequence on its way from the owner tiles to tile 0
   unsigned * epoch;     // completed fused launches of this handle; the tag of the running launch is *epoch + 1
   unsigned * host_err;  // pinned host word (behind the result packets): a bounded poll gave up inside this handle's kernels
-  int k3_fast;          // the stream layout's path-cost kernel may take its lean per-trajectory total (MPPI_K3_FAST=0: never)
 };
 
 // A bounded poll timed out: sticky flag in device memory and, for the cycles whose result leaves as packets (no D2H of the
@@ -172,8 +170,7 @@ struct FusedCtx
   const float * s_hot, * s_cs;
   const float * s_cvx, * s_cvy, * s_cwz, * s_yaw, * s_x, * s_y;   // time-major tile planes [T][33]
   int n_cap, iteration;   // n_cap: path capacity the shared-memory carve-up was sized for (>= the record's N)
-  int tile, ntiles;       // this block's tile of the problem and the number of tiles (blockIdx.x / gridDim.x for a launch
-                          // of one problem; ticket-derived when one launch serves several robots)
+  int tile, ntiles;       // this block's tile of the problem and the number of tiles (blockIdx.x / gridDim.x)
   unsigned tag;           // tag of this launch's packets
   // zero-copy upload: the cycle's record + costmap sit in pinned host memory (up_host, up_vecs 16-byte vectors, laid
   // out like the device buffer that starts at the record); every tile reads the hot part of the record straight from
@@ -476,34 +473,8 @@ __device__ __forceinline__ void rollout_tile_body(
     if (!use_vy) {pvy = 0.0f;}
   }
 
-  // ---- P2 (experiment, MPPI_SCAN=warp): the same cumsum as a warp-shuffle inclusive scan ALONG THE HORIZON (lane = time
-  //      step, 32 steps per pass, carry between passes), trajectories dealt to the warps.  This is what north_star item (2)
-  //      names; it re-associates the fp32 sums, so poses - and with them costmap cells - can differ from the reference's
-  //      sequential order.  Measured and rejected for the parity path (profiles/r02_scan_experiment.json).  Compiled into
-  //      the generic instance only: the host runs that one while the switch is set (stream_feature_need), so the exact
-  //      instances carry none of its code.
-  const bool warp_scan = !kExact && mode == 0 && p.scan_mode != 0;
-  if (warp_scan) {
-    const float yaw0 = p.yaw0;
-    for (int r = seg; r < kTile && b0 + r < B; r += S) {
-      float carry = -0.0f;
-      for (int c0 = 0; c0 < T; c0 += 32) {
-        const int t = c0 + lane;
-        float term = 0.0f;
-        if (t < T) {term = __fmul_rn(t == 0 ? s_v0[2 * kTile + r] : s_cwz[(t - 1) * kPad + r], dt);}
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-          const float up = __shfl_up_sync(0xffffffffu, term, d);
-          if (lane >= d) {term = __fadd_rn(up, term);}
-        }
-        const float v = __fadd_rn(carry, term);
-        if (t < T) {s_yaw[t * kPad + r] = __fadd_rn(v, yaw0);}
-        carry = __shfl_sync(0xffffffffu, v, 31);
-      }
-    }
-  }
   // ---- P2: yaw = cumsum(wz * dt) + yaw0, sequential in t (optimizer.cpp:319-320)
-  if (mode != 2 && seg == 0 && live && !warp_scan) {
+  if (mode != 2 && seg == 0 && live) {
     // chunks of 8: the eight loads are independent (pipelined), only the eight adds form the carried chain
     const float yaw0 = p.yaw0;
     float acc = -0.0f;                       // (-0) + x == x bit for bit: the first element of the cumsum is the term itself
@@ -616,30 +587,7 @@ __device__ __forceinline__ void rollout_tile_body(
   if (mode != 2) {
     __syncthreads();
     // ---- P4: x = pose.x (double) + cumsum(dx*dt) (float), sequential in t (optimizer.cpp:339-342)
-    if (warp_scan) {
-      // experiment (see P2): x and y as warp-shuffle scans along the horizon
-      for (int r = seg; r < kTile && b0 + r < B; r += S) {
-#pragma unroll
-        for (int pl = 0; pl < 2; ++pl) {
-          float * plane = pl == 0 ? s_x : s_y;
-          const double origin = pl == 0 ? p.pose_x : p.pose_y;
-          float carry = -0.0f;
-          for (int c0 = 0; c0 < T; c0 += 32) {
-            const int t = c0 + lane;
-            float term = t < T ? plane[t * kPad + r] : 0.0f;
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-              const float up = __shfl_up_sync(0xffffffffu, term, d);
-              if (lane >= d) {term = __fadd_rn(up, term);}
-            }
-            const float v = __fadd_rn(carry, term);
-            if (t < T) {plane[t * kPad + r] = static_cast<float>(origin + static_cast<double>(v));}
-            carry = __shfl_sync(0xffffffffu, v, 31);
-          }
-        }
-      }
-    }
-    if (live && seg < 2 && !warp_scan) {
+    if (live && seg < 2) {
       const bool do_x = seg == 0, do_y = (S > 1) ? (seg == 1) : true;
       // one plane per warp (x: warp 0, y: warp 1), chunks of 8 as above; the fp64 pose add is off the carried chain
       auto scan_plane = [&](float * plane, const double origin) {
@@ -1979,7 +1927,7 @@ __device__ __forceinline__ void path_costs_tm_body(const DevParams * __restrict_
   const int B = P->B, T = P->T;
   float m = 3.402823466e+38f;
   // block-uniform: the usual pass runs the lean total (k3_trajectory_total_fast), anything else the general one
-  const bool fast = bufs.k3_fast && P->mode == 0 && !P->want_critic_rows && !dec.legacy_go && !dec.angle_go && !(dec.align_go && P->align_use_yaw);
+  const bool fast = P->mode == 0 && !P->want_critic_rows && !dec.legacy_go && !dec.angle_go && !(dec.align_go && P->align_use_yaw);
   __shared__ unsigned s_srcw[kMaxCritics / 4];
   if (tid < kMaxCritics / 4) {   // where the term of every list position comes from this pass, four positions to a word
     unsigned v = 0u;
@@ -2450,7 +2398,7 @@ __device__ __forceinline__ void put_result(float * out, uint2 * host_res, int id
 #ifndef MPPI_FUSED_MIN_BLOCKS
 #define MPPI_FUSED_MIN_BLOCKS 2
 #endif
-// the work of one block on tile `tile` of `G` of one problem (see the header comment above)
+// the work of one block on tile `tile` of `G` (blockIdx.x of gridDim.x; see the header comment above)
 template<unsigned F, bool kExact>
 __device__ __forceinline__ void tile_fused_body(
   const DevParams * Pg, const uint8_t * cm, const DevBuffers & bufs, const int B, const int T, const int n_cap,
@@ -2775,53 +2723,6 @@ __global__ void __launch_bounds__(256, MPPI_FUSED_MIN_BLOCKS) tile_fused_kernel(
   const int iteration, uint2 * host_res, const uint4 * up_host, const int up_vecs, const int tail_mode, float * hist)
 {
   tile_fused_body<F, kExact>(Pg, cm, bufs, B, T, n_cap, iteration, host_res, up_host, up_vecs, blockIdx.x, gridDim.x, tail_mode, hist);
-}
-
-// One launch for several robots (independent problems of the same shape: BASELINE configs[4]).  Block r * G + tile works
-// on tile `tile` of robot r.  The tiles of one robot wait for each other (packet exchanges), and a grid this large is not
-// co-resident, so a block does not take its work from blockIdx: it draws a TICKET from a counter when it starts running.
-// Tickets are consecutive, so at any time at most one robot is incomplete (has tickets not yet drawn); every earlier robot
-// has all its blocks running or finished and therefore completes without waiting for anything that is not resident, which
-// frees the slots the incomplete robot's remaining blocks need: no deadlock whatever the dispatch order.  The counter is
-// never reset: the host passes the number of tickets drawn by earlier launches (base).
-struct __align__(16) FusedJob
-{
-  const DevParams * Pg;
-  const uint8_t * cm;
-  DevBuffers bufs;
-  int B, T, n_cap, iteration;
-  uint2 * host_res;
-  const uint4 * up_host;
-  int up_vecs, pad;
-};
-static_assert(sizeof(FusedJob) % 16 == 0, "jobs are copied as 16-byte vectors");
-
-template<unsigned F, bool kExact>
-__global__ void __launch_bounds__(256, MPPI_FUSED_MIN_BLOCKS) tile_fused_batch_kernel(
-  const FusedJob * __restrict__ jobs, const int G, unsigned * ticket_counter, const unsigned ticket_base)
-{
-  __shared__ __align__(16) FusedJob s_job;
-  __shared__ unsigned s_ticket;
-  const int tid = threadIdx.y * kTile + threadIdx.x, nthr = blockDim.y * kTile;
-  constexpr int kVecs = sizeof(FusedJob) / 16;
-  // the ticket is an atomic round trip; the job it will most likely name (in-order dispatch) is fetched meanwhile
-  if (tid == 0) {s_ticket = atomicAdd(ticket_counter, 1u) - ticket_base;}
-  int r = blockIdx.x / G;
-  for (int i = tid; i < kVecs; i += nthr) {
-    reinterpret_cast<uint4 *>(&s_job)[i] = __ldg(reinterpret_cast<const uint4 *>(jobs + r) + i);
-  }
-  __syncthreads();
-  const unsigned ticket = s_ticket;
-  if (static_cast<int>(ticket / G) != r) {
-    r = ticket / G;
-    __syncthreads();
-    for (int i = tid; i < kVecs; i += nthr) {
-      reinterpret_cast<uint4 *>(&s_job)[i] = __ldg(reinterpret_cast<const uint4 *>(jobs + r) + i);
-    }
-    __syncthreads();
-  }
-  tile_fused_body<F, kExact>(s_job.Pg, s_job.cm, s_job.bufs, s_job.B, s_job.T, s_job.n_cap, s_job.iteration, s_job.host_res,
-    s_job.up_host, s_job.up_vecs, static_cast<int>(ticket % G), G, 0, nullptr);
 }
 
 // K3c (stream layout): softmax weights and weighted control sums over time-major noise [T][B]; a GEMV
@@ -3501,6 +3402,16 @@ __global__ void optimized_trajectory_kernel(const float * __restrict__ cs, float
 // ONCE for all robots of a group; the robot is the last grid dimension and its buffers come from the job table.
 // Robots are independent problems (own record, costmap, noise, control sequence, state), so nothing else changes.
 // ---------------------------------------------------------------------------------------------------
+// one robot of a group: where its record, costmap, buffers and pinned result packets are
+struct __align__(16) FusedJob
+{
+  const DevParams * Pg;
+  const uint8_t * cm;
+  DevBuffers bufs;
+  uint2 * host_res;
+};
+static_assert(sizeof(FusedJob) % 16 == 0, "the job table is an array of 16-byte aligned records");
+
 template<unsigned F, bool kExact>
 __global__ void __launch_bounds__(kStreamThreads, MPPI_STREAM_MIN_BLOCKS) rollout_score_stream_batch_kernel(const FusedJob * __restrict__ jobs)
 {

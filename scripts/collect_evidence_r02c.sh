@@ -6,8 +6,4 @@ SMI=$!
 timeout 600 python bench.py > $O/bench_default_1gpu.json 2> $O/bench_default_1gpu.err
 kill $SMI
 timeout 300 python bench.py --impl reference > $O/bench_reference_arm.json 2> $O/bench_reference_arm.err
-# block size of the stream rollout at 262144 x 100 (wave tail): 128 (default) against 64 and 32 threads per block, cold L2
-for t in 128 64 32; do
-  MPPI_STREAM_THREADS=$t timeout 200 python scripts/time_variants.py --flush --cycles 20 2>&1 | tail -1 | sed "s/^/threads=$t /" >> $O/stream_threads_262144x100.txt
-done
-cat $O/test_gpu_1gpu.log $O/stream_threads_262144x100.txt; tail -n 2 $O/*.err
+cat $O/test_gpu_1gpu.log; tail -n 2 $O/*.err

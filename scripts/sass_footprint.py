@@ -3,7 +3,7 @@
 
   python scripts/sass_footprint.py [path/to/libmppi_b200.so] [--lines 25] [--bucket 20] [--match tile_fused]
 
-For every tile_fused_kernel / tile_fused_batch_kernel instance: registers and stack frame (cuobjdump -res-usage), the SASS
+For every tile_fused_kernel instance: registers and stack frame (cuobjdump -res-usage), the SASS
 instruction count of the kernel's text section (which holds its __noinline__ callees too: all of it can be fetched by one
 launch), the CALL, LDL / STL, SHFL and BAR counts, and where the instructions come from (nvdisasm --print-line-info-inline):
   - by the innermost source line (device helpers show as themselves), the largest --lines entries;

@@ -135,16 +135,13 @@ def test_costmap_resize_and_large_costmap_fall_back_to_the_copy_engine(product_f
     g.close(); o.close()
 
 
-@pytest.mark.parametrize("mode", ["stream", "tile"])
-def test_bound_group_against_the_single_calls(product_fns, oracle_fns, monkeypatch, mode):
-    """mppi_batch_bind, both forms.  "tile": mppi_optimize_batch over the group = ONE kernel launch
-    (tile_fused_batch_kernel, blocks draw tickets) with the same bits as one mppi_optimize per robot.  "stream" (default):
-    the members move to the stream layout, one strided upload and FOUR launches serve all robots; same controls within
-    the tolerance (different summation order).  A member keeps working on its own afterwards, and the group dissolves when
-    a member is destroyed."""
+@pytest.mark.parametrize("mode", ["stream"])
+def test_bound_group_against_the_single_calls(product_fns, oracle_fns, mode):
+    """mppi_batch_bind: the members move to the stream layout, one strided upload and FOUR launches serve all robots;
+    same controls as one mppi_optimize per robot within the tolerance (different summation order).  A member keeps
+    working on its own afterwards, and the group dissolves when a member is destroyed."""
     import ctypes as C
     from mpcholonavigation_b200 import abi
-    monkeypatch.setenv("MPPI_BATCH_MODE", mode)
     n = 9
     scs = [scenarios.config5_robot(r, batch=700) for r in range(n)]   # 22 tiles each: 198 blocks in one launch
     T = scs[0].cfg["time_steps"]
@@ -175,20 +172,17 @@ def test_bound_group_against_the_single_calls(product_fns, oracle_fns, monkeypat
             assert product_fns["optimize_batch_resident"](hs, outs, n) == 0
         for i in range(n):
             for a, name in zip(bufs[i], ("vx", "vy", "wz")):
-                if mode == "tile":
-                    assert np.array_equal(a, getattr(refs[i], name)), f"cycle {cycle} robot {i} {name}"
-                else:
-                    np.testing.assert_allclose(a, getattr(refs[i], name), rtol=RTOL, atol=ATOL, err_msg=f"cycle {cycle} robot {i} {name}")
+                np.testing.assert_allclose(a, getattr(refs[i], name), rtol=RTOL, atol=ATOL, err_msg=f"cycle {cycle} robot {i} {name}")
             assert outs[i].fail_flag == refs[i].fail_flag
             assert outs[i].furthest_reached_path_point == refs[i].furthest_reached_path_point
-        if mode == "stream":   # keep both sides on the same warm start so that the comparison stays point-wise
-            for i, e in enumerate(group):
-                e.set_control_sequence(refs[i].vx, refs[i].vy, refs[i].wz)
+        # keep both sides on the same warm start so that the comparison stays point-wise
+        for i, e in enumerate(group):
+            e.set_control_sequence(refs[i].vx, refs[i].vy, refs[i].wz)
         np.testing.assert_allclose(bufs[4][0], ro.vx, rtol=RTOL, atol=ATOL)
         np.testing.assert_allclose(bufs[4][2], ro.wz, rtol=RTOL, atol=ATOL)
         orc.set_control_sequence(*[b.copy() for b in bufs[4]])
     n_launches = sum(e.get_profile()["kernel_launches"] for e in group) - launches0
-    assert n_launches == (6 if mode == "tile" else 24)   # per cycle: one launch (tile) / four launches (stream) for 9 robots
+    assert n_launches == 24   # per cycle: four launches for 9 robots
     # a bound member on its own (shares the leader's stream), then the group again, then without the leader
     r_alone = group[3].optimize(scs[3].cycle)
     r_ref = single[3].optimize(scs[3].cycle)

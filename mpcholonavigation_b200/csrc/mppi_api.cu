@@ -138,6 +138,7 @@ struct mppi_handle
   FusedJob * h_jobs{nullptr};             // leader only: job table, pinned ...
   FusedJob * d_jobs{nullptr};             // ... and its device copy (re-sent only when an entry changes)
   std::vector<char> jobs_sent;            // what the device copy holds
+  NoiseJob * d_noise_jobs{nullptr};       // leader only: the regenerate_noises members, in bind order (fixed at bind)
   char * arena_h{nullptr};                // leader: the [record | costmap] buffers of all members, one slice each,
   char * arena_d{nullptr};                //   so that the whole group uploads with ONE strided copy
   size_t arena_slice{0};
@@ -1303,6 +1304,14 @@ mppi_status wait_result_packets(mppi_handle * h)
   return MPPI_OK;
 }
 
+// the event behind the cycle's result: a batched group step ends at the leader's ev1 (its redraw runs behind that), a
+// regenerate_noises handle of its own at ev_result (ahead of its redraw), any other cycle at ev1
+cudaEvent_t result_event(const mppi_handle * h)
+{
+  if (h->ev_src) {return h->ev_src->ev1;}
+  return h->cfg.regenerate_noises ? h->ev_result : h->ev1;
+}
+
 mppi_status finish_optimize(mppi_handle * h, mppi_cycle_out * out)
 {
   const uint64_t t_a = now_ns();
@@ -1321,7 +1330,7 @@ mppi_status finish_optimize(mppi_handle * h, mppi_cycle_out * out)
       return fail(h, h->nranks > 1 ? MPPI_E_NCCL : MPPI_E_CUDA,
                "an in-kernel packet exchange timed out (a tile or rank never delivered): result discarded");
     }
-    if (h->timing) {CUDA_TRY(h, cudaEventSynchronize(h->cfg.regenerate_noises ? h->ev_result : (h->ev_src ? h->ev_src : h)->ev1));}
+    if (h->timing) {CUDA_TRY(h, cudaEventSynchronize(result_event(h)));}
   } else if (h->cfg.regenerate_noises) {
     CUDA_TRY(h, cudaEventSynchronize(h->ev_result));
   } else {
@@ -1350,7 +1359,7 @@ mppi_status finish_optimize(mppi_handle * h, mppi_cycle_out * out)
   float ms = 0.0f;
   if (h->timing) {
     const mppi_handle * es = h->ev_src ? h->ev_src : h;
-    cudaEventElapsedTime(&ms, es->ev0, h->cfg.regenerate_noises ? h->ev_result : es->ev1);
+    cudaEventElapsedTime(&ms, es->ev0, result_event(h));
   }
   h->prof_ms[3] = ms;
   if (out) {out->device_ms = ms;}
@@ -1493,6 +1502,7 @@ void batch_unbind_group(mppi_handle * leader)
   leader->jobs_sent.clear();
   if (leader->h_jobs) {cudaFreeHost(leader->h_jobs); leader->h_jobs = nullptr;}
   if (leader->d_jobs) {cudaFree(leader->d_jobs); leader->d_jobs = nullptr;}
+  if (leader->d_noise_jobs) {cudaFree(leader->d_noise_jobs); leader->d_noise_jobs = nullptr;}
 }
 
 // is hs[0..n) exactly a bound group, in bind order?
@@ -1544,20 +1554,39 @@ bool batch_stream_ok(mppi_handle ** hs, int n)
   mppi_handle * L = hs[0];
   for (int i = 0; i < n; ++i) {
     const mppi_handle * h = hs[i];
-    if (!h->stream_layout || !h->params_in_arena || h->tail_mode != 0 || h->cfg.iteration_count != 1 || h->profiling ||
-      h->cfg.regenerate_noises || h->nranks > 1)
-    {
+    if (!h->stream_layout || !h->params_in_arena || h->tail_mode != 0 || h->profiling || h->nranks > 1) {
       L->err = std::string("batched launch not used: member ") + std::to_string(i) + " does not qualify this cycle";
+      return false;
+    }
+    if (h->cfg.iteration_count != L->cfg.iteration_count) {
+      L->err = std::string("batched launch not used: member ") + std::to_string(i) + " has another iteration_count than member 0";
       return false;
     }
   }
   return true;
 }
 
-// One cycle of the members [c0, c0 + n) of a stream-layout group (records built): ONE strided upload, then K2 / K3a /
-// K3c / K4 launched once each with the robot as the last grid dimension; results as packets (tag) in each member's pinned
-// result buffer.  first / last: the leader's events bracket the whole call.
-mppi_status batch_stream_launch(mppi_handle * L, mppi_handle ** hs, int c0, int n, bool with_upload, uint32_t tag, bool first, bool last)
+// regenerate_noises redraw of the entries [k0, k0 + kn) of the group's noise table, then their Philox stream indices
+// advance (a separate launch, like launch_regenerate: every block of the redraw reads the index first)
+mppi_status batch_redraw(mppi_handle * L, int k0, int kn)
+{
+  if (kn <= 0) {return MPPI_OK;}
+  const long long total = static_cast<long long>(L->B) * ((L->T + 3) / 4);
+  const int blocks = static_cast<int>(std::min<long long>((total + 255) / 256, 148LL * 16));
+  noise_philox_batch_kernel<<<dim3(std::max(blocks, 1), kn), 256, 0, L->stream>>>(L->d_noise_jobs + k0);
+  advance_epoch_batch_kernel<<<(kn + 255) / 256, 256, 0, L->stream>>>(L->d_noise_jobs + k0, kn);
+  CUDA_TRY(L, cudaGetLastError());
+  L->launches += 2;
+  return MPPI_OK;
+}
+
+// One cycle of the members [c0, c0 + n) of a stream-layout group (records built): ONE strided upload, then per iteration
+// K2 / K3a / K3c / K4 launched once each with the robot as the last grid dimension; results as packets (tag) in each
+// member's pinned result buffer, written by the last iteration's K4.  Between iterations the chunk's regenerate_noises
+// members, entries [k0, k0 + kn) of the noise table, draw a fresh set.  first / last: the leader's events bracket the
+// whole call.
+mppi_status batch_stream_launch(mppi_handle * L, mppi_handle ** hs, int c0, int n, int k0, int kn, bool with_upload, uint32_t tag,
+  bool first, bool last)
 {
   unsigned inst = pick_stream_instance(stream_feature_need(hs[0]->last));
   size_t max_used = 0;
@@ -1598,37 +1627,46 @@ mppi_status batch_stream_launch(mppi_handle * L, mppi_handle ** hs, int c0, int 
   }
   const FusedJob * jobs = L->d_jobs + c0;
   const int T = L->T, B = L->B;
-  {
-    const int nthr = stream_block_threads(L);
-    const int Tp = ((T + kStreamChunk - 1) / kStreamChunk) * kStreamChunk;
-    const size_t smem = kHotBytes + sizeof(float) * 3 * (Tp + nthr);
-    cudaError_t e;
-    switch (inst) {
-      case kSfOmniDefault: e = launch_stream_batch_instance<kSfOmniDefault, true>(L, jobs, n, nthr, smem); break;
-      case kSfOmniDefaultFp: e = launch_stream_batch_instance<kSfOmniDefaultFp, true>(L, jobs, n, nthr, smem); break;
-      case kSfObstaclesFp: e = launch_stream_batch_instance<kSfObstaclesFp, true>(L, jobs, n, nthr, smem); break;
-      default: e = launch_stream_batch_instance<SF_ALL, false>(L, jobs, n, nthr, smem); break;
+  const int iterations = L->cfg.iteration_count;   // shared by every member (batch_stream_ok)
+  for (int it = 0; it < iterations; ++it) {
+    {
+      const int nthr = stream_block_threads(L);
+      const int Tp = ((T + kStreamChunk - 1) / kStreamChunk) * kStreamChunk;
+      const size_t smem = kHotBytes + sizeof(float) * 3 * (Tp + nthr);
+      cudaError_t e;
+      switch (inst) {
+        case kSfOmniDefault: e = launch_stream_batch_instance<kSfOmniDefault, true>(L, jobs, n, nthr, smem); break;
+        case kSfOmniDefaultFp: e = launch_stream_batch_instance<kSfOmniDefaultFp, true>(L, jobs, n, nthr, smem); break;
+        case kSfObstaclesFp: e = launch_stream_batch_instance<kSfObstaclesFp, true>(L, jobs, n, nthr, smem); break;
+        default: e = launch_stream_batch_instance<SF_ALL, false>(L, jobs, n, nthr, smem); break;
+      }
+      CUDA_TRY(L, e);
     }
-    CUDA_TRY(L, e);
-  }
-  {
-    const int grid = std::min((B + kUpdThreads - 1) / kUpdThreads, 148 * 8);
-    path_costs_tm_batch_kernel<<<dim3(grid, n), kUpdThreads, k3_common_smem_bytes(), L->stream>>>(jobs);
-    CUDA_TRY(L, cudaGetLastError());
-  }
-  const int chunks = (B + kWsChunk - 1) / kWsChunk;
-  {
-    const int gy = weighted_sums_row_groups(T, chunks * n);   // the rows are split less when many robots fill the machine
-    weighted_sums_tm_batch_kernel<<<dim3(chunks, gy, n), kWsThreads, 0, L->stream>>>(jobs);
-    CUDA_TRY(L, cudaGetLastError());
-  }
-  {
-    const int merge_grid = (T + kMergeT - 1) / kMergeT;
-    merge_finalize_batch_kernel<<<dim3(merge_grid, n), kUpdThreads, 0, L->stream>>>(jobs, chunks, 3 * T + 2, tag);
-    CUDA_TRY(L, cudaGetLastError());
+    {
+      // iteration > 0: the costs accumulate onto the previous iteration's (quirk R20)
+      const int grid = std::min((B + kUpdThreads - 1) / kUpdThreads, 148 * 8);
+      path_costs_tm_batch_kernel<<<dim3(grid, n), kUpdThreads, k3_common_smem_bytes(), L->stream>>>(jobs, it);
+      CUDA_TRY(L, cudaGetLastError());
+    }
+    const int chunks = (B + kWsChunk - 1) / kWsChunk;
+    {
+      const int gy = weighted_sums_row_groups(T, chunks * n);   // the rows are split less when many robots fill the machine
+      weighted_sums_tm_batch_kernel<<<dim3(chunks, gy, n), kWsThreads, 0, L->stream>>>(jobs);
+      CUDA_TRY(L, cudaGetLastError());
+    }
+    const bool final_it = it + 1 == iterations;
+    {
+      const int merge_grid = (T + kMergeT - 1) / kMergeT;
+      merge_finalize_batch_kernel<<<dim3(merge_grid, n), kUpdThreads, 0, L->stream>>>(jobs, chunks, 3 * T + 2, tag, final_it ? 1 : 0);
+      CUDA_TRY(L, cudaGetLastError());
+    }
+    L->launches += 4;
+    if (!final_it) {
+      const mppi_status s = batch_redraw(L, k0, kn);
+      if (s != MPPI_OK) {return s;}
+    }
   }
   if (last && L->timing) {CUDA_TRY(L, cudaEventRecord(L->ev1, L->stream));}
-  L->launches += 4;
   return MPPI_OK;
 }
 
@@ -1660,8 +1698,11 @@ mppi_status batch_run_group(mppi_handle ** hs, const mppi_cycle_in * ins, mppi_c
   std::vector<char> pending(n, 0);
   const uint32_t tag = 0x80000000u | (++L->batch_tag);   // never a tag of the fused kernel's epochs
   const int chunk = ins ? kStreamBatchChunk : n;
+  int k0 = 0;   // the chunk's first entry in the noise table (regenerate_noises members, in bind order)
   for (int c0 = 0; c0 < n; c0 += chunk) {
     const int cn = std::min(chunk, n - c0);
+    int kn = 0;
+    for (int i = c0; i < c0 + cn; ++i) {kn += hs[i]->cfg.regenerate_noises ? 1 : 0;}
     mppi_status s = MPPI_OK;
     for (int i = c0; i < c0 + cn && s == MPPI_OK; ++i) {
       if (ins) {
@@ -1672,12 +1713,25 @@ mppi_status batch_run_group(mppi_handle ** hs, const mppi_cycle_in * ins, mppi_c
         s = fail(hs[i], MPPI_E_STATE, "mppi_optimize_batch_resident before mppi_upload_cycle");
       }
     }
-    if (s == MPPI_OK) {s = batch_stream_launch(L, hs + c0, c0, cn, ins != nullptr, tag, c0 == 0, c0 + cn == n);}
+    if (s == MPPI_OK) {s = batch_stream_launch(L, hs + c0, c0, cn, k0, kn, ins != nullptr, tag, c0 == 0, c0 + cn == n);}
     if (s == MPPI_OK) {
       for (int i = c0; i < c0 + cn; ++i) {pending[i] = 1;}
     } else if (first == MPPI_OK) {
       first = s;
     }
+    k0 += kn;
+  }
+  // regenerate_noises: the set for the next step, drawn behind the last chunk's results (the host polls their packets,
+  // not the stream) in one launch over every member that ran; finish_optimize advances each host mirror to match
+  int run0 = 0, k = 0;
+  for (int i = 0; i <= n; ++i) {
+    if (i < n && !hs[i]->cfg.regenerate_noises) {continue;}
+    if (i == n || !pending[i]) {
+      const mppi_status s = batch_redraw(L, run0, k - run0);
+      if (s != MPPI_OK && first == MPPI_OK) {first = s;}
+      run0 = k + 1;
+    }
+    ++k;
   }
   for (int i = 0; i < n; ++i) {
     if (!pending[i]) {continue;}
@@ -2132,8 +2186,8 @@ mppi_status mppi_get_control_history(mppi_handle * h, float hist12[12])
 
 // Multi-robot server: bind n handles of one device (same batch_size / time_steps, not sharded) into a group.  They
 // move to the stream layout and share the first handle's stream from here on, and mppi_optimize_batch[_resident] over
-// exactly this group (same order) runs as four kernel launches per chunk of up to 64 robots.  Everything else keeps
-// working on bound handles.
+// exactly this group (same order) runs as four kernel launches per iteration per chunk of up to 64 robots, plus the
+// regenerate_noises redraws.  Everything else keeps working on bound handles.
 mppi_status mppi_batch_bind(mppi_handle ** hs, int32_t n)
 {
   if (!hs || n < 1 || !hs[0]) {return MPPI_E_CONFIG;}
@@ -2142,7 +2196,7 @@ mppi_status mppi_batch_bind(mppi_handle ** hs, int32_t n)
     mppi_handle * h = hs[i];
     if (!h) {return MPPI_E_CONFIG;}
     if (h->device != L->device || h->B != L->B || h->T != L->T) {return fail(L, MPPI_E_CONFIG, "mppi_batch_bind: handles must share device, batch_size and time_steps");}
-    if (h->nranks > 1 || h->cfg.regenerate_noises) {return fail(L, MPPI_E_CONFIG, "mppi_batch_bind: unsharded handles without regenerate_noises only");}
+    if (h->nranks > 1) {return fail(L, MPPI_E_CONFIG, "mppi_batch_bind: unsharded handles only");}
     for (int k = 0; k < i; ++k) {if (hs[k] == h) {return fail(L, MPPI_E_CONFIG, "mppi_batch_bind: duplicate handle");}}
   }
   for (int i = 0; i < n; ++i) {
@@ -2178,6 +2232,26 @@ mppi_status mppi_batch_bind(mppi_handle ** hs, int32_t n)
     std::memset(h->h_res, 0, (3 * static_cast<size_t>(h->T) + 10) * sizeof(uint2));
     h->batch_leader = L;
     if (h != L) {h->own_stream = h->stream; h->stream = L->stream;}
+  }
+  // regenerate_noises members: what their redraw needs, fixed for the life of the group (planes, configuration, epoch)
+  std::vector<NoiseJob> noise_jobs;
+  for (int i = 0; i < n; ++i) {
+    const mppi_handle * h = hs[i];
+    if (!h->cfg.regenerate_noises) {continue;}
+    NoiseJob j{};
+    for (int p = 0; p < 3; ++p) {j.noise[p] = h->d_noise[p];}
+    j.epoch = h->d_epoch;
+    j.seed = h->cfg.seed;
+    j.B = h->B; j.T = h->T;
+    j.sx = h->cfg.vx_std; j.sy = h->cfg.vy_std; j.sw = h->cfg.wz_std;
+    j.holonomic = holonomic(h) ? 1 : 0;
+    noise_jobs.push_back(j);
+  }
+  if (!noise_jobs.empty()) {
+    const size_t bytes = sizeof(NoiseJob) * noise_jobs.size();
+    CUDA_TRY(L, cudaMalloc(&L->d_noise_jobs, bytes));
+    CUDA_TRY(L, cudaMemcpyAsync(L->d_noise_jobs, noise_jobs.data(), bytes, cudaMemcpyHostToDevice, L->stream));
+    CUDA_TRY(L, cudaStreamSynchronize(L->stream));
   }
   return MPPI_OK;
 }

@@ -15,6 +15,7 @@
 //                                  the update, the merge and the evalControl tail in ONE cooperative launch; zero-copy upload
 //                                  in, result packets out (the default 1000 x 56 path)
 //     *_batch_kernel (stream)     K2 / K3a / K3c / K4 of the stream layout with the robot as the last grid dimension
+//                                  (and K1's regenerate_noises redraw, noise_philox_batch_kernel)
 //
 // Work shape of K2: one CTA owns a tile of 32 trajectories (lane == trajectory) and S warps split the
 // horizon into S contiguous segments.  The tile lives in shared memory time-major, [T][33] floats per
@@ -210,12 +211,12 @@ __device__ __forceinline__ void box_muller(uint32_t a, uint32_t b, float & z0, f
   z1 = __fmul_rn(r, s);
 }
 
-__global__ void __launch_bounds__(256) noise_philox_kernel(
+// one noise set (three planes) of one handle, grid-stride over blockIdx.x; shared by the single-handle and group kernels
+// so that both draw the same bits for the same (seed, stream)
+__device__ __forceinline__ void noise_philox_body(
   float * __restrict__ nvx, float * __restrict__ nvy, float * __restrict__ nwz, int B, int T, float sx, float sy, float sw,
-  int holonomic, uint64_t seed, uint64_t stream, uint64_t shard_offset, int time_major, const unsigned long long * __restrict__ d_epoch)
+  int holonomic, uint64_t seed, uint64_t stream, uint64_t shard_offset, int time_major)
 {
-  // regenerate_noises: the Philox stream index lives in device memory so that a captured graph draws a new set per replay
-  if (d_epoch) {stream = *d_epoch;}
   const int quads = (T + 3) >> 2;
   const long long total = static_cast<long long>(B) * quads;
   for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
@@ -253,6 +254,34 @@ __global__ void __launch_bounds__(256) noise_philox_kernel(
   }
 }
 
+__global__ void __launch_bounds__(256) noise_philox_kernel(
+  float * __restrict__ nvx, float * __restrict__ nvy, float * __restrict__ nwz, int B, int T, float sx, float sy, float sw,
+  int holonomic, uint64_t seed, uint64_t stream, uint64_t shard_offset, int time_major, const unsigned long long * __restrict__ d_epoch)
+{
+  // regenerate_noises: the Philox stream index lives in device memory so that a captured graph draws a new set per replay
+  if (d_epoch) {stream = *d_epoch;}
+  noise_philox_body(nvx, nvy, nwz, B, T, sx, sy, sw, holonomic, seed, stream, shard_offset, time_major);
+}
+
+// regenerate_noises members of a robot group (unsharded, stream layout): what launch_regenerate passes for one handle
+struct __align__(16) NoiseJob
+{
+  float * noise[3];
+  unsigned long long * epoch;   // the member's Philox stream index of the next draw
+  uint64_t seed;
+  int B, T;
+  float sx, sy, sw;
+  int holonomic;
+};
+static_assert(sizeof(NoiseJob) % 16 == 0, "the noise table is an array of 16-byte aligned records");
+
+// the redraw of every listed member in one launch (member = blockIdx.y), bit-equal to noise_philox_kernel per member
+__global__ void __launch_bounds__(256) noise_philox_batch_kernel(const NoiseJob * __restrict__ jobs)
+{
+  const NoiseJob & j = jobs[blockIdx.y];
+  noise_philox_body(j.noise[0], j.noise[1], j.noise[2], j.B, j.T, j.sx, j.sy, j.sw, j.holonomic, j.seed, *j.epoch, 0, 1);
+}
+
 // Compile-time feature sets of the K2 kernels.  An EXACT instance (kExact) is straight-line code for one set of active
 // features (no per-cycle flag tests, no dead critic code: smaller, fewer registers, fewer instruction-cache misses);
 // the generic instance (SF_ALL, !kExact) tests the per-cycle flags of the record at run time.  The host picks the exact
@@ -276,6 +305,13 @@ enum StreamFeature : unsigned
 #define MPPI_SF(bit, flag) (((F & (bit)) != 0) && (kExact || (flag)))
 
 __global__ void advance_epoch_kernel(unsigned long long * d_epoch) {*d_epoch += 1ull;}
+
+// the same for n members of a robot group, behind their noise_philox_batch_kernel
+__global__ void advance_epoch_batch_kernel(const NoiseJob * __restrict__ jobs, int n)
+{
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) {*jobs[i].epoch += 1ull;}
+}
 
 // ---------------------------------------------------------------------------------------------------
 // K2
@@ -3419,10 +3455,10 @@ __global__ void __launch_bounds__(kStreamThreads, MPPI_STREAM_MIN_BLOCKS) rollou
   rollout_score_stream_body<F, kExact>(j.Pg, j.cm, j.bufs);
 }
 
-__global__ void __launch_bounds__(kUpdThreads, 5) path_costs_tm_batch_kernel(const FusedJob * __restrict__ jobs)
+__global__ void __launch_bounds__(kUpdThreads, 5) path_costs_tm_batch_kernel(const FusedJob * __restrict__ jobs, int iteration)
 {
   const FusedJob & j = jobs[blockIdx.y];
-  path_costs_tm_body(j.Pg, j.bufs, 0);
+  path_costs_tm_body(j.Pg, j.bufs, iteration);
 }
 
 __global__ void __launch_bounds__(kWsThreads) weighted_sums_tm_batch_kernel(const FusedJob * __restrict__ jobs)
@@ -3431,10 +3467,11 @@ __global__ void __launch_bounds__(kWsThreads) weighted_sums_tm_batch_kernel(cons
   weighted_sums_tm_body(j.Pg, j.bufs);
 }
 
-__global__ void __launch_bounds__(kUpdThreads) merge_finalize_batch_kernel(const FusedJob * __restrict__ jobs, int n_parts, int stride, unsigned tag)
+// deliver = 0: an earlier iteration of a multi-iteration cycle, which only updates the control sequence
+__global__ void __launch_bounds__(kUpdThreads) merge_finalize_batch_kernel(const FusedJob * __restrict__ jobs, int n_parts, int stride, unsigned tag, int deliver)
 {
   const FusedJob & j = jobs[blockIdx.y];
-  merge_finalize_body(j.Pg, j.bufs.partials, n_parts, stride, j.bufs, 1, nullptr, j.host_res, tag);
+  merge_finalize_body(j.Pg, j.bufs.partials, n_parts, stride, j.bufs, 1, nullptr, deliver ? j.host_res : nullptr, tag);
 }
 
 }  // namespace mppi

@@ -221,10 +221,12 @@ mppi_status mppi_get_control_history(mppi_handle * h, float hist12[12]);
 /* batched multi-robot form: n independent handles (possibly on several devices) launched back to back
  * and then joined, so their kernels overlap */
 mppi_status mppi_optimize_batch(mppi_handle ** hs, const mppi_cycle_in * ins, mppi_cycle_out * outs, int32_t n);
-/* Multi-robot server (BASELINE configs[4]): bind n unsharded handles of ONE device with the same batch_size / time_steps
- * into a group.  The members move to the stream layout and share the first handle's stream from then on, and
+/* Multi-robot server (BASELINE configs[4]): bind n unsharded handles of ONE device into a group.  Members may differ in
+ * batch_size and time_steps (robot types with their own horizon; a handle re-created after a parameter change binds
+ * back with the others).  The members move to the stream layout and share the first handle's stream from then on, and
  * mppi_optimize_batch[_resident] over exactly this group, in this order, runs in chunks of up to 64 robots: each chunk is
- * one strided upload plus four kernel launches per iteration.  Members with regenerate_noises redraw their noise in
+ * one strided upload plus four kernel launches per iteration, each launch sized for the chunk's largest member.  Members
+ * with regenerate_noises redraw their noise in
  * batched launches too (between iterations per chunk, and once for the whole group behind the last chunk's results), and
  * continue the same Philox stream sequence after mppi_batch_unbind.  Every other call keeps working on a bound handle; a
  * cycle whose members do not all qualify (evalControl tail, profiling, members with different iteration_count, ...) runs

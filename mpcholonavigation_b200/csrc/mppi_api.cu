@@ -139,6 +139,7 @@ struct mppi_handle
   FusedJob * d_jobs{nullptr};             // ... and its device copy (re-sent only when an entry changes)
   std::vector<char> jobs_sent;            // what the device copy holds
   NoiseJob * d_noise_jobs{nullptr};       // leader only: the regenerate_noises members, in bind order (fixed at bind)
+  std::vector<long long> noise_items;     // leader only: B * ceil(T / 4) of each entry, the work of its redraw
   char * arena_h{nullptr};                // leader: the [record | costmap] buffers of all members, one slice each,
   char * arena_d{nullptr};                //   so that the whole group uploads with ONE strided copy
   size_t arena_slice{0};
@@ -831,16 +832,22 @@ unsigned pick_stream_instance(unsigned need)
   return SF_ALL;
 }
 
-int stream_block_threads(const mppi_handle * h)
+int stream_block_threads(int B)
 {
   // fewer threads per block below ~4 full blocks per SM: same number of warps, spread evenly over the 148 SMs
-  return h->B >= 148 * 4 * kStreamThreads ? kStreamThreads : 64;
+  return B >= 148 * 4 * kStreamThreads ? kStreamThreads : 64;
+}
+
+// blocks of path_costs_tm_kernel (grid-stride over the trajectories)
+int path_cost_blocks(int B)
+{
+  return std::min((B + kUpdThreads - 1) / kUpdThreads, 148 * 8);
 }
 
 template<unsigned F, bool kExact>
 void launch_stream_instance(mppi_handle * h, int mode)
 {
-  const int nthr = stream_block_threads(h);
+  const int nthr = stream_block_threads(h->B);
   const int Tp = ((h->T + kStreamChunk - 1) / kStreamChunk) * kStreamChunk;
   const size_t smem = kHotBytes + sizeof(float) * 3 * (Tp + nthr);   // hot record, control sequence, footprint slots
   rollout_score_stream_kernel<F, kExact><<<(h->B + nthr - 1) / nthr, nthr, smem, h->stream>>>(
@@ -1030,7 +1037,7 @@ mppi_status launch_update(mppi_handle * h, int mode, int iteration)
 {
   if (mode == 0 && h->stream_layout) {
     // stream layout: totals + global minimum here, weights and weighted sums in weighted_sums_tm_kernel
-    const int grid = std::min((h->B + kUpdThreads - 1) / kUpdThreads, 148 * 8);
+    const int grid = path_cost_blocks(h->B);
     // the iteration that completes the result advances the packet epoch when the result leaves as packets
     const int bump = (stream_packets(h) && iteration + 1 == h->cfg.iteration_count) ? 1 : 0;
     // programmatic dependent launch behind the rollout kernel (not behind an NCCL all-reduce: that is a library launch)
@@ -1503,6 +1510,7 @@ void batch_unbind_group(mppi_handle * leader)
   if (leader->h_jobs) {cudaFreeHost(leader->h_jobs); leader->h_jobs = nullptr;}
   if (leader->d_jobs) {cudaFree(leader->d_jobs); leader->d_jobs = nullptr;}
   if (leader->d_noise_jobs) {cudaFree(leader->d_noise_jobs); leader->d_noise_jobs = nullptr;}
+  leader->noise_items.clear();
 }
 
 // is hs[0..n) exactly a bound group, in bind order?
@@ -1542,9 +1550,9 @@ mppi_status to_stream_layout(mppi_handle * h)
 constexpr int kStreamBatchChunk = 64;   // robots per upload + four launches: the host builds the next chunk's records meanwhile
 
 template<unsigned F, bool kExact>
-cudaError_t launch_stream_batch_instance(mppi_handle * L, const FusedJob * jobs, int n, int nthr, size_t smem)
+cudaError_t launch_stream_batch_instance(mppi_handle * L, const FusedJob * jobs, int n, int blocks, int nthr, size_t smem)
 {
-  rollout_score_stream_batch_kernel<F, kExact><<<dim3((L->B + nthr - 1) / nthr, n), nthr, smem, L->stream>>>(jobs);
+  rollout_score_stream_batch_kernel<F, kExact><<<dim3(blocks, n), nthr, smem, L->stream>>>(jobs);
   return cudaGetLastError();
 }
 
@@ -1567,11 +1575,12 @@ bool batch_stream_ok(mppi_handle ** hs, int n)
 }
 
 // regenerate_noises redraw of the entries [k0, k0 + kn) of the group's noise table, then their Philox stream indices
-// advance (a separate launch, like launch_regenerate: every block of the redraw reads the index first)
+// advance (a separate launch, like launch_regenerate: every block of the redraw reads the index first).  The grid is sized
+// for the largest of these members; the body is grid-stride, so the smaller ones are covered by the same blocks.
 mppi_status batch_redraw(mppi_handle * L, int k0, int kn)
 {
   if (kn <= 0) {return MPPI_OK;}
-  const long long total = static_cast<long long>(L->B) * ((L->T + 3) / 4);
+  const long long total = *std::max_element(L->noise_items.begin() + k0, L->noise_items.begin() + k0 + kn);
   const int blocks = static_cast<int>(std::min<long long>((total + 255) / 256, 148LL * 16));
   noise_philox_batch_kernel<<<dim3(std::max(blocks, 1), kn), 256, 0, L->stream>>>(L->d_noise_jobs + k0);
   advance_epoch_batch_kernel<<<(kn + 255) / 256, 256, 0, L->stream>>>(L->d_noise_jobs + k0, kn);
@@ -1584,16 +1593,22 @@ mppi_status batch_redraw(mppi_handle * L, int k0, int kn)
 // K2 / K3a / K3c / K4 launched once each with the robot as the last grid dimension; results as packets (tag) in each
 // member's pinned result buffer, written by the last iteration's K4.  Between iterations the chunk's regenerate_noises
 // members, entries [k0, k0 + kn) of the noise table, draw a fresh set.  first / last: the leader's events bracket the
-// whole call.
+// whole call.  Members may differ in B and T: every grid dimension spans the chunk's largest extent, and each member's job
+// carries its own extents, so that its surplus blocks return at once.
 mppi_status batch_stream_launch(mppi_handle * L, mppi_handle ** hs, int c0, int n, int k0, int kn, bool with_upload, uint32_t tag,
   bool first, bool last)
 {
   unsigned inst = pick_stream_instance(stream_feature_need(hs[0]->last));
   size_t max_used = 0;
+  int B_max = 0, T_max = 0;
   for (int i = 0; i < n; ++i) {
     if (pick_stream_instance(stream_feature_need(hs[i]->last)) != inst) {inst = SF_ALL;}
     max_used = std::max(max_used, upload_bytes(hs[i]));
+    B_max = std::max(B_max, hs[i]->B);
+    T_max = std::max(T_max, hs[i]->T);
   }
+  const int nthr = stream_block_threads(B_max);
+  int rollout_grid = 0, cost_grid = 0, ws_grid = 0, ws_total = 0, merge_grid = 0;
   if (first && L->timing) {CUDA_TRY(L, cudaEventRecord(L->ev0, L->stream));}
   if (with_upload) {
     // the chunk's slices travel on the group's copy stream, i.e. beside the kernels of the previous chunk (the slices of
@@ -1613,6 +1628,16 @@ mppi_status batch_stream_launch(mppi_handle * L, mppi_handle ** hs, int c0, int 
     j.cm = h->d_costmap;
     j.bufs = make_bufs(h, 0);
     j.host_res = h->h_res;
+    j.rollout_blocks = (h->B + nthr - 1) / nthr;
+    j.cost_blocks = path_cost_blocks(h->B);
+    j.ws_chunks = (h->B + kWsChunk - 1) / kWsChunk;
+    j.merge_blocks = (h->T + kMergeT - 1) / kMergeT;
+    j.stride = 3 * h->T + 2;
+    rollout_grid = std::max(rollout_grid, j.rollout_blocks);
+    cost_grid = std::max(cost_grid, j.cost_blocks);
+    ws_grid = std::max(ws_grid, j.ws_chunks);
+    ws_total += j.ws_chunks;
+    merge_grid = std::max(merge_grid, j.merge_blocks);
     h->wait_packets = true;
     h->zero_copy_now = false;
     h->ev_src = L;
@@ -1626,38 +1651,33 @@ mppi_status batch_stream_launch(mppi_handle * L, mppi_handle ** hs, int c0, int 
     std::memcpy(L->jobs_sent.data() + off, L->h_jobs + c0, bytes);
   }
   const FusedJob * jobs = L->d_jobs + c0;
-  const int T = L->T, B = L->B;
   const int iterations = L->cfg.iteration_count;   // shared by every member (batch_stream_ok)
   for (int it = 0; it < iterations; ++it) {
     {
-      const int nthr = stream_block_threads(L);
-      const int Tp = ((T + kStreamChunk - 1) / kStreamChunk) * kStreamChunk;
+      const int Tp = ((T_max + kStreamChunk - 1) / kStreamChunk) * kStreamChunk;
       const size_t smem = kHotBytes + sizeof(float) * 3 * (Tp + nthr);
       cudaError_t e;
       switch (inst) {
-        case kSfOmniDefault: e = launch_stream_batch_instance<kSfOmniDefault, true>(L, jobs, n, nthr, smem); break;
-        case kSfOmniDefaultFp: e = launch_stream_batch_instance<kSfOmniDefaultFp, true>(L, jobs, n, nthr, smem); break;
-        case kSfObstaclesFp: e = launch_stream_batch_instance<kSfObstaclesFp, true>(L, jobs, n, nthr, smem); break;
-        default: e = launch_stream_batch_instance<SF_ALL, false>(L, jobs, n, nthr, smem); break;
+        case kSfOmniDefault: e = launch_stream_batch_instance<kSfOmniDefault, true>(L, jobs, n, rollout_grid, nthr, smem); break;
+        case kSfOmniDefaultFp: e = launch_stream_batch_instance<kSfOmniDefaultFp, true>(L, jobs, n, rollout_grid, nthr, smem); break;
+        case kSfObstaclesFp: e = launch_stream_batch_instance<kSfObstaclesFp, true>(L, jobs, n, rollout_grid, nthr, smem); break;
+        default: e = launch_stream_batch_instance<SF_ALL, false>(L, jobs, n, rollout_grid, nthr, smem); break;
       }
       CUDA_TRY(L, e);
     }
     {
       // iteration > 0: the costs accumulate onto the previous iteration's (quirk R20)
-      const int grid = std::min((B + kUpdThreads - 1) / kUpdThreads, 148 * 8);
-      path_costs_tm_batch_kernel<<<dim3(grid, n), kUpdThreads, k3_common_smem_bytes(), L->stream>>>(jobs, it);
+      path_costs_tm_batch_kernel<<<dim3(cost_grid, n), kUpdThreads, k3_common_smem_bytes(), L->stream>>>(jobs, it);
       CUDA_TRY(L, cudaGetLastError());
     }
-    const int chunks = (B + kWsChunk - 1) / kWsChunk;
     {
-      const int gy = weighted_sums_row_groups(T, chunks * n);   // the rows are split less when many robots fill the machine
-      weighted_sums_tm_batch_kernel<<<dim3(chunks, gy, n), kWsThreads, 0, L->stream>>>(jobs);
+      const int gy = weighted_sums_row_groups(T_max, ws_total);   // the rows are split less when many robots fill the machine
+      weighted_sums_tm_batch_kernel<<<dim3(ws_grid, gy, n), kWsThreads, 0, L->stream>>>(jobs);
       CUDA_TRY(L, cudaGetLastError());
     }
     const bool final_it = it + 1 == iterations;
     {
-      const int merge_grid = (T + kMergeT - 1) / kMergeT;
-      merge_finalize_batch_kernel<<<dim3(merge_grid, n), kUpdThreads, 0, L->stream>>>(jobs, chunks, 3 * T + 2, tag, final_it ? 1 : 0);
+      merge_finalize_batch_kernel<<<dim3(merge_grid, n), kUpdThreads, 0, L->stream>>>(jobs, tag, final_it ? 1 : 0);
       CUDA_TRY(L, cudaGetLastError());
     }
     L->launches += 4;
@@ -2184,7 +2204,7 @@ mppi_status mppi_get_control_history(mppi_handle * h, float hist12[12])
   return MPPI_OK;
 }
 
-// Multi-robot server: bind n handles of one device (same batch_size / time_steps, not sharded) into a group.  They
+// Multi-robot server: bind n handles of one device (any batch_size / time_steps, not sharded) into a group.  They
 // move to the stream layout and share the first handle's stream from here on, and mppi_optimize_batch[_resident] over
 // exactly this group (same order) runs as four kernel launches per iteration per chunk of up to 64 robots, plus the
 // regenerate_noises redraws.  Everything else keeps working on bound handles.
@@ -2195,7 +2215,7 @@ mppi_status mppi_batch_bind(mppi_handle ** hs, int32_t n)
   for (int i = 0; i < n; ++i) {
     mppi_handle * h = hs[i];
     if (!h) {return MPPI_E_CONFIG;}
-    if (h->device != L->device || h->B != L->B || h->T != L->T) {return fail(L, MPPI_E_CONFIG, "mppi_batch_bind: handles must share device, batch_size and time_steps");}
+    if (h->device != L->device) {return fail(L, MPPI_E_CONFIG, "mppi_batch_bind: handles must share one device");}
     if (h->nranks > 1) {return fail(L, MPPI_E_CONFIG, "mppi_batch_bind: unsharded handles only");}
     for (int k = 0; k < i; ++k) {if (hs[k] == h) {return fail(L, MPPI_E_CONFIG, "mppi_batch_bind: duplicate handle");}}
   }
@@ -2246,6 +2266,7 @@ mppi_status mppi_batch_bind(mppi_handle ** hs, int32_t n)
     j.sx = h->cfg.vx_std; j.sy = h->cfg.vy_std; j.sw = h->cfg.wz_std;
     j.holonomic = holonomic(h) ? 1 : 0;
     noise_jobs.push_back(j);
+    L->noise_items.push_back(static_cast<long long>(h->B) * ((h->T + 3) / 4));
   }
   if (!noise_jobs.empty()) {
     const size_t bytes = sizeof(NoiseJob) * noise_jobs.size();

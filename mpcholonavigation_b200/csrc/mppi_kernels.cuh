@@ -963,14 +963,17 @@ static_assert(kStreamChunk <= kNoisePadRows, "prefetch reads up to kStreamChunk 
 
 // kExact: the mask IS the set of active features (no runtime flag tests inside the loop); otherwise the mask is an
 // upper bound and every feature is still gated by its per-cycle runtime flag (generic instance).
+// nblocks: a block at or beyond it returns at once (a robot-group member in a launch sized for a larger member); the
+// check sits behind the PDL trigger, where it leaves the kernel's register allocation as it is without it
 template<unsigned F, bool kExact>
 __device__ __forceinline__ void rollout_score_stream_body(
-  const DevParams * __restrict__ P, const uint8_t * __restrict__ cm, const DevBuffers & bufs)
+  const DevParams * __restrict__ P, const uint8_t * __restrict__ cm, const DevBuffers & bufs, int nblocks = 0x7fffffff)
 {
   extern __shared__ float smem[];
   const int tid = threadIdx.x;
   const int nthr = blockDim.x;
   pdl_launch_dependents();   // the path-cost kernel behind this one may stage its tables while this grid drains
+  if (static_cast<int>(blockIdx.x) >= nblocks) {return;}
   float * s_hot = smem;
   load_hot_params(s_hot, P, tid, nthr);
   __syncthreads();
@@ -1949,7 +1952,10 @@ __device__ __forceinline__ void k3_publish_flags(const DevParams * P, DevState *
 // SM oversubscribed, 5 (96 registers) below that (measured on B200, profiles/).
 // bump_epoch: the last block also advances the handle's packet epoch, so that the merge kernel behind this one can tag the
 // result packets it writes to pinned host memory (stream layout, unsharded: no copy node, no stream synchronisation)
-__device__ __forceinline__ void path_costs_tm_body(const DevParams * __restrict__ Pg, const DevBuffers & bufs, int iteration, int bump_epoch = 0)
+// nblocks: the blocks that work on this problem (blockIdx.x < nblocks), i.e. its grid stride, ticket count and number of
+// partial minima; gridDim.x for one handle, the member's own count in a group launched at the largest member's extent
+__device__ __forceinline__ void path_costs_tm_body(const DevParams * __restrict__ Pg, const DevBuffers & bufs, int iteration, int bump_epoch,
+  unsigned nblocks)
 {
   extern __shared__ float smem[];
   __shared__ K3Decisions dec;
@@ -1984,12 +1990,12 @@ __device__ __forceinline__ void path_costs_tm_body(const DevParams * __restrict_
     // points per metre of the path: the start of the per-sample search in the arc-length prefix (efficiency only)
     const float d_all = path.s_D[max(P->N - 1, 0)];
     const float inv_h = d_all > 0.0f ? static_cast<float>(P->N - 1) / d_all : 0.0f;
-    for (int base = blockIdx.x * kUpdThreads; base < B; base += gridDim.x * kUpdThreads) {
+    for (int base = blockIdx.x * kUpdThreads; base < B; base += nblocks * kUpdThreads) {
       const int b = base + tid;
       if (b < B) {m = fminf(m, k3_trajectory_total_fast(b, P, dec, path, bufs, iteration, src_w, inv_h));}
     }
   } else {
-    for (int base = blockIdx.x * kUpdThreads; base < B; base += gridDim.x * kUpdThreads) {
+    for (int base = blockIdx.x * kUpdThreads; base < B; base += nblocks * kUpdThreads) {
       const int b = base + tid;
       if (b < B) {m = fminf(m, k3_trajectory_total_general(b, P, dec, path, bufs, iteration));}
     }
@@ -2003,13 +2009,13 @@ __device__ __forceinline__ void path_costs_tm_body(const DevParams * __restrict_
     for (int w = 1; w < kUpdThreads / 32; ++w) {m = fminf(m, s_red[w]);}
     bufs.partials[static_cast<size_t>(blockIdx.x) * stride] = m;
     __threadfence();
-    sc_last = atomicAdd(&bufs.st->ticket, 1u) == gridDim.x - 1 ? 1u : 0u;
+    sc_last = atomicAdd(&bufs.st->ticket, 1u) == nblocks - 1 ? 1u : 0u;
   }
   __syncthreads();
   if (!sc_last) {return;}
   __threadfence();
   float gm = 3.402823466e+38f;
-  for (int i = tid; i < static_cast<int>(gridDim.x); i += kUpdThreads) {gm = fminf(gm, bufs.partials[static_cast<size_t>(i) * stride]);}
+  for (int i = tid; i < static_cast<int>(nblocks); i += kUpdThreads) {gm = fminf(gm, bufs.partials[static_cast<size_t>(i) * stride]);}
   gm = warp_min(gm);
   __syncthreads();
   if ((tid & 31) == 0) {s_red[tid >> 5] = gm;}
@@ -2027,7 +2033,7 @@ template<int kMinBlocks>
 __global__ void __launch_bounds__(kUpdThreads, kMinBlocks) path_costs_tm_kernel(
   const DevParams * __restrict__ Pg, const __grid_constant__ DevBuffers bufs, int iteration, int bump_epoch)
 {
-  path_costs_tm_body(Pg, bufs, iteration, bump_epoch);
+  path_costs_tm_body(Pg, bufs, iteration, bump_epoch, gridDim.x);
 }
 
 // K3, tile layout (small and medium batches; latency matters more than throughput here).  One block owns
@@ -3437,14 +3443,22 @@ __global__ void optimized_trajectory_kernel(const float * __restrict__ cs, float
 // Multi-robot groups in the stream layout (BASELINE configs[4]): the four kernels of the large-batch path, launched
 // ONCE for all robots of a group; the robot is the last grid dimension and its buffers come from the job table.
 // Robots are independent problems (own record, costmap, noise, control sequence, state), so nothing else changes.
+// Members may differ in batch_size and time_steps: each launch spans the largest member's extent in every grid dimension,
+// and a block beyond its own member's extent returns before it touches anything (its partial records, its ticket).
 // ---------------------------------------------------------------------------------------------------
-// one robot of a group: where its record, costmap, buffers and pinned result packets are
+// one robot of a group: where its record, costmap, buffers and pinned result packets are, and its launch extents (set by
+// the host with the rules of the single-handle launches for this member's B and T)
 struct __align__(16) FusedJob
 {
   const DevParams * Pg;
   const uint8_t * cm;
   DevBuffers bufs;
   uint2 * host_res;
+  int rollout_blocks;   // blocks of the rollout at the launch's block size
+  int cost_blocks;      // path-cost blocks == partial minima (d_partials holds upd_blocks >= this many records)
+  int ws_chunks;        // weighted-sums chunks == partial records the merge reads
+  int merge_blocks;     // merge blocks (kMergeT steps each)
+  int stride;           // floats per partial record, 3T + 2
 };
 static_assert(sizeof(FusedJob) % 16 == 0, "the job table is an array of 16-byte aligned records");
 
@@ -3452,26 +3466,31 @@ template<unsigned F, bool kExact>
 __global__ void __launch_bounds__(kStreamThreads, MPPI_STREAM_MIN_BLOCKS) rollout_score_stream_batch_kernel(const FusedJob * __restrict__ jobs)
 {
   const FusedJob & j = jobs[blockIdx.y];
-  rollout_score_stream_body<F, kExact>(j.Pg, j.cm, j.bufs);
+  rollout_score_stream_body<F, kExact>(j.Pg, j.cm, j.bufs, j.rollout_blocks);
 }
 
 __global__ void __launch_bounds__(kUpdThreads, 5) path_costs_tm_batch_kernel(const FusedJob * __restrict__ jobs, int iteration)
 {
   const FusedJob & j = jobs[blockIdx.y];
-  path_costs_tm_body(j.Pg, j.bufs, iteration);
+  if (static_cast<int>(blockIdx.x) >= j.cost_blocks) {return;}
+  path_costs_tm_body(j.Pg, j.bufs, iteration, 0, static_cast<unsigned>(j.cost_blocks));
 }
 
+// blockIdx.y splits the member's 3T rows over gridDim.y groups: with a smaller T than the launch's, the trailing groups
+// have no rows and only the first writes the record's [m, s]
 __global__ void __launch_bounds__(kWsThreads) weighted_sums_tm_batch_kernel(const FusedJob * __restrict__ jobs)
 {
   const FusedJob & j = jobs[blockIdx.z];
+  if (static_cast<int>(blockIdx.x) >= j.ws_chunks) {return;}
   weighted_sums_tm_body(j.Pg, j.bufs);
 }
 
 // deliver = 0: an earlier iteration of a multi-iteration cycle, which only updates the control sequence
-__global__ void __launch_bounds__(kUpdThreads) merge_finalize_batch_kernel(const FusedJob * __restrict__ jobs, int n_parts, int stride, unsigned tag, int deliver)
+__global__ void __launch_bounds__(kUpdThreads) merge_finalize_batch_kernel(const FusedJob * __restrict__ jobs, unsigned tag, int deliver)
 {
   const FusedJob & j = jobs[blockIdx.y];
-  merge_finalize_body(j.Pg, j.bufs.partials, n_parts, stride, j.bufs, 1, nullptr, deliver ? j.host_res : nullptr, tag);
+  if (static_cast<int>(blockIdx.x) >= j.merge_blocks) {return;}
+  merge_finalize_body(j.Pg, j.bufs.partials, j.ws_chunks, j.stride, j.bufs, 1, nullptr, deliver ? j.host_res : nullptr, tag);
 }
 
 }  // namespace mppi

@@ -13,7 +13,8 @@
  *  - all [B,T] planes are float32, row-major (b major, t minor), exactly the xtensor layout of the
  *    reference (models/state.hpp:30-56); [T] and [N] vectors are float32;
  *  - the caller owns every input buffer for the duration of the call only; the library copies what it
- *    needs (pinned staging + async copies) before returning;
+ *    needs (pinned staging + async copies) before returning (a device-resident costmap is read in place, see
+ *    mppi_set_costmap_residency);
  *  - a handle is externally synchronised and non-re-entrant (the reference holds the parameter and
  *    costmap mutexes around evalControl, src/controller.cpp:94-103); distinct handles are independent;
  *  - there is NO CPU fallback: if no CUDA device is usable the calls fail with MPPI_E_CUDA.
@@ -136,7 +137,8 @@ typedef struct mppi_robot_desc {
 /* Costmap2D view for one cycle. ref: nav2_costmap_2d::Costmap2D (getCharMap, getSizeInCellsX/Y,
  * getResolution, getOriginX/Y), read under the costmap mutex at controller.cpp:99-100. */
 typedef struct mppi_costmap {
-  const uint8_t * cells;     /* size_y rows of size_x bytes; index = my * size_x + mx */
+  const uint8_t * cells;     /* size_y rows of size_x bytes; index = my * size_x + mx.  Host memory, or device memory
+                                of the handle's device after mppi_set_costmap_residency(h, MPPI_COSTMAP_DEVICE) */
   uint32_t size_x, size_y;
   double resolution;
   double origin_x, origin_y;
@@ -202,10 +204,33 @@ mppi_status mppi_get_control_sequence(mppi_handle * h, float * vx, float * vy, f
 /* ref: Optimizer::shiftControlSequence optimizer.cpp:206-225 */
 mppi_status mppi_shift_control_sequence(mppi_handle * h);
 
+/* ---- where the cycle's costmap lives ---- */
+/* MPPI_COSTMAP_HOST (default): costmap.cells of every cycle entry point is host memory; the library stages and copies it.
+ * MPPI_COSTMAP_DEVICE: costmap.cells is device memory of the handle's device (a GPU costmap producer, a map shared by a
+ * fleet); the map is read in place, never copied, and the path-validity tables that depend on it are made on the device.
+ * Applies to mppi_optimize, mppi_eval_control, mppi_upload_cycle (+ mppi_optimize_resident), mppi_optimize_batch[_resident]
+ * (bound or not; members choose independently and may share one map) and mppi_optimize_sharded (every handle must be on
+ * the map's device).  The geometry fields keep their meaning.  Contract:
+ *  - the map's contents are complete before the call (the library does not wait on the caller's streams);
+ *  - the map stays unchanged until the call that consumes it returns: for mppi_upload_cycle, the mppi_optimize_resident
+ *    that follows;
+ *  - nothing reads the map after that call returns (the regenerate_noises redraw behind the result does not);
+ *  - the pointer may differ in every cycle.
+ * The pointer is checked before anything is enqueued: host, managed or another device's memory, or an allocation smaller
+ * than size_x * size_y, fails with MPPI_E_CONFIG.  The last pointer that passed is remembered and not checked again while
+ * the map's size does not grow: an address that is freed and handed out again must not come back with an allocation
+ * smaller than the map (mppi_set_costmap_residency forgets the remembered pointer).  A failed mppi_upload_cycle in device
+ * mode leaves nothing to run: mppi_optimize_resident then fails with MPPI_E_STATE.  mppi_optimize_sharded needs every
+ * shard in the same residency.  mppi_integrate_state_velocities keeps working (it needs no map);
+ * mppi_score_trajectories takes host maps only and fails with MPPI_E_CONFIG in device mode. */
+#define MPPI_COSTMAP_HOST 0
+#define MPPI_COSTMAP_DEVICE 1
+mppi_status mppi_set_costmap_residency(mppi_handle * h, int32_t residency);
+
 /* ---- the hot path ---- */
 /* prepare() + optimize() (optimizer.cpp:141-145 without the fallback loop, which stays in the host
  * mirror because it throws): costs are zeroed, then iteration_count x {noised rollout, critics,
- * softmax update}.  Host buffers in, host buffers out. */
+ * softmax update}.  Host buffers in (the costmap may be device memory: mppi_set_costmap_residency), host buffers out. */
 mppi_status mppi_optimize(mppi_handle * h, const mppi_cycle_in * in, mppi_cycle_out * out);
 /* Optimizer::evalControl (optimizer.cpp:134-155) for one attempt: prepare() + optimize() and, if fail_flag stayed clear,
  * utils::savitskyGolayFilter (utils.hpp:442-605), getControlFromSequenceAsTwist (optimizer.cpp:396-410) and, when
@@ -223,7 +248,9 @@ mppi_status mppi_get_control_history(mppi_handle * h, float hist12[12]);
 mppi_status mppi_optimize_batch(mppi_handle ** hs, const mppi_cycle_in * ins, mppi_cycle_out * outs, int32_t n);
 /* Multi-robot server (BASELINE configs[4]): bind n unsharded handles of ONE device into a group.  Members may differ in
  * batch_size and time_steps (robot types with their own horizon; a handle re-created after a parameter change binds
- * back with the others).  The members move to the stream layout and share the first handle's stream from then on, and
+ * back with the others).  A host-resident costmap travels in the member's slice of the group's upload buffer (at least
+ * 64 KB, or the largest member's staging capacity at bind time); a device-resident one (mppi_set_costmap_residency) stays
+ * where it is, whatever its size, and several members may point at the same map.  The members move to the stream layout and share the first handle's stream from then on, and
  * mppi_optimize_batch[_resident] over exactly this group, in this order, runs in chunks of up to 64 robots: each chunk is
  * one strided upload plus four kernel launches per iteration, each launch sized for the chunk's largest member.  Members
  * with regenerate_noises redraw their noise in
@@ -240,7 +267,8 @@ mppi_status mppi_optimize_batch_resident(mppi_handle ** handles, mppi_cycle_out 
 mppi_status mppi_batch_span_ms(mppi_handle ** handles, int32_t n, float * ms_out);
 
 /* Split-phase form for data already resident on the device (bench "value" leg, CUDA-graph replay):
- * upload once, then run the device part only. */
+ * upload once, then run the device part only.  A device-resident costmap is read by mppi_optimize_resident: it must stay
+ * unchanged until that call returns. */
 mppi_status mppi_upload_cycle(mppi_handle * h, const mppi_cycle_in * in);
 mppi_status mppi_optimize_resident(mppi_handle * h, mppi_cycle_out * out);
 
@@ -303,8 +331,8 @@ mppi_status mppi_get_profile(mppi_handle * h, float ms_out[4], uint64_t * kernel
                              uint64_t * h2d_bytes, uint64_t * d2h_bytes);
 
 /* ---- sharding over GPUs (SURVEY 8e) ---- */
-/* single process: n handles (one per shard, cfg.shard_offset / shard_total set, any mix of devices) solve ONE
- * problem; the two tiny exchanges (furthest path point + survivor flags; softmax partials) go through pinned
+/* single process: n handles (one per shard, cfg.shard_offset / shard_total set, any mix of devices; with a device-resident
+ * costmap every handle on the map's device) solve ONE problem; the two tiny exchanges (furthest path point + survivor flags; softmax partials) go through pinned
  * host memory.  Every handle ends with the same control sequence; `out` is filled from hs[0]. */
 mppi_status mppi_optimize_sharded(mppi_handle ** hs, int32_t n, const mppi_cycle_in * in, mppi_cycle_out * out);
 /* one process per GPU: one handle per rank, the same exchanges as one ncclAllReduce(MAX) and one ncclAllGather */

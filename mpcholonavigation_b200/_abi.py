@@ -40,6 +40,7 @@ IPC_HANDLE_BYTES = 64
 UINT32_MAX = 0xFFFFFFFF
 
 WANT_TRAJECTORIES, WANT_CELLS, WANT_CRITIC_COSTS = 1, 2, 4
+COSTMAP_HOST, COSTMAP_DEVICE = 0, 1
 
 f32p = C.POINTER(C.c_float)
 i32p = C.POINTER(C.c_int32)
@@ -201,6 +202,7 @@ PRODUCT_ONLY = {
     "get_visualization": (C.c_int, [H, f32p, f32p]),
     "set_profiling": (C.c_int, [H, C.c_int32]),
     "set_timing": (C.c_int, [H, C.c_int32]),
+    "set_costmap_residency": (C.c_int, [H, C.c_int32]),
     "register_costmap_memory": (C.c_int, [H, C.c_void_p, C.c_uint64]),
     "unregister_costmap_memory": (C.c_int, [H, C.c_void_p]),
     "get_profile": (C.c_int, [H, f32p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),

@@ -44,6 +44,22 @@ def _p(a):
     return a.ctypes.data_as(abi.f32p)
 
 
+def _torch():
+    import torch
+    return torch
+
+
+def _is_cuda_tensor(a):
+    return getattr(a, "is_cuda", False) and hasattr(a, "data_ptr")
+
+
+def _sync_device_costmap(cm):
+    """The library reads a device costmap without waiting on any stream: the writes torch has queued to it on the
+    current stream must be complete before the call."""
+    if _is_cuda_tensor(cm):
+        _torch().cuda.current_stream(cm.device).synchronize()
+
+
 @dataclass
 class Cycle:
     """Inputs of one Optimizer::evalControl (optimizer.cpp:134-141)."""
@@ -54,7 +70,9 @@ class Cycle:
     path_x: np.ndarray = field(default_factory=lambda: np.zeros(1, np.float32))
     path_y: np.ndarray = field(default_factory=lambda: np.zeros(1, np.float32))
     path_yaw: np.ndarray = field(default_factory=lambda: np.zeros(1, np.float32))
-    costmap: np.ndarray = field(default_factory=lambda: np.zeros((50, 50), np.uint8))  # [size_y, size_x]
+    # [size_y, size_x] uint8: a numpy array, or a contiguous CUDA torch tensor for an engine in device-costmap mode
+    # (Engine.set_costmap_residency(True))
+    costmap: np.ndarray = field(default_factory=lambda: np.zeros((50, 50), np.uint8))
     resolution: float = 0.1
     origin: Sequence[float] = (0.0, 0.0)
 
@@ -69,11 +87,20 @@ class Cycle:
         """-> (CycleIn, keepalive list)"""
         cached = getattr(self, "_packed", None)
         if cached is not None:
+            _sync_device_costmap(self.costmap)
             return cached
         px, py, pyaw = _f32(self.path_x), _f32(self.path_y), _f32(self.path_yaw)
         assert px.shape == py.shape == pyaw.shape and px.ndim == 1
-        cm = np.ascontiguousarray(self.costmap, dtype=np.uint8)
-        assert cm.ndim == 2
+        if _is_cuda_tensor(self.costmap):
+            cm = self.costmap
+            if cm.dtype != _torch().uint8 or cm.dim() != 2 or not cm.is_contiguous():
+                raise ValueError("a device costmap must be a contiguous 2-D uint8 CUDA tensor")
+            cells = C.cast(C.c_void_p(cm.data_ptr()), abi.u8p)
+            _sync_device_costmap(cm)
+        else:
+            cm = np.ascontiguousarray(self.costmap, dtype=np.uint8)
+            assert cm.ndim == 2
+            cells = cm.ctypes.data_as(abi.u8p)
         cin = abi.CycleIn()
         cin.pose_x, cin.pose_y, cin.pose_yaw = (float(v) for v in self.pose)
         cin.speed_vx, cin.speed_vy, cin.speed_wz = (float(v) for v in self.speed)
@@ -81,7 +108,7 @@ class Cycle:
         cin.goal_checker_xy_tolerance = float(self.goal_checker_xy_tolerance)
         cin.path_size = px.shape[0]
         cin.path_x, cin.path_y, cin.path_yaw = _p(px), _p(py), _p(pyaw)
-        cin.costmap.cells = cm.ctypes.data_as(abi.u8p)
+        cin.costmap.cells = cells
         cin.costmap.size_y, cin.costmap.size_x = cm.shape
         cin.costmap.resolution = float(self.resolution)
         cin.costmap.origin_x, cin.costmap.origin_y = (float(v) for v in self.origin)
@@ -305,6 +332,11 @@ class Engine:
 
     def unregister_costmap_memory(self, array):
         self._check(self.f["unregister_costmap_memory"](self.h, array.ctypes.data))
+
+    def set_costmap_residency(self, device: bool):
+        """device=True: the costmap of every cycle is a CUDA tensor on this engine's device, read in place by the kernels
+        (no host copy, no upload); False: numpy arrays in host memory (the default)."""
+        self._check(self.f["set_costmap_residency"](self.h, abi.COSTMAP_DEVICE if device else abi.COSTMAP_HOST))
 
     def set_timing(self, enable=True):
         """device_ms of every cycle (two event records + a read-back per call); off: device_ms reads 0"""

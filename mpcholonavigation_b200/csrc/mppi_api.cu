@@ -150,6 +150,10 @@ struct mppi_handle
   // device straight from the caller's buffer, without the staging memcpy
   std::vector<std::pair<const char *, size_t>> pinned_ranges;
   const uint8_t * costmap_direct{nullptr};   // this cycle's costmap source when it is copied directly
+  // mppi_set_costmap_residency(MPPI_COSTMAP_DEVICE): the cycle entry points read costmap.cells in place in device memory
+  bool costmap_device{false};
+  const void * cm_checked{nullptr};          // the last device costmap that passed check_device_costmap ...
+  size_t cm_checked_bytes{0};                // ... and its size
   uint64_t host_ns[8]{0, 0, 0, 0, 0, 0, 0, 0};   // host-side time of the steady-state call by phase (mppi_debug_get_host_ns)
   bool zero_copy_enabled{true};   // MPPI_ZERO_COPY=0 disables
   bool fused_enabled{true};    // small batches: one cooperative launch per iteration (tile_fused_kernel); MPPI_FUSED=0 disables
@@ -300,10 +304,17 @@ void set_common(CriticCommon & c, const mppi_critic_desc * d, int idx, bool gate
   c.weight = d ? d->cost_weight : 0.0f;
 }
 
+mppi_status check_device_costmap(mppi_handle * h, const mppi_costmap & cm);
+
 // Fill the per-cycle record.  `in` may be null for integrate-only calls (mode 1).
 mppi_status build_params(mppi_handle * h, const mppi_cycle_in * in, int mode, unsigned preset_furthest, bool critics_active,
   const float * first_pose = nullptr)
 {
+  if (h->costmap_device && mode == 0) {
+    // a device map is checked before the record (or h->last, which a group's launch takes the map pointer from) sees it
+    const mppi_status c = check_device_costmap(h, in->costmap);
+    if (c != MPPI_OK) {return c;}
+  }
   DevParams & p = *reinterpret_cast<DevParams *>(h->h_params);
   std::memset(&p, 0, sizeof(p));
   const mppi_config & cfg = h->cfg;
@@ -366,7 +377,10 @@ mppi_status build_params(mppi_handle * h, const mppi_cycle_in * in, int mode, un
     const float curr_dist = sqrtf(dx * dx + dy * dy);
     D[i] = D[i - 1] + curr_dist;
   }
-  // host-made tables behind the path arrays: valid[n16] | flags[n16] | follow_idx[N] (uint16); see DevParams
+  // tables behind the path arrays: valid[n16] | flags[n16] | follow_idx[N] (uint16); see DevParams.  With a device-resident
+  // costmap the host writes only the PathAngle bit of the flags: path_tables_kernel makes the rest on the device.
+  const bool dev_map = h->costmap_device && mode == 0;
+  p.cm_dev = dev_map ? in->costmap.cells : nullptr;
   const int n16 = ((N + 15) / 16) * 16;
   uint8_t * valid = reinterpret_cast<uint8_t *>(tail + 4 * N);
   uint8_t * flags = valid + n16;
@@ -385,20 +399,10 @@ mppi_status build_params(mppi_handle * h, const mppi_cycle_in * in, int mode, un
   }
   // utils::findPathCosts (utils.hpp:361-394): validity of every path point but the last, against the costmap the
   // caller holds for this cycle; prefix counts of the invalid ones for PathAlign's occupancy gate
-  for (int j = 0; j < N; ++j) {
+  for (int j = 0; j < N && !dev_map; ++j) {
     bool ok = false;
     if (j < N - 1 && in->costmap.cells) {
-      const double wx = in->path_x[j], wy = in->path_y[j];
-      if (!(wx < p.ox || wy < p.oy)) {
-        const double qx = (wx - p.ox) / p.res, qy = (wy - p.oy) / p.res;
-        if (qx < static_cast<double>(p.size_x) && qy < static_cast<double>(p.size_y)) {
-          const unsigned mx = static_cast<unsigned>(qx), my = static_cast<unsigned>(qy);
-          if (mx < p.size_x && my < p.size_y) {
-            const int c = in->costmap.cells[static_cast<size_t>(my) * p.size_x + mx];
-            ok = !(c == LETHAL_OBSTACLE || c == INSCRIBED_INFLATED_OBSTACLE || (c == NO_INFORMATION && !h->robot.track_unknown));
-          }
-        }
-      }
+      ok = path_point_valid(in->costmap.cells, p.size_x, p.size_y, p.res, p.ox, p.oy, h->robot.track_unknown, in->path_x[j], in->path_y[j]);
     }
     valid[j] = ok ? 1 : 0;
     invalid_before[j + 1] = static_cast<uint16_t>(invalid_before[j] + (ok ? 0 : 1));
@@ -618,24 +622,12 @@ mppi_status build_params(mppi_handle * h, const mppi_cycle_in * in, int mode, un
     std::vector<int> & next_valid = h->scratch_next;
     next_valid.assign(N + 1, N);
     for (int i = N - 1; i >= 0; --i) {next_valid[i] = valid[i] ? i : next_valid[i + 1];}
-    const int path_size = N - 1;
-    auto align_gate = [&](int f, int offset, float max_ratio) -> bool {
-        if (f < offset) {return false;}
-        const int closest = p.closest_path_pt;
-        const float range = static_cast<float>(static_cast<long long>(f) - closest);
-        unsigned invalid_ctr = 0;
-        if (f > closest) {invalid_ctr = static_cast<unsigned>(invalid_before[f]) - static_cast<unsigned>(invalid_before[closest]);}
-        // the reference bails out of its counting loop as soon as ctr / range > ratio with ctr > 2; the count only
-        // grows and the range is fixed, so the final count decides
-        return !(invalid_ctr > 2 && static_cast<float>(invalid_ctr) / range > max_ratio);
-      };
     for (int f = 0; f < N; ++f) {
-      int fidx = std::min(f + p.follow_offset, path_size);
-      if (fidx < path_size - 1) {fidx = std::min(next_valid[fidx], path_size - 1);}
-      follow_tab[f] = static_cast<uint16_t>(std::max(fidx, 0));
       unsigned fl = 0;
-      if (align_gate(f, p.align_offset, p.align_max_ratio) && f > 0) {fl |= 1u;}
-      if (align_gate(f, p.legacy_offset, p.legacy_max_ratio) && (N - 1) >= 1) {fl |= 2u;}
+      if (!dev_map) {
+        follow_tab[f] = static_cast<uint16_t>(path_follow_index(f, p.follow_offset, N, next_valid.data()));
+        fl = path_align_flag_bits(p, f, invalid_before.data());
+      }
       if (gate[std::min(f + p.angle_offset, N - 1)]) {fl |= 4u;}
       flags[f] = static_cast<uint8_t>(fl);
     }
@@ -781,6 +773,90 @@ mppi_status stage_costmap(mppi_handle * h, const mppi_costmap & cm)
   return MPPI_OK;
 }
 
+// The caller's device-resident costmap: device memory of this handle's device (not managed, not host, not another GPU's),
+// size_x * size_y bytes inside one allocation.  Checked before anything of the cycle is enqueued; a kernel never sees a
+// pointer that did not pass.  The last pointer that passed is remembered (a producer usually hands over the same buffer).
+mppi_status check_device_costmap_impl(mppi_handle * h, const mppi_costmap & cm)
+{
+  const size_t bytes = static_cast<size_t>(cm.size_x) * cm.size_y;
+  if (bytes == 0 || !cm.cells) {return fail(h, MPPI_E_CONFIG, "empty costmap");}
+  if (!(cm.resolution > 0.0)) {return fail(h, MPPI_E_CONFIG, "costmap resolution must be > 0");}
+  if (cm.cells == h->cm_checked && bytes <= h->cm_checked_bytes) {return MPPI_OK;}
+  CUDA_TRY(h, cudaSetDevice(h->device));
+  cudaPointerAttributes a;
+  if (cudaPointerGetAttributes(&a, cm.cells) != cudaSuccess) {
+    cudaGetLastError();
+    return fail(h, MPPI_E_CONFIG, "device costmap: not a CUDA pointer");
+  }
+  if (a.type != cudaMemoryTypeDevice) {
+    return fail(h, MPPI_E_CONFIG, a.type == cudaMemoryTypeManaged ? "device costmap: managed memory is not accepted" :
+      "device costmap: costmap.cells is host memory (MPPI_COSTMAP_DEVICE expects device memory)");
+  }
+  if (a.device != h->device) {
+    return fail(h, MPPI_E_CONFIG, "device costmap: the map is on device " + std::to_string(a.device) + ", the handle on device " +
+      std::to_string(h->device));
+  }
+  // the allocation must hold the whole map (cuMemGetAddressRange, a driver entry point fetched through the runtime)
+  typedef CUresult (*RangeFn)(CUdeviceptr *, size_t *, CUdeviceptr);
+  static RangeFn range_fn = nullptr;
+  if (!range_fn) {
+    void * fn = nullptr;
+    cudaDriverEntryPointQueryResult qres;
+    if (cudaGetDriverEntryPoint("cuMemGetAddressRange", &fn, cudaEnableDefault, &qres) != cudaSuccess || qres != cudaDriverEntryPointSuccess || !fn) {
+      cudaGetLastError();
+      return fail(h, MPPI_E_CUDA, "cuMemGetAddressRange unavailable");
+    }
+    range_fn = reinterpret_cast<RangeFn>(fn);
+  }
+  CUdeviceptr base = 0;
+  size_t size = 0;
+  const CUdeviceptr ptr = reinterpret_cast<CUdeviceptr>(cm.cells);
+  if (range_fn(&base, &size, ptr) != CUDA_SUCCESS || ptr - base + bytes > size) {
+    return fail(h, MPPI_E_CONFIG, "device costmap: size_x * size_y bytes do not fit the allocation behind costmap.cells");
+  }
+  h->cm_checked = cm.cells;
+  h->cm_checked_bytes = bytes;
+  return MPPI_OK;
+}
+
+// a rejected map also ends the resident cycle: mppi_optimize_resident must not replay a record whose map's call is over
+mppi_status check_device_costmap(mppi_handle * h, const mppi_costmap & cm)
+{
+  const mppi_status s = check_device_costmap_impl(h, cm);
+  if (s != MPPI_OK) {h->cycle_uploaded = false;}
+  return s;
+}
+
+// the costmap of a cycle entry point: staged for the upload (host map), or left where it is (device map: build_params
+// checked it and put the pointer into the record, which is the whole upload)
+mppi_status stage_cycle_costmap(mppi_handle * h, const mppi_costmap & cm)
+{
+  if (!h->costmap_device) {return stage_costmap(h, cm);}
+  h->d_costmap = nullptr; h->h_costmap = nullptr;
+  h->costmap_direct = nullptr;
+  h->costmap_bytes = 0;
+  return MPPI_OK;
+}
+
+// every device-mode handle of a multi-handle call checks its map before the first of them enqueues anything
+mppi_status check_device_costmaps(mppi_handle ** hs, const mppi_cycle_in * ins, int n, bool shared_input)
+{
+  for (int i = 0; i < n; ++i) {
+    if (!hs[i] || !hs[i]->costmap_device) {continue;}
+    const mppi_status s = check_device_costmap(hs[i], (shared_input ? ins[0] : ins[i]).costmap);
+    if (s != MPPI_OK) {return s;}
+  }
+  return MPPI_OK;
+}
+
+mppi_status launch_path_tables(mppi_handle * h)
+{
+  path_tables_kernel<<<1, kTablesThreads, 0, h->stream>>>(reinterpret_cast<DevParams *>(h->d_params));
+  CUDA_TRY(h, cudaGetLastError());
+  h->launches++;
+  return MPPI_OK;
+}
+
 // bytes of [record | costmap], contiguous on both sides (stage_costmap)
 size_t upload_bytes(const mppi_handle * h)
 {
@@ -844,14 +920,25 @@ int path_cost_blocks(int B)
   return std::min((B + kUpdThreads - 1) / kUpdThreads, 148 * 8);
 }
 
-template<unsigned F, bool kExact>
+template<unsigned F, bool kExact, bool kDev>
 void launch_stream_instance(mppi_handle * h, int mode)
 {
   const int nthr = stream_block_threads(h->B);
   const int Tp = ((h->T + kStreamChunk - 1) / kStreamChunk) * kStreamChunk;
   const size_t smem = kHotBytes + sizeof(float) * 3 * (Tp + nthr);   // hot record, control sequence, footprint slots
-  rollout_score_stream_kernel<F, kExact><<<(h->B + nthr - 1) / nthr, nthr, smem, h->stream>>>(
+  rollout_score_stream_kernel<F, kExact, kDev><<<(h->B + nthr - 1) / nthr, nthr, smem, h->stream>>>(
     reinterpret_cast<const DevParams *>(h->d_params), h->d_costmap, make_bufs(h, mode));
+}
+
+template<bool kDev>
+void launch_stream_dispatch(mppi_handle * h, int mode)
+{
+  switch (pick_stream_instance(stream_feature_need(h->last))) {
+    case kSfOmniDefault: launch_stream_instance<kSfOmniDefault, true, kDev>(h, mode); break;
+    case kSfOmniDefaultFp: launch_stream_instance<kSfOmniDefaultFp, true, kDev>(h, mode); break;
+    case kSfObstaclesFp: launch_stream_instance<kSfObstaclesFp, true, kDev>(h, mode); break;
+    default: launch_stream_instance<SF_ALL, false, kDev>(h, mode); break;
+  }
 }
 
 mppi_status launch_regenerate(mppi_handle * h);
@@ -906,7 +993,7 @@ bool use_fused(mppi_handle * h)
   return h->fused_fits;
 }
 
-template<unsigned F, bool kExact>
+template<unsigned F, bool kExact, bool kDev>
 cudaError_t launch_fused_instance(mppi_handle * h, int iteration, uint2 * host_res, bool zero_copy, int tail_mode)
 {
   const int S = pick_segments(h);
@@ -922,18 +1009,25 @@ cudaError_t launch_fused_instance(mppi_handle * h, int iteration, uint2 * host_r
   int up_vecs = zero_copy ? static_cast<int>((upload_bytes(h) + 15) / 16) : 0;
   float * hist = h->d_hist;
   void * args[] = {&dp, &cm, &bufs, &B, &T, &N, &iteration, &host_res, &up_host, &up_vecs, &tail_mode, &hist};
-  return cudaLaunchCooperativeKernel(reinterpret_cast<const void *>(&tile_fused_kernel<F, kExact>), grid, block, args, smem, h->stream);
+  return cudaLaunchCooperativeKernel(reinterpret_cast<const void *>(&tile_fused_kernel<F, kExact, kDev>), grid, block, args, smem,
+    h->stream);
+}
+
+template<bool kDev>
+cudaError_t launch_fused_dispatch(mppi_handle * h, int iteration, uint2 * host_res, bool zero_copy, int tail_mode)
+{
+  switch (pick_stream_instance(stream_feature_need(h->last))) {
+    case kSfOmniDefault: return launch_fused_instance<kSfOmniDefault, true, kDev>(h, iteration, host_res, zero_copy, tail_mode);
+    case kSfOmniDefaultFp: return launch_fused_instance<kSfOmniDefaultFp, true, kDev>(h, iteration, host_res, zero_copy, tail_mode);
+    case kSfObstaclesFp: return launch_fused_instance<kSfObstaclesFp, true, kDev>(h, iteration, host_res, zero_copy, tail_mode);
+    default: return launch_fused_instance<SF_ALL, false, kDev>(h, iteration, host_res, zero_copy, tail_mode);
+  }
 }
 
 mppi_status launch_fused(mppi_handle * h, int iteration, uint2 * host_res, bool zero_copy, int tail_mode)
 {
-  cudaError_t e;
-  switch (pick_stream_instance(stream_feature_need(h->last))) {
-    case kSfOmniDefault: e = launch_fused_instance<kSfOmniDefault, true>(h, iteration, host_res, zero_copy, tail_mode); break;
-    case kSfOmniDefaultFp: e = launch_fused_instance<kSfOmniDefaultFp, true>(h, iteration, host_res, zero_copy, tail_mode); break;
-    case kSfObstaclesFp: e = launch_fused_instance<kSfObstaclesFp, true>(h, iteration, host_res, zero_copy, tail_mode); break;
-    default: e = launch_fused_instance<SF_ALL, false>(h, iteration, host_res, zero_copy, tail_mode); break;
-  }
+  const cudaError_t e = h->last.cm_dev ? launch_fused_dispatch<true>(h, iteration, host_res, zero_copy, tail_mode) :
+    launch_fused_dispatch<false>(h, iteration, host_res, zero_copy, tail_mode);
   CUDA_TRY(h, e);
   h->launches++;
   return MPPI_OK;
@@ -941,13 +1035,9 @@ mppi_status launch_fused(mppi_handle * h, int iteration, uint2 * host_res, bool 
 
 mppi_status launch_rollout(mppi_handle * h, int mode)
 {
+  const bool dev_map = mode == 0 && h->last.cm_dev;
   if (mode == 0 && h->stream_layout) {
-    switch (pick_stream_instance(stream_feature_need(h->last))) {
-      case kSfOmniDefault: launch_stream_instance<kSfOmniDefault, true>(h, mode); break;
-      case kSfOmniDefaultFp: launch_stream_instance<kSfOmniDefaultFp, true>(h, mode); break;
-      case kSfObstaclesFp: launch_stream_instance<kSfObstaclesFp, true>(h, mode); break;
-      default: launch_stream_instance<SF_ALL, false>(h, mode); break;
-    }
+    if (dev_map) {launch_stream_dispatch<true>(h, mode);} else {launch_stream_dispatch<false>(h, mode);}
     CUDA_TRY(h, cudaGetLastError());
     h->launches++;
     return MPPI_OK;
@@ -958,20 +1048,20 @@ mppi_status launch_rollout(mppi_handle * h, int mode)
   const dim3 grid((h->B + kTile - 1) / kTile), block(kTile, S);
   const DevParams * dp = reinterpret_cast<const DevParams *>(h->d_params);
   const unsigned inst = mode == 0 ? pick_stream_instance(stream_feature_need(h->last)) : SF_ALL;
-#define MPPI_LAUNCH_TILE(F, EXACT, MODE) \
-  rollout_score_kernel<F, EXACT, MODE><<<grid, block, smem, h->stream>>>(dp, h->d_costmap, make_bufs(h, mode), h->B, h->T)
+#define MPPI_LAUNCH_TILE(F, EXACT, MODE, DEV) \
+  rollout_score_kernel<F, EXACT, MODE, DEV><<<grid, block, smem, h->stream>>>(dp, h->d_costmap, make_bufs(h, mode), h->B, h->T)
   if (mode == 1) {
-    MPPI_LAUNCH_TILE(SF_ALL, false, 1);
+    MPPI_LAUNCH_TILE(SF_ALL, false, 1, false);
   } else if (mode == 2) {
-    MPPI_LAUNCH_TILE(SF_ALL, false, 2);
+    MPPI_LAUNCH_TILE(SF_ALL, false, 2, false);
   } else if (inst == kSfOmniDefault) {
-    MPPI_LAUNCH_TILE(kSfOmniDefault, true, 0);
+    if (dev_map) {MPPI_LAUNCH_TILE(kSfOmniDefault, true, 0, true);} else {MPPI_LAUNCH_TILE(kSfOmniDefault, true, 0, false);}
   } else if (inst == kSfOmniDefaultFp) {
-    MPPI_LAUNCH_TILE(kSfOmniDefaultFp, true, 0);
+    if (dev_map) {MPPI_LAUNCH_TILE(kSfOmniDefaultFp, true, 0, true);} else {MPPI_LAUNCH_TILE(kSfOmniDefaultFp, true, 0, false);}
   } else if (inst == kSfObstaclesFp) {
-    MPPI_LAUNCH_TILE(kSfObstaclesFp, true, 0);
+    if (dev_map) {MPPI_LAUNCH_TILE(kSfObstaclesFp, true, 0, true);} else {MPPI_LAUNCH_TILE(kSfObstaclesFp, true, 0, false);}
   } else {
-    MPPI_LAUNCH_TILE(SF_ALL, false, 0);
+    if (dev_map) {MPPI_LAUNCH_TILE(SF_ALL, false, 0, true);} else {MPPI_LAUNCH_TILE(SF_ALL, false, 0, false);}
   }
 #undef MPPI_LAUNCH_TILE
   CUDA_TRY(h, cudaGetLastError());
@@ -1066,6 +1156,10 @@ mppi_status enqueue_kernels(mppi_handle * h, bool prof)
 {
   const int stride = 3 * h->T + 2;
   const bool fused = use_fused(h);
+  if (h->last.cm_dev) {
+    const mppi_status s = launch_path_tables(h);
+    if (s != MPPI_OK) {return s;}
+  }
   for (int it = 0; it < h->cfg.iteration_count; ++it) {
     if (prof) {CUDA_TRY(h, cudaEventRecord(h->pev[0], h->stream));}
     if (fused) {
@@ -1194,7 +1288,8 @@ mppi_status enqueue_optimize_impl(mppi_handle * h, bool with_upload)
   h->ev_src = nullptr;
   const bool fused_now = use_fused(h);
   h->wait_packets = fused_now || stream_packets(h);
-  h->zero_copy_now = with_upload && fused_now && h->zero_copy_enabled && upload_bytes(h) <= kZeroCopyMaxBytes;
+  // (not with a device-resident costmap: the tiles would copy the record over the tables the tables kernel writes)
+  h->zero_copy_now = with_upload && fused_now && h->zero_copy_enabled && !h->last.cm_dev && upload_bytes(h) <= kZeroCopyMaxBytes;
   if (h->wait_packets) {
     // the fused kernel advances the epoch once per launch, the stream layout once per cycle
     h->fepoch_host += fused_now ? static_cast<uint32_t>(h->cfg.iteration_count) : 1u;
@@ -1625,7 +1720,7 @@ mppi_status batch_stream_launch(mppi_handle * L, mppi_handle ** hs, int c0, int 
     FusedJob & j = L->h_jobs[c0 + i];
     std::memset(&j, 0, sizeof(j));
     j.Pg = reinterpret_cast<const DevParams *>(h->d_params);
-    j.cm = h->d_costmap;
+    j.cm = h->last.cm_dev ? h->last.cm_dev : h->d_costmap;
     j.bufs = make_bufs(h, 0);
     j.host_res = h->h_res;
     j.rollout_blocks = (h->B + nthr - 1) / nthr;
@@ -1651,6 +1746,14 @@ mppi_status batch_stream_launch(mppi_handle * L, mppi_handle ** hs, int c0, int 
     std::memcpy(L->jobs_sent.data() + off, L->h_jobs + c0, bytes);
   }
   const FusedJob * jobs = L->d_jobs + c0;
+  bool any_dev_map = false;
+  for (int i = 0; i < n; ++i) {any_dev_map = any_dev_map || hs[i]->last.cm_dev != nullptr;}
+  if (any_dev_map) {
+    // device-resident maps: the members' path tables, one block per member (host-map members return at once)
+    path_tables_batch_kernel<<<dim3(1, n), kTablesThreads, 0, L->stream>>>(jobs);
+    CUDA_TRY(L, cudaGetLastError());
+    L->launches++;
+  }
   const int iterations = L->cfg.iteration_count;   // shared by every member (batch_stream_ok)
   for (int it = 0; it < iterations; ++it) {
     {
@@ -1697,6 +1800,10 @@ mppi_status batch_run_group(mppi_handle ** hs, const mppi_cycle_in * ins, mppi_c
 {
   mppi_handle * L = hs[0];
   CUDA_TRY(L, cudaSetDevice(L->device));
+  if (ins) {
+    const mppi_status c = check_device_costmaps(hs, ins, n, false);
+    if (c != MPPI_OK) {return c;}
+  }
   mppi_status first = MPPI_OK;
   if (!batch_stream_ok(hs, n)) {
     if (L->timing) {cudaEventRecord(L->ev0, L->stream);}
@@ -1704,7 +1811,7 @@ mppi_status batch_run_group(mppi_handle ** hs, const mppi_cycle_in * ins, mppi_c
       mppi_status f = MPPI_OK;
       if (ins) {
         f = build_params(hs[i], &ins[i], 0, kUnset, true);
-        if (f == MPPI_OK) {f = stage_costmap(hs[i], ins[i].costmap);}
+        if (f == MPPI_OK) {f = stage_cycle_costmap(hs[i], ins[i].costmap);}
         if (f == MPPI_OK) {hs[i]->cycle_uploaded = true;}
       } else if (!hs[i]->cycle_uploaded) {
         f = fail(hs[i], MPPI_E_STATE, "mppi_optimize_batch_resident before mppi_upload_cycle");
@@ -1727,7 +1834,7 @@ mppi_status batch_run_group(mppi_handle ** hs, const mppi_cycle_in * ins, mppi_c
     for (int i = c0; i < c0 + cn && s == MPPI_OK; ++i) {
       if (ins) {
         s = build_params(hs[i], &ins[i], 0, kUnset, true);
-        if (s == MPPI_OK) {s = stage_costmap(hs[i], ins[i].costmap);}
+        if (s == MPPI_OK) {s = stage_cycle_costmap(hs[i], ins[i].costmap);}
         if (s == MPPI_OK) {hs[i]->cycle_uploaded = true;}
       } else if (!hs[i]->cycle_uploaded) {
         s = fail(hs[i], MPPI_E_STATE, "mppi_optimize_batch_resident before mppi_upload_cycle");
@@ -1897,6 +2004,10 @@ mppi_status mppi_create(const mppi_config * cfg, mppi_handle ** out)
     CUDA_TRY(h, cudaFuncSetAttribute(rollout_score_kernel<kSfOmniDefault, true, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
     CUDA_TRY(h, cudaFuncSetAttribute(rollout_score_kernel<kSfOmniDefaultFp, true, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
     CUDA_TRY(h, cudaFuncSetAttribute(rollout_score_kernel<kSfObstaclesFp, true, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+    CUDA_TRY(h, cudaFuncSetAttribute(rollout_score_kernel<SF_ALL, false, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+    CUDA_TRY(h, cudaFuncSetAttribute(rollout_score_kernel<kSfOmniDefault, true, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+    CUDA_TRY(h, cudaFuncSetAttribute(rollout_score_kernel<kSfOmniDefaultFp, true, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+    CUDA_TRY(h, cudaFuncSetAttribute(rollout_score_kernel<kSfObstaclesFp, true, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
   }
   {
     const int big = kFusedSmemMax;   // the kernel also has a little static shared memory
@@ -1904,6 +2015,10 @@ mppi_status mppi_create(const mppi_config * cfg, mppi_handle ** out)
     CUDA_TRY(h, cudaFuncSetAttribute(tile_fused_kernel<kSfOmniDefault, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
     CUDA_TRY(h, cudaFuncSetAttribute(tile_fused_kernel<kSfOmniDefaultFp, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
     CUDA_TRY(h, cudaFuncSetAttribute(tile_fused_kernel<kSfObstaclesFp, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+    CUDA_TRY(h, cudaFuncSetAttribute(tile_fused_kernel<SF_ALL, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+    CUDA_TRY(h, cudaFuncSetAttribute(tile_fused_kernel<kSfOmniDefault, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+    CUDA_TRY(h, cudaFuncSetAttribute(tile_fused_kernel<kSfOmniDefaultFp, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+    CUDA_TRY(h, cudaFuncSetAttribute(tile_fused_kernel<kSfObstaclesFp, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
     int coop = 0;
     CUDA_TRY(h, cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, h->device));
     CUDA_TRY(h, cudaDeviceGetAttribute(&h->num_sms, cudaDevAttrMultiProcessorCount, h->device));
@@ -2124,13 +2239,30 @@ mppi_status mppi_set_outputs(mppi_handle * h, uint32_t want_mask)
   return MPPI_OK;
 }
 
+mppi_status mppi_set_costmap_residency(mppi_handle * h, int32_t residency)
+{
+  if (!h) {return MPPI_E_CONFIG;}
+  if (residency != MPPI_COSTMAP_HOST && residency != MPPI_COSTMAP_DEVICE) {
+    return fail(h, MPPI_E_CONFIG, "residency must be MPPI_COSTMAP_HOST or MPPI_COSTMAP_DEVICE");
+  }
+  CUDA_TRY(h, cudaSetDevice(h->device));
+  CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+  drop_graphs(h);
+  h->costmap_device = residency == MPPI_COSTMAP_DEVICE;
+  h->cm_checked = nullptr; h->cm_checked_bytes = 0;
+  h->cycle_uploaded = false;
+  return MPPI_OK;
+}
+
 mppi_status mppi_upload_cycle(mppi_handle * h, const mppi_cycle_in * in)
 {
   if (!h || !in) {return MPPI_E_CONFIG;}
   CUDA_TRY(h, cudaSetDevice(h->device));
+  // device map: a failed upload leaves nothing to run (the resident record would read a map whose cycle is over)
+  if (h->costmap_device) {h->cycle_uploaded = false;}
   mppi_status s = build_params(h, in, 0, kUnset, true);
   if (s != MPPI_OK) {return s;}
-  if ((s = stage_costmap(h, in->costmap)) != MPPI_OK) {return s;}
+  if ((s = stage_cycle_costmap(h, in->costmap)) != MPPI_OK) {return s;}
   if ((s = enqueue_uploads(h)) != MPPI_OK) {return s;}
   CUDA_TRY(h, cudaStreamSynchronize(h->stream));
   h->cycle_uploaded = true;
@@ -2157,7 +2289,7 @@ static mppi_status optimize_begin(mppi_handle * h, const mppi_cycle_in * in)
   mppi_status s = build_params(h, in, 0, kUnset, true);
   if (s != MPPI_OK) {return s;}
   const uint64_t t_b = now_ns();
-  if ((s = stage_costmap(h, in->costmap)) != MPPI_OK) {return s;}
+  if ((s = stage_cycle_costmap(h, in->costmap)) != MPPI_OK) {return s;}
   h->host_ns[0] += t_b - t_a;
   h->host_ns[1] += now_ns() - t_b;
   h->cycle_uploaded = true;
@@ -2288,7 +2420,8 @@ mppi_status mppi_optimize_batch(mppi_handle ** hs, const mppi_cycle_in * ins, mp
 {
   if (!hs || !ins || n < 0) {return MPPI_E_CONFIG;}
   if (batch_is_group(hs, n)) {return batch_run_group(hs, ins, outs, n);}
-  mppi_status first = MPPI_OK;
+  mppi_status first = check_device_costmaps(hs, ins, n, false);
+  if (first != MPPI_OK) {return first;}
   std::vector<char> launched(n, 0);
   for (int i = 0; i < n; ++i) {
     const mppi_status s = optimize_begin(hs[i], &ins[i]);
@@ -2494,6 +2627,7 @@ mppi_status mppi_score_trajectories(
   const float * y, const float * yaw, float * costs_inout, uint32_t * furthest_inout, int32_t * fail_flag_out)
 {
   if (!h || !in || !vx || !vy || !wz || !x || !y || !yaw || !costs_inout) {return MPPI_E_CONFIG;}
+  if (h->costmap_device) {return fail(h, MPPI_E_CONFIG, "mppi_score_trajectories takes a host costmap: set MPPI_COSTMAP_HOST first");}
   CUDA_TRY(h, cudaSetDevice(h->device));
   mppi_status s = ensure_injection_buffers(h);
   if (s != MPPI_OK) {return s;}
@@ -2604,6 +2738,16 @@ mppi_status mppi_optimize_sharded(mppi_handle ** hs, int32_t n, const mppi_cycle
     }
     if (hs[i]->comm) {return fail(hs[i], MPPI_E_CONFIG, "handle is bound to an NCCL communicator");}
   }
+  for (int i = 1; i < n; ++i) {
+    // the shards read the same costmap.cells: as host memory or as device memory, never both
+    if (hs[i]->costmap_device != hs[0]->costmap_device) {
+      return fail(hs[i], MPPI_E_CONFIG, "mppi_optimize_sharded: the shards must share one costmap residency");
+    }
+  }
+  {
+    const mppi_status c = check_device_costmaps(hs, in, n, true);
+    if (c != MPPI_OK) {return c;}
+  }
   const int T = hs[0]->T, stride = 3 * T + 2;
   const int words = 1 + kMaxCritics;
   std::vector<unsigned> st_host(static_cast<size_t>(n) * words);
@@ -2615,9 +2759,10 @@ mppi_status mppi_optimize_sharded(mppi_handle ** hs, int32_t n, const mppi_cycle
     h->nranks = n;   // K3 must not finalize on its own (restored to 1 on every exit path, below)
     if ((s = ensure_gathered(h, n)) != MPPI_OK) {break;}
     if ((s = build_params(h, in, 0, kUnset, true)) != MPPI_OK) {break;}
-    if ((s = stage_costmap(h, in->costmap)) != MPPI_OK) {break;}
+    if ((s = stage_cycle_costmap(h, in->costmap)) != MPPI_OK) {break;}
     if ((s = enqueue_uploads(h)) != MPPI_OK) {break;}
     cudaEventRecord(h->ev0, h->stream);
+    if (h->last.cm_dev && (s = launch_path_tables(h)) != MPPI_OK) {break;}
   }
   for (int it = 0; it < hs[0]->cfg.iteration_count && s == MPPI_OK; ++it) {
     for (int i = 0; i < n && s == MPPI_OK; ++i) {

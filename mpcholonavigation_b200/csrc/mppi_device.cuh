@@ -3,7 +3,8 @@
 // HBM layout (all owned by one mppi_handle, allocated once at create):
 //   noise_vx/vy/wz   float [B][T] row-major   the reference's layout (models/state.hpp), so that injected
 //                                              noise is a plain copy; read once per kernel, coalesced
-//   costmap          uint8 [size_y][size_x]    uploaded once per cycle with one async copy
+//   costmap          uint8 [size_y][size_x]    uploaded once per cycle with one async copy, or read in place from
+//                                              the caller's device memory (mppi_set_costmap_residency)
 //   DevParams + path one packed record         uploaded once per cycle with one async copy
 //   crit_rows        float [R][B]              per-critic contribution rows + 3 gamma rows (plane-major =
 //                                              coalesced for lane == trajectory)
@@ -94,9 +95,10 @@ struct DevParams
   int noise_tm;                              // noise planes are stored time-major [T][B] (stream layout) instead of [B][T]
   // offsets (in floats) of the path arrays that follow this struct in the same buffer
   int off_path_x, off_path_y, off_path_yaw, off_path_D;
-  // host-made tables behind the path arrays (build_params): valid[n16] (utils::findPathCosts, utils.hpp:361-394),
-  // flags[n16] and follow_idx[N] (uint16), the last two indexed by the furthest reached path point: bit 0 PathAlign
-  // gate, bit 1 PathAlignLegacy gate, bit 2 PathAngle gate; PathFollow's target index
+  // tables behind the path arrays, made by build_params (host map) or path_tables_kernel (device map; bit 2 of the
+  // flags always by the host): valid[n16] (utils::findPathCosts, utils.hpp:361-394), flags[n16] and follow_idx[N]
+  // (uint16), the last two indexed by the furthest reached path point: bit 0 PathAlign gate, bit 1 PathAlignLegacy gate,
+  // bit 2 PathAngle gate; PathFollow's target index
   int obstacle_q[2];                         // list positions of the enabled obstacle-type critics (Cost / Obstacles), -1 if none
   int first_path_q;                          // list position of the first enabled path critic, -1 if none
   int closest_path_pt;                       // utils::findPathTrajectoryInitialPoint (utils.hpp:327-344), host decided
@@ -116,8 +118,54 @@ struct DevParams
   // obstacle-critic look-up tables indexed by the byte cost: [0] point cost, [1] footprint cost
   float obst_lut_crit[2][256];               // (d < margin) ? margin - d : 0
   float obst_lut_rep[2][256];                // (d < margin) ? 0 : inflation_radius - d
+  // the caller's device-resident costmap of this cycle (mppi_set_costmap_residency), null for a host map.  The kDevMap
+  // instances of the rollout kernels read their map from here, so that a captured graph follows the pointer of every cycle.
+  const uint8_t * cm_dev;
 };
 constexpr int kHotBytes = (static_cast<int>(offsetof(DevParams, fp_x)) + 15) & ~15;
+
+// ---- the costmap-dependent path tables, one definition for build_params (host map) and path_tables_kernel (device
+//      map).  Integer logic and IEEE sub / div only (no product to contract), so both sides produce the same bits.
+// utils::findPathCosts (utils.hpp:361-394): the path point (wx, wy) is valid unless worldToMap fails (fp64) or its cell is
+// lethal, inscribed, or unknown while unknown space is not tracked
+__host__ __device__ inline bool path_point_valid(const uint8_t * cells, unsigned size_x, unsigned size_y, double res, double ox,
+  double oy, int track_unknown, double wx, double wy)
+{
+  if (wx < ox || wy < oy) {return false;}
+  const double qx = (wx - ox) / res, qy = (wy - oy) / res;
+  if (!(qx < static_cast<double>(size_x) && qy < static_cast<double>(size_y))) {return false;}
+  const unsigned mx = static_cast<unsigned>(qx), my = static_cast<unsigned>(qy);
+  if (!(mx < size_x && my < size_y)) {return false;}
+  const int c = cells[static_cast<size_t>(my) * size_x + mx];
+  return !(c == LETHAL_OBSTACLE || c == INSCRIBED_INFLATED_OBSTACLE || (c == NO_INFORMATION && !track_unknown));
+}
+// PathAlign's occupancy gate for the furthest reached point f (path_align_critic.cpp:56-72); invalid_before[j] = number of
+// invalid points among [0, j).  The reference bails out of its counting loop as soon as ctr / range > ratio with ctr > 2;
+// the count only grows and the range is fixed, so the final count decides.
+__host__ __device__ inline bool path_align_gate(int f, int offset, float max_ratio, int closest, const uint16_t * invalid_before)
+{
+  if (f < offset) {return false;}
+  const float range = static_cast<float>(static_cast<long long>(f) - closest);
+  unsigned invalid_ctr = 0;
+  if (f > closest) {invalid_ctr = static_cast<unsigned>(invalid_before[f]) - static_cast<unsigned>(invalid_before[closest]);}
+  return !(invalid_ctr > 2 && static_cast<float>(invalid_ctr) / range > max_ratio);
+}
+// bits 0 (PathAlign) and 1 (PathAlignLegacy) of the flag byte of furthest point f
+__host__ __device__ inline unsigned path_align_flag_bits(const DevParams & p, int f, const uint16_t * invalid_before)
+{
+  unsigned fl = 0;
+  if (path_align_gate(f, p.align_offset, p.align_max_ratio, p.closest_path_pt, invalid_before) && f > 0) {fl |= 1u;}
+  if (path_align_gate(f, p.legacy_offset, p.legacy_max_ratio, p.closest_path_pt, invalid_before) && (p.N - 1) >= 1) {fl |= 2u;}
+  return fl;
+}
+// PathFollow's target for furthest point f (path_follow_critic.cpp:45-58); next_valid[i] = first valid index >= i
+__host__ __device__ inline int path_follow_index(int f, int offset, int N, const int * next_valid)
+{
+  const int path_size = N - 1;
+  int fidx = f + offset < path_size ? f + offset : path_size;
+  if (fidx < path_size - 1) {fidx = next_valid[fidx] < path_size - 1 ? next_valid[fidx] : path_size - 1;}
+  return fidx > 0 ? fidx : 0;
+}
 constexpr int kHotFloats = kHotBytes / 4;
 
 // cooperative copy of the hot part of the record into shared memory (16-byte vectors, coalesced)

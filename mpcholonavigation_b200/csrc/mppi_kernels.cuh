@@ -930,11 +930,14 @@ __device__ __forceinline__ void rollout_tile_body(
   MPPI_TRACE_AT(9);
 }
 
-template<unsigned F, bool kExact, int kMode>
+// kDevMap: the cycle's costmap is the caller's device memory, whose pointer the record carries (DevParams::cm_dev), so that
+// a replayed graph reads the pointer of every cycle; cm is not used then.  Separate instances, so that the host-map
+// instances stay the code they are.
+template<unsigned F, bool kExact, int kMode, bool kDevMap = false>
 __global__ void __launch_bounds__(256, MPPI_K2_MIN_BLOCKS) rollout_score_kernel(
   const DevParams * __restrict__ P, const uint8_t * __restrict__ cm, DevBuffers bufs, const int B, const int T)
 {
-  rollout_tile_body<F, kExact, kMode, false>(P, cm, bufs, B, T, nullptr);
+  rollout_tile_body<F, kExact, kMode, false>(P, kDevMap ? P->cm_dev : cm, bufs, B, T, nullptr);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -1396,11 +1399,12 @@ __device__ __forceinline__ void rollout_score_stream_body(
   }
 }
 
-template<unsigned F, bool kExact>
+// kDevMap: see rollout_score_kernel (the group's batched form takes the member's map pointer from its job instead)
+template<unsigned F, bool kExact, bool kDevMap = false>
 __global__ void __launch_bounds__(kStreamThreads, MPPI_STREAM_MIN_BLOCKS) rollout_score_stream_kernel(
   const DevParams * __restrict__ P, const uint8_t * __restrict__ cm, DevBuffers bufs)
 {
-  rollout_score_stream_body<F, kExact>(P, cm, bufs);
+  rollout_score_stream_body<F, kExact>(P, kDevMap ? P->cm_dev : cm, bufs);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -2759,12 +2763,14 @@ __device__ __forceinline__ void tile_fused_body(
 }
 
 // (Pg, cm: no __restrict__ -- the tiles write both during the zero-copy upload)
-template<unsigned F, bool kExact>
+// kDevMap: see rollout_score_kernel (never with the zero-copy upload: the record is in device memory before the launch)
+template<unsigned F, bool kExact, bool kDevMap = false>
 __global__ void __launch_bounds__(256, MPPI_FUSED_MIN_BLOCKS) tile_fused_kernel(
   const DevParams * Pg, const uint8_t * cm, DevBuffers bufs, const int B, const int T, const int n_cap,
   const int iteration, uint2 * host_res, const uint4 * up_host, const int up_vecs, const int tail_mode, float * hist)
 {
-  tile_fused_body<F, kExact>(Pg, cm, bufs, B, T, n_cap, iteration, host_res, up_host, up_vecs, blockIdx.x, gridDim.x, tail_mode, hist);
+  tile_fused_body<F, kExact>(Pg, kDevMap ? Pg->cm_dev : cm, bufs, B, T, n_cap, iteration, host_res, up_host, up_vecs, blockIdx.x,
+    gridDim.x, tail_mode, hist);
 }
 
 // K3c (stream layout): softmax weights and weighted control sums over time-major noise [T][B]; a GEMV
@@ -3491,6 +3497,81 @@ __global__ void __launch_bounds__(kUpdThreads) merge_finalize_batch_kernel(const
   const FusedJob & j = jobs[blockIdx.y];
   if (static_cast<int>(blockIdx.x) >= j.merge_blocks) {return;}
   merge_finalize_body(j.Pg, j.bufs.partials, j.ws_chunks, j.stride, j.bufs, 1, nullptr, deliver ? j.host_res : nullptr, tag);
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Path tables of a cycle whose costmap is device-resident (mppi_set_costmap_residency): build_params wrote the record
+// without them, this kernel reads the map in place and writes valid[j], bits 0 / 1 of flags[f] (beside the PathAngle bit
+// the host wrote) and follow_idx[f] into the device copy of the record, with build_params' own rules (mppi_device.cuh).
+// One block, one thread per path point; both scans are integer, so the tables are the host's bit for bit.  A record
+// without a device map (cm_dev == null: a host-mode member of a group) is left alone.
+// ---------------------------------------------------------------------------------------------------
+constexpr int kTablesThreads = MPPI_MAX_PATH_POINTS;
+static_assert(kTablesThreads == 32 * 32, "the scans below combine 32 warps of 32 lanes");
+
+__device__ __forceinline__ void path_tables_body(DevParams * P)
+{
+  __shared__ uint16_t s_inv[kTablesThreads + 1];   // invalid points among [0, j)
+  __shared__ int s_next[kTablesThreads + 1];        // first valid index >= j, N if none
+  __shared__ int s_warp[2][32];
+  const uint8_t * cm = P->cm_dev;
+  if (cm == nullptr) {return;}
+  const int N = P->N, n16 = ((N + 15) / 16) * 16;
+  const int j = threadIdx.x, lane = j & 31, warp = j >> 5;
+  const float * path = reinterpret_cast<const float *>(P + 1);
+  uint8_t * valid = reinterpret_cast<uint8_t *>(const_cast<float *>(path) + 4 * N);
+  uint8_t * flags = valid + n16;
+  uint16_t * follow = reinterpret_cast<uint16_t *>(valid + 2 * n16);
+  bool ok = false;
+  if (j < N - 1) {
+    ok = path_point_valid(cm, P->size_x, P->size_y, P->res, P->ox, P->oy, P->track_unknown,
+      static_cast<double>(path[P->off_path_x + j]), static_cast<double>(path[P->off_path_y + j]));
+  }
+  // inclusive prefix count of the invalid points (the last point counts: it is never valid) and suffix minimum of the
+  // valid indices, per warp with shuffles, then across the 32 warp totals
+  int inv = (j < N && !ok) ? 1 : 0;
+  int nxt = (j < N && ok) ? j : N;
+  for (int o = 1; o < 32; o <<= 1) {
+    const int a = __shfl_up_sync(0xffffffffu, inv, o), b = __shfl_down_sync(0xffffffffu, nxt, o);
+    if (lane >= o) {inv += a;}
+    if (lane + o < 32) {nxt = min(nxt, b);}
+  }
+  if (lane == 31) {s_warp[0][warp] = inv;}
+  if (lane == 0) {s_warp[1][warp] = nxt;}
+  __syncthreads();
+  if (warp == 0) {
+    int wi = s_warp[0][lane], wn = s_warp[1][lane];
+    for (int o = 1; o < 32; o <<= 1) {
+      const int a = __shfl_up_sync(0xffffffffu, wi, o), b = __shfl_down_sync(0xffffffffu, wn, o);
+      if (lane >= o) {wi += a;}
+      if (lane + o < 32) {wn = min(wn, b);}
+    }
+    s_warp[0][lane] = wi;
+    s_warp[1][lane] = wn;
+  }
+  __syncthreads();
+  if (warp > 0) {inv += s_warp[0][warp - 1];}
+  if (warp < 31) {nxt = min(nxt, s_warp[1][warp + 1]);}
+  s_inv[j + 1] = static_cast<uint16_t>(inv);
+  if (j == 0) {s_inv[0] = 0;}
+  s_next[j] = nxt;
+  __syncthreads();
+  if (j < N) {
+    valid[j] = ok ? 1 : 0;
+    follow[j] = static_cast<uint16_t>(path_follow_index(j, P->follow_offset, N, s_next));
+    flags[j] = static_cast<uint8_t>((flags[j] & 4u) | path_align_flag_bits(*P, j, s_inv));
+  }
+}
+
+__global__ void __launch_bounds__(kTablesThreads) path_tables_kernel(DevParams * P)
+{
+  path_tables_body(P);
+}
+
+// a chunk of a robot group: member = blockIdx.y
+__global__ void __launch_bounds__(kTablesThreads) path_tables_batch_kernel(const FusedJob * __restrict__ jobs)
+{
+  path_tables_body(const_cast<DevParams *>(jobs[blockIdx.y].Pg));
 }
 
 }  // namespace mppi

@@ -170,6 +170,16 @@ typedef struct mppi_cycle_out {
                                 captured cycle); 0 when mppi_set_timing(h, 0) */
 } mppi_cycle_out;
 
+/* Cycle inputs of a bound group (mppi_optimize_group_device), in device memory of the group's device, one row per member
+ * in bind order: what mppi_cycle_in carries besides the costmap. */
+typedef struct mppi_group_inputs {
+  const double * state;      /* [n][8]: pose_x, pose_y, pose_yaw, speed_vx, speed_vy, speed_wz, goal_x, goal_y */
+  const double * goal_checker_xy_tolerance;   /* [n]; < 0: goal_checker == nullptr */
+  const int32_t * path_size; /* [n]; each in [1, MPPI_MAX_PATH_POINTS] and <= path_stride */
+  const float * path;        /* [n][3][path_stride]: x, y, yaw */
+  int32_t path_stride;       /* >= every path_size */
+} mppi_group_inputs;
+
 typedef struct mppi_handle mppi_handle;
 
 /* ---- life cycle (ref: Optimizer::initialize/shutdown/reset optimizer.cpp:35-60,116-132) ---- */
@@ -265,6 +275,31 @@ mppi_status mppi_optimize_batch_resident(mppi_handle ** handles, mppi_cycle_out 
 /* Device time of the last batch call over these handles (one device, timing on): first start event to latest end
  * event; the handles run concurrently on their own streams, so their device_ms overlap. */
 mppi_status mppi_batch_span_ms(mppi_handle ** handles, int32_t n, float * ms_out);
+/* mppi_optimize_batch over exactly a bound group (bind order) whose cycle inputs are already in device memory: a GPU
+ * simulator's state tensors, or a fleet server's one packed upload.  Every member must be in MPPI_COSTMAP_DEVICE mode and
+ * qualify for the group's batched launches.  maps[n] are HOST descriptors whose cells point into device memory (checked
+ * as for mppi_set_costmap_residency); outs as for mppi_optimize_batch.  The members' cycle records are built on the
+ * device, so the host does no per-robot work besides the job table; the result is bit for bit what mppi_optimize_batch
+ * returns for the same inputs (one exception, DESIGN.md section 2: PathAngle's gate for a path point within 1e-5 of the
+ * threshold's cosine is decided with the device's atan2f).
+ * Contract, as for a device costmap: the inputs are complete before the call, stay unchanged until it returns, and
+ * nothing reads them afterwards (the caller synchronises its own streams first).
+ * MPPI_E_CONFIG before anything is enqueued: hs is not exactly a bound group, a member is in host-costmap mode or does not
+ * qualify (evalControl tail, profiling, another iteration_count than member 0; there is no one-by-one fallback), both
+ * PathAlign critics enabled with different trajectory_point_step, an input pointer is not device memory of the group's
+ * device or its allocation holds fewer than n rows, a map is rejected.
+ * A path_size outside [1, min(MPPI_MAX_PATH_POINTS, path_stride)] is seen on the device: that member's launches are
+ * cancelled, its outputs and warm start (control sequence, costs, noise) stay as they were, the other members run, and the
+ * call returns MPPI_E_CONFIG with the member's index in mppi_last_error(hs[0]).  The call leaves a staged cycle for
+ * mppi_optimize_batch_resident like mppi_optimize_batch does (not for a member that failed). */
+mppi_status mppi_optimize_group_device(mppi_handle ** hs, int32_t n, const mppi_group_inputs * in,
+                                       const mppi_costmap * maps, mppi_cycle_out * outs);
+/* Test hook: the first `capacity` bytes of the device copy of the handle's last cycle record (record + path tail), its
+ * meaningful length in *record_bytes, and in *angle_band_hits the number of PathAngle gate decisions the device inputs
+ * of mppi_optimize_group_device have left to the device's atan2f since create (a path point exactly under the robot is
+ * not counted: atan2f(0, 0) = 0 on either side). */
+mppi_status mppi_debug_get_record(mppi_handle * h, void * out, uint64_t capacity, uint64_t * record_bytes,
+                                  uint64_t * angle_band_hits);
 
 /* Split-phase form for data already resident on the device (bench "value" leg, CUDA-graph replay):
  * upload once, then run the device part only.  A device-resident costmap is read by mppi_optimize_resident: it must stay

@@ -8,7 +8,7 @@ declared in ``include/mppi_b200.h``) and a thin ctypes binding (``_abi``, ``api`
 """
 from . import _abi as abi  # noqa: F401
 from .api import (Cycle, Engine, MppiError, Result, circle_footprint, load_product, make_config,  # noqa: F401
-                  make_critic, make_robot, optimize_sharded)
+                  make_critic, make_robot, optimize_group_device, optimize_sharded)
 
 
 def MppiOptimizer(**cfg_kw):

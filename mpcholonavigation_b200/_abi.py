@@ -153,6 +153,17 @@ class CycleOut(C.Structure):
     ]
 
 
+class GroupInputs(C.Structure):
+    """mppi_group_inputs: cycle inputs of a bound group in device memory, one row per member"""
+    _fields_ = [
+        ("state", C.c_void_p),                      # const double [n][8]
+        ("goal_checker_xy_tolerance", C.c_void_p),  # const double [n]
+        ("path_size", C.c_void_p),                  # const int32 [n]
+        ("path", C.c_void_p),                       # const float [n][3][path_stride]
+        ("path_stride", C.c_int32),
+    ]
+
+
 H = C.c_void_p  # opaque handle
 
 # name -> (restype, argtypes); names are without prefix
@@ -195,6 +206,8 @@ PRODUCT_ONLY = {
     "batch_bind": (C.c_int, [C.POINTER(H), C.c_int32]),
     "batch_unbind": (C.c_int, [H]),
     "batch_span_ms": (C.c_int, [C.POINTER(H), C.c_int32, f32p]),
+    "optimize_group_device": (C.c_int, [C.POINTER(H), C.c_int32, C.POINTER(GroupInputs), C.POINTER(Costmap), C.POINTER(CycleOut)]),
+    "debug_get_record": (C.c_int, [H, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "upload_cycle": (C.c_int, [H, C.POINTER(CycleIn)]),
     "optimize_resident": (C.c_int, [H, C.POINTER(CycleOut)]),
     "set_outputs": (C.c_int, [H, C.c_uint32]),

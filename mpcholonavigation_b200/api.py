@@ -448,3 +448,44 @@ def optimize_sharded(engines, cycle: Cycle) -> Result:
         msgs = [e.f["last_error"](e.h).decode() for e in engines]
         raise MppiError(f"mppi status {status}: {msgs}")
     return Engine._result(out, arrs)
+
+
+def optimize_group_device(engines, state, tolerance, path_size, path, maps):
+    """mppi_optimize_group_device: one cycle of a bound group (``engines`` in bind order, every one in device-costmap
+    mode) whose inputs are CUDA tensors on the group's device, one row per member:
+    state float64 [n, 8] (pose x, y, yaw, speed vx, vy, wz, goal x, y), tolerance float64 [n] (< 0: no goal checker),
+    path_size int32 [n], path float32 [n, 3, stride] (x, y, yaw).  maps: per member (uint8 CUDA tensor [size_y, size_x],
+    resolution, (origin_x, origin_y)).  The records are built on the device; returns a list of Result."""
+    torch = _torch()
+    n = len(engines)
+    e0 = engines[0]
+    tensors = {"state": (state, torch.float64, (n, 8)), "tolerance": (tolerance, torch.float64, (n,)),
+               "path_size": (path_size, torch.int32, (n,)), "path": (path, torch.float32, None)}
+    for name, (t, dtype, shape) in tensors.items():
+        if not _is_cuda_tensor(t) or t.dtype != dtype or not t.is_contiguous() or (shape and tuple(t.shape) != shape):
+            raise ValueError(f"{name}: a contiguous {dtype} CUDA tensor{' of shape ' + str(shape) if shape else ''} is expected")
+    if path.dim() != 3 or path.shape[0] != n or path.shape[1] != 3:
+        raise ValueError("path: [n, 3, stride] expected")
+    gi = abi.GroupInputs()
+    gi.state, gi.goal_checker_xy_tolerance = state.data_ptr(), tolerance.data_ptr()
+    gi.path_size, gi.path, gi.path_stride = path_size.data_ptr(), path.data_ptr(), path.shape[2]
+    cms = (abi.Costmap * n)()
+    for i, (cells, resolution, origin) in enumerate(maps):
+        if not _is_cuda_tensor(cells) or cells.dtype != torch.uint8 or cells.dim() != 2 or not cells.is_contiguous():
+            raise ValueError("maps: contiguous 2-D uint8 CUDA tensors expected")
+        cms[i].cells = C.cast(C.c_void_p(cells.data_ptr()), abi.u8p)
+        cms[i].size_y, cms[i].size_x = cells.shape
+        cms[i].resolution = float(resolution)
+        cms[i].origin_x, cms[i].origin_y = (float(v) for v in origin)
+    # the library reads the inputs without waiting on any stream: torch's queued writes must be complete
+    for device in {t.device for t in [state, tolerance, path_size, path] + [m[0] for m in maps]}:
+        torch.cuda.current_stream(device).synchronize()
+    outs = (abi.CycleOut * n)()
+    arrs = []
+    for i, e in enumerate(engines):
+        o, a = e._out()
+        outs[i] = o
+        arrs.append(a)
+    hs = (abi.H * n)(*[e.h for e in engines])
+    e0._check(e0.f["optimize_group_device"](hs, n, C.byref(gi), cms, outs))
+    return [Engine._result(outs[i], arrs[i]) for i in range(n)]

@@ -139,6 +139,8 @@ struct mppi_handle
   FusedJob * d_jobs{nullptr};             // ... and its device copy (re-sent only when an entry changes)
   std::vector<char> jobs_sent;            // what the device copy holds
   NoiseJob * d_noise_jobs{nullptr};       // leader only: the regenerate_noises members, in bind order (fixed at bind)
+  std::vector<NoiseJob> noise_jobs_h;     // leader only: ... its host copy
+  int * d_noise_index{nullptr};           // leader only: [n] each member's entry in it, -1 for none (record_batch_kernel)
   std::vector<long long> noise_items;     // leader only: B * ceil(T / 4) of each entry, the work of its redraw
   char * arena_h{nullptr};                // leader: the [record | costmap] buffers of all members, one slice each,
   char * arena_d{nullptr};                //   so that the whole group uploads with ONE strided copy
@@ -146,6 +148,15 @@ struct mppi_handle
   bool params_in_arena{false};            // member: h_params / d_params point into the leader's arena
   uint32_t batch_tag{0};                  // leader: counter behind the tag of the group's result packets
   uint32_t result_tag{0};                 // tag the cycle in flight delivers its result packets with
+  // cycle inputs in device memory (mppi_optimize_group_device): each member's record template (record_batch_kernel),
+  // rebuilt when the configuration behind it changes (rec_gen: bumped by every setter build_params reads) or the map geometry
+  char * tmpl_h{nullptr};                 // leader: [n][kTemplateStride] pinned ...
+  char * tmpl_d{nullptr};                 //   ... and the device copy the kernel reads
+  uint64_t rec_gen{1};                    // member: configuration generation
+  uint64_t tmpl_gen{0};                   // member: the generation its template was built for (0: none)
+  mppi_costmap tmpl_map{};                // member: the map geometry of its template
+  bool record_from_device{false};         // member: the cycle in flight built its record on the device; h->last follows
+  uint64_t angle_band_hits{0};            // member: PathAngle decisions left to the device's atan2f (mppi_debug_get_record)
   // caller memory registered as pinned (mppi_register_costmap_memory): a costmap inside such a range is copied to the
   // device straight from the caller's buffer, without the staging memcpy
   std::vector<std::pair<const char *, size_t>> pinned_ranges;
@@ -233,22 +244,7 @@ mppi_status fail(mppi_handle * h, mppi_status s, const std::string & msg)
 bool holonomic(const mppi_handle * h) {return h->cfg.motion_model == MPPI_MODEL_OMNI;}
 
 // ---- host-side scalar helpers, restating the reference's host code --------------------------------
-// utils::withinPositionGoalTolerance(float, ...) utils.hpp:233-249
-bool within_tolerance(float pose_tolerance, double rx, double ry, double gx, double gy)
-{
-  const double dist_sq = std::pow(gx - rx, 2) + std::pow(gy - ry, 2);
-  const float pose_tolerance_sq = pose_tolerance * pose_tolerance;
-  return dist_sq < pose_tolerance_sq;
-}
-// utils::withinPositionGoalTolerance(GoalChecker*, ...) utils.hpp:201-224
-bool within_checker_tolerance(double tol, double rx, double ry, double gx, double gy)
-{
-  if (tol >= 0.0) {
-    const double dx = rx - gx, dy = ry - gy;
-    if (dx * dx + dy * dy < tol * tol) {return true;}
-  }
-  return false;
-}
+// (within_tolerance / within_checker_tolerance: mppi_device.cuh, shared with record_batch_kernel)
 double normalize_angle(double angle)
 {
   const double result = std::fmod(angle + M_PI, 2.0 * M_PI);
@@ -556,10 +552,8 @@ mppi_status build_params(mppi_handle * h, const mppi_cycle_in * in, int mode, un
       if (p.angle.on) {
         // path_angle_critic.cpp:79-83 for every index the furthest point could select.  The reference's test is
         // posePointAngle(...) < max_angle (atan2f + fmod per point: most of this function's time at 40 points).  With
-        // forward_preference the angle A in [0, pi] is the one between the heading and the direction to the point, so
-        // "A < max" is "cos A > cos max": decided from a dot product wherever that is further than 1e-5 from the
-        // threshold (atan2f, the float roundings of the reference and the rounding of A to float move cos A by < 1e-6);
-        // the reference's own arithmetic decides the rest, so the gate is the reference's gate bit for bit.
+        // forward_preference path_angle_fast_gate decides it from a dot product away from the threshold; the reference's
+        // own arithmetic decides the rest, so the gate is the reference's gate bit for bit.
         const float thr = d->max_angle_to_furthest;
         const bool fast = forward_preference && thr > 1.0e-3f && thr < 3.1f;
         const float pose_xf = static_cast<float>(rx), pose_yf = static_cast<float>(ry), pose_yawf = static_cast<float>(in->pose_yaw);
@@ -567,15 +561,7 @@ mppi_status build_params(mppi_handle * h, const mppi_cycle_in * in, int mode, un
         const double ct = std::cos(static_cast<double>(thr));
         for (int j = 0; j < N; ++j) {
           const float gxj = in->path_x[j], gyj = in->path_y[j];
-          int decided = -1;
-          if (fast) {
-            const double dxj = static_cast<double>(gxj - pose_xf), dyj = static_cast<double>(gyj - pose_yf);   // float differences, as atan2f gets them
-            const double dd = dxj * dxj + dyj * dyj;
-            if (dd > 1.0e-12) {
-              const double c = (dxj * ch + dyj * sh) / std::sqrt(dd);
-              if (c < ct - 1.0e-5) {decided = 1;} else if (c > ct + 1.0e-5) {decided = 0;}
-            }
-          }
+          const int decided = fast ? path_angle_fast_gate(gxj, gyj, pose_xf, pose_yf, ch, sh, ct) : -1;
           const bool open = decided >= 0 ? decided == 1 :
             !(pose_point_angle(rx, ry, in->pose_yaw, gxj, gyj, forward_preference) < thr);
           gate[j] = open ? 1 : 0;
@@ -773,30 +759,24 @@ mppi_status stage_costmap(mppi_handle * h, const mppi_costmap & cm)
   return MPPI_OK;
 }
 
-// The caller's device-resident costmap: device memory of this handle's device (not managed, not host, not another GPU's),
-// size_x * size_y bytes inside one allocation.  Checked before anything of the cycle is enqueued; a kernel never sees a
-// pointer that did not pass.  The last pointer that passed is remembered (a producer usually hands over the same buffer).
-mppi_status check_device_costmap_impl(mppi_handle * h, const mppi_costmap & cm)
+// `bytes` bytes at p inside one allocation of device memory of h's device (not managed, not host, not another GPU's)
+mppi_status check_device_range(mppi_handle * h, const void * p, size_t bytes, const std::string & what)
 {
-  const size_t bytes = static_cast<size_t>(cm.size_x) * cm.size_y;
-  if (bytes == 0 || !cm.cells) {return fail(h, MPPI_E_CONFIG, "empty costmap");}
-  if (!(cm.resolution > 0.0)) {return fail(h, MPPI_E_CONFIG, "costmap resolution must be > 0");}
-  if (cm.cells == h->cm_checked && bytes <= h->cm_checked_bytes) {return MPPI_OK;}
   CUDA_TRY(h, cudaSetDevice(h->device));
   cudaPointerAttributes a;
-  if (cudaPointerGetAttributes(&a, cm.cells) != cudaSuccess) {
+  if (!p || cudaPointerGetAttributes(&a, p) != cudaSuccess) {
     cudaGetLastError();
-    return fail(h, MPPI_E_CONFIG, "device costmap: not a CUDA pointer");
+    return fail(h, MPPI_E_CONFIG, what + ": not a CUDA pointer");
   }
   if (a.type != cudaMemoryTypeDevice) {
-    return fail(h, MPPI_E_CONFIG, a.type == cudaMemoryTypeManaged ? "device costmap: managed memory is not accepted" :
-      "device costmap: costmap.cells is host memory (MPPI_COSTMAP_DEVICE expects device memory)");
+    return fail(h, MPPI_E_CONFIG, a.type == cudaMemoryTypeManaged ? what + ": managed memory is not accepted" :
+      what + " is host memory (device memory expected)");
   }
   if (a.device != h->device) {
-    return fail(h, MPPI_E_CONFIG, "device costmap: the map is on device " + std::to_string(a.device) + ", the handle on device " +
+    return fail(h, MPPI_E_CONFIG, what + " is on device " + std::to_string(a.device) + ", the handle on device " +
       std::to_string(h->device));
   }
-  // the allocation must hold the whole map (cuMemGetAddressRange, a driver entry point fetched through the runtime)
+  // the allocation must hold all the bytes (cuMemGetAddressRange, a driver entry point fetched through the runtime)
   typedef CUresult (*RangeFn)(CUdeviceptr *, size_t *, CUdeviceptr);
   static RangeFn range_fn = nullptr;
   if (!range_fn) {
@@ -810,10 +790,24 @@ mppi_status check_device_costmap_impl(mppi_handle * h, const mppi_costmap & cm)
   }
   CUdeviceptr base = 0;
   size_t size = 0;
-  const CUdeviceptr ptr = reinterpret_cast<CUdeviceptr>(cm.cells);
+  const CUdeviceptr ptr = reinterpret_cast<CUdeviceptr>(p);
   if (range_fn(&base, &size, ptr) != CUDA_SUCCESS || ptr - base + bytes > size) {
-    return fail(h, MPPI_E_CONFIG, "device costmap: size_x * size_y bytes do not fit the allocation behind costmap.cells");
+    return fail(h, MPPI_E_CONFIG, what + ": " + std::to_string(bytes) + " bytes do not fit the allocation behind it");
   }
+  return MPPI_OK;
+}
+
+// The caller's device-resident costmap: size_x * size_y bytes of device memory (check_device_range).  Checked before
+// anything of the cycle is enqueued; a kernel never sees a pointer that did not pass.  The last pointer that passed is
+// remembered (a producer usually hands over the same buffer).
+mppi_status check_device_costmap_impl(mppi_handle * h, const mppi_costmap & cm)
+{
+  const size_t bytes = static_cast<size_t>(cm.size_x) * cm.size_y;
+  if (bytes == 0 || !cm.cells) {return fail(h, MPPI_E_CONFIG, "empty costmap");}
+  if (!(cm.resolution > 0.0)) {return fail(h, MPPI_E_CONFIG, "costmap resolution must be > 0");}
+  if (cm.cells == h->cm_checked && bytes <= h->cm_checked_bytes) {return MPPI_OK;}
+  const mppi_status s = check_device_range(h, cm.cells, bytes, "device costmap: costmap.cells");
+  if (s != MPPI_OK) {return s;}
   h->cm_checked = cm.cells;
   h->cm_checked_bytes = bytes;
   return MPPI_OK;
@@ -1373,12 +1367,9 @@ mppi_status enqueue_optimize_impl(mppi_handle * h, bool with_upload)
 // {value, tag}; a packet whose tag is the tag of the last launch enqueued is complete.  Polling them replaces the D2H
 // copy node and the stream synchronisation.  The stream is queried every few thousand polls so that a failed launch
 // surfaces as an error instead of a hang.
-mppi_status wait_result_packets(mppi_handle * h)
+mppi_status wait_packets(mppi_handle * h, const uint2 * src, int n, uint32_t tag, uint32_t * dst)
 {
-  const int n = 3 * h->T + 2 + (h->tail_mode ? 3 : 0);
-  const uint32_t tag = h->result_tag;
-  const uint64_t * pk = reinterpret_cast<const uint64_t *>(h->h_res);
-  uint32_t * dst = reinterpret_cast<uint32_t *>(h->h_out);
+  const uint64_t * pk = reinterpret_cast<const uint64_t *>(src);
   uint64_t spins = 0;
   bool drained = false;
   for (int i = 0; i < n; ++i) {
@@ -1404,6 +1395,11 @@ mppi_status wait_result_packets(mppi_handle * h)
     }
   }
   return MPPI_OK;
+}
+
+mppi_status wait_result_packets(mppi_handle * h)
+{
+  return wait_packets(h, h->h_res, 3 * h->T + 2 + (h->tail_mode ? 3 : 0), h->result_tag, reinterpret_cast<uint32_t *>(h->h_out));
 }
 
 // the event behind the cycle's result: a batched group step ends at the leader's ev1 (its redraw runs behind that), a
@@ -1441,6 +1437,11 @@ mppi_status finish_optimize(mppi_handle * h, mppi_cycle_out * out)
   const uint64_t t_b = now_ns();
   h->host_ns[5] += t_b - t_a;
   const int T = h->T;
+  if (h->record_from_device) {
+    // the hot part of the record the device built, copied back ahead of the kernels that delivered the packets above
+    std::memcpy(&h->last, h->h_params, kHotBytes);
+    h->record_from_device = false;
+  }
   h->spilled_traj = h->last.spill_traj != 0;
   h->spilled_cells = h->last.want_cells != 0;
   h->vis_valid = h->last.vis_b_step > 0;
@@ -1548,6 +1549,7 @@ mppi_status do_reset(mppi_handle * h)
 {
   const size_t T = h->T, B = h->B;
   h->cur = h->base;
+  h->rec_gen++;
   CUDA_TRY(h, cudaMemsetAsync(h->d_cs, 0, 3 * T * sizeof(float), h->stream));
   CUDA_TRY(h, cudaMemsetAsync(h->d_hist, 0, 12 * sizeof(float), h->stream));   // control_history_ (optimizer.cpp:120-123)
   CUDA_TRY(h, cudaMemsetAsync(h->d_costs, 0, B * sizeof(float), h->stream));
@@ -1599,12 +1601,16 @@ void batch_unbind_group(mppi_handle * leader)
   }
   if (leader->arena_h) {cudaFreeHost(leader->arena_h); leader->arena_h = nullptr;}
   if (leader->arena_d) {cudaFree(leader->arena_d); leader->arena_d = nullptr;}
+  if (leader->tmpl_h) {cudaFreeHost(leader->tmpl_h); leader->tmpl_h = nullptr;}
+  if (leader->tmpl_d) {cudaFree(leader->tmpl_d); leader->tmpl_d = nullptr;}
   leader->arena_slice = 0;
   leader->batch_group.clear();
   leader->jobs_sent.clear();
   if (leader->h_jobs) {cudaFreeHost(leader->h_jobs); leader->h_jobs = nullptr;}
   if (leader->d_jobs) {cudaFree(leader->d_jobs); leader->d_jobs = nullptr;}
   if (leader->d_noise_jobs) {cudaFree(leader->d_noise_jobs); leader->d_noise_jobs = nullptr;}
+  if (leader->d_noise_index) {cudaFree(leader->d_noise_index); leader->d_noise_index = nullptr;}
+  leader->noise_jobs_h.clear();
   leader->noise_items.clear();
 }
 
@@ -1691,7 +1697,7 @@ mppi_status batch_redraw(mppi_handle * L, int k0, int kn)
 // whole call.  Members may differ in B and T: every grid dimension spans the chunk's largest extent, and each member's job
 // carries its own extents, so that its surplus blocks return at once.
 mppi_status batch_stream_launch(mppi_handle * L, mppi_handle ** hs, int c0, int n, int k0, int kn, bool with_upload, uint32_t tag,
-  bool first, bool last)
+  bool first, bool last, const mppi_group_inputs * din = nullptr)
 {
   unsigned inst = pick_stream_instance(stream_feature_need(hs[0]->last));
   size_t max_used = 0;
@@ -1702,6 +1708,8 @@ mppi_status batch_stream_launch(mppi_handle * L, mppi_handle ** hs, int c0, int 
     B_max = std::max(B_max, hs[i]->B);
     T_max = std::max(T_max, hs[i]->T);
   }
+  // records built on the device: the host does not see the gates, so the generic instance (flags tested at run time)
+  if (din) {inst = SF_ALL;}
   const int nthr = stream_block_threads(B_max);
   int rollout_grid = 0, cost_grid = 0, ws_grid = 0, ws_total = 0, merge_grid = 0;
   if (first && L->timing) {CUDA_TRY(L, cudaEventRecord(L->ev0, L->stream));}
@@ -1739,6 +1747,7 @@ mppi_status batch_stream_launch(mppi_handle * L, mppi_handle ** hs, int c0, int 
     h->result_tag = tag;
     h->d2h_bytes = sizeof(uint2) * (3 * h->T + 2);
     h->h2d_bytes = with_upload ? upload_bytes(h) : 0;
+    h->record_from_device = din != nullptr;
   }
   const size_t off = sizeof(FusedJob) * static_cast<size_t>(c0), bytes = sizeof(FusedJob) * static_cast<size_t>(n);
   if (std::memcmp(L->jobs_sent.data() + off, L->h_jobs + c0, bytes) != 0) {
@@ -1746,6 +1755,17 @@ mppi_status batch_stream_launch(mppi_handle * L, mppi_handle ** hs, int c0, int 
     std::memcpy(L->jobs_sent.data() + off, L->h_jobs + c0, bytes);
   }
   const FusedJob * jobs = L->d_jobs + c0;
+  if (din) {
+    // the chunk's records from the cycle inputs in device memory, where the strided upload would have put them; then
+    // their hot parts back to the host slices (finish_optimize: h->last), ahead of the kernels that deliver the results
+    record_batch_kernel<<<dim3(1, n), kRecordThreads, 0, L->stream>>>(L->d_jobs + c0, L->tmpl_d, *din, c0, tag, L->d_noise_jobs,
+      L->d_noise_index);
+    CUDA_TRY(L, cudaGetLastError());
+    L->launches++;
+    const size_t off = L->arena_slice * static_cast<size_t>(c0);
+    CUDA_TRY(L, cudaMemcpy2DAsync(L->arena_h + off, L->arena_slice, L->arena_d + off, L->arena_slice, kHotBytes, n,
+      cudaMemcpyDeviceToHost, L->stream));
+  }
   bool any_dev_map = false;
   for (int i = 0; i < n; ++i) {any_dev_map = any_dev_map || hs[i]->last.cm_dev != nullptr;}
   if (any_dev_map) {
@@ -1864,6 +1884,153 @@ mppi_status batch_run_group(mppi_handle ** hs, const mppi_cycle_in * ins, mppi_c
     if (!pending[i]) {continue;}
     const mppi_status f = finish_optimize(hs[i], outs ? &outs[i] : nullptr);
     if (f != MPPI_OK && first == MPPI_OK) {first = f;}
+  }
+  return first;
+}
+
+// ---- cycle inputs in device memory (mppi_optimize_group_device) -------------------------------------------------------
+// Member i's record template (record_batch_kernel): build_params over placeholder inputs (one path point, the robot on its
+// goal) writes every field that depends on the configuration and the map geometry alone, with the host's own code (the
+// ObstaclesCritic LUTs need host logf); the thresholds of the per-cycle gates follow the record.
+mppi_status build_template(mppi_handle * L, mppi_handle * h, int i, const mppi_costmap & map)
+{
+  static const float zero = 0.0f;
+  mppi_cycle_in in;
+  std::memset(&in, 0, sizeof(in));
+  in.goal_checker_xy_tolerance = -1.0;
+  in.path_size = 1; in.path_x = &zero; in.path_y = &zero; in.path_yaw = &zero;
+  in.costmap = map;
+  h->cycle_uploaded = false;   // h->last and the host slice hold the placeholder record from here on
+  h->tmpl_gen = 0;
+  const mppi_status s = build_params(h, &in, 0, kUnset, true);
+  if (s != MPPI_OK) {return s;}
+  char * slot = L->tmpl_h + static_cast<size_t>(i) * kTemplateStride;
+  std::memcpy(slot, h->h_params, sizeof(DevParams));
+  const DevParams & p = *reinterpret_cast<const DevParams *>(slot);
+  RecordGates & g = *reinterpret_cast<RecordGates *>(slot + sizeof(DevParams));
+  std::memset(&g, 0, sizeof(g));
+  int idx;
+  const mppi_critic_desc * d;
+  if ((d = find_kind(h, MPPI_CRITIC_COST, &idx))) {g.has_cost = 1; g.cost_near = d->near_goal_distance;}
+  if ((d = find_kind(h, MPPI_CRITIC_OBSTACLES, &idx))) {g.has_obst = 1; g.obst_near = d->near_goal_distance;}
+  struct {int kind; int * en; float * thr;} gated[] = {
+    {MPPI_CRITIC_GOAL, &g.goal_en, &g.goal_thr}, {MPPI_CRITIC_GOAL_ANGLE, &g.goal_angle_en, &g.goal_angle_thr},
+    {MPPI_CRITIC_PREFER_FORWARD, &g.forward_en, &g.forward_thr}, {MPPI_CRITIC_TWIRLING, &g.twirl_en, nullptr},
+    {MPPI_CRITIC_PATH_FOLLOW, &g.follow_en, &g.follow_thr}, {MPPI_CRITIC_PATH_ALIGN, &g.align_en, &g.align_thr},
+    {MPPI_CRITIC_PATH_ALIGN_LEGACY, &g.legacy_en, &g.legacy_thr}, {MPPI_CRITIC_PATH_ANGLE, &g.angle_en, &g.angle_thr}};
+  for (const auto & k : gated) {
+    if ((d = find_kind(h, k.kind, &idx))) {
+      *k.en = d->enabled ? 1 : 0;
+      if (k.thr) {*k.thr = d->threshold_to_consider;}
+    }
+  }
+  // build_params refuses the two PathAlign critics with different steps when both gates are open; which gates open is
+  // only known on the device
+  if (g.align_en && g.legacy_en && p.align_step != p.legacy_step) {
+    return fail(h, MPPI_E_CONFIG, "device inputs: PathAlignCritic and PathAlignLegacyCritic must share trajectory_point_step");
+  }
+  if ((d = find_kind(h, MPPI_CRITIC_PATH_ANGLE, &idx))) {
+    const float thr = d->max_angle_to_furthest;
+    g.angle_max = thr;
+    g.angle_fast = (p.angle_forward_pref && thr > 1.0e-3f && thr < 3.1f) ? 1 : 0;   // build_params' `fast`
+    g.angle_cos_max = std::cos(static_cast<double>(thr));
+  }
+  g.want_traj = (h->want_mask & MPPI_WANT_TRAJECTORIES) ? 1 : 0;
+  CUDA_TRY(L, cudaMemcpyAsync(L->tmpl_d + static_cast<size_t>(i) * kTemplateStride, slot, kTemplateStride, cudaMemcpyHostToDevice,
+    L->stream));
+  h->tmpl_gen = h->rec_gen;
+  h->tmpl_map = map;
+  return MPPI_OK;
+}
+
+bool template_current(const mppi_handle * h, const mppi_costmap & m)
+{
+  const mppi_costmap & t = h->tmpl_map;
+  return h->tmpl_gen == h->rec_gen && t.size_x == m.size_x && t.size_y == m.size_y && t.resolution == m.resolution &&
+    t.origin_x == m.origin_x && t.origin_y == m.origin_y;
+}
+
+// member k of the noise table rejected on the device (record_batch_kernel): its redraws drew nothing, but its epoch
+// advanced with the others'.  Put its table entry back and the epoch to the host mirror, which did not advance.
+mppi_status restore_noise_entry(mppi_handle * L, mppi_handle * h, int k)
+{
+  CUDA_TRY(L, cudaMemcpyAsync(L->d_noise_jobs + k, &L->noise_jobs_h[k], sizeof(NoiseJob), cudaMemcpyHostToDevice, L->stream));
+  return sync_epoch(h);
+}
+
+mppi_status group_device_run(mppi_handle ** hs, int n, const mppi_group_inputs * in, const mppi_costmap * maps, mppi_cycle_out * outs)
+{
+  mppi_handle * L = hs[0];
+  CUDA_TRY(L, cudaSetDevice(L->device));
+  for (int i = 0; i < n; ++i) {
+    if (!hs[i]->costmap_device) {
+      return fail(L, MPPI_E_CONFIG, "mppi_optimize_group_device: member " + std::to_string(i) +
+        " is in host-costmap mode (MPPI_COSTMAP_DEVICE expected)");
+    }
+  }
+  if (!batch_stream_ok(hs, n)) {return MPPI_E_CONFIG;}   // L->err names the member
+  if (in->path_stride < 1) {return fail(L, MPPI_E_CONFIG, "mppi_optimize_group_device: path_stride must be >= 1");}
+  const size_t rows = static_cast<size_t>(n);
+  const struct {const void * p; size_t bytes; const char * what;} arrays[] = {
+    {in->state, rows * 8 * sizeof(double), "group inputs: state"},
+    {in->goal_checker_xy_tolerance, rows * sizeof(double), "group inputs: goal_checker_xy_tolerance"},
+    {in->path_size, rows * sizeof(int32_t), "group inputs: path_size"},
+    {in->path, rows * 3 * static_cast<size_t>(in->path_stride) * sizeof(float), "group inputs: path"}};
+  for (const auto & a : arrays) {
+    const mppi_status s = check_device_range(L, a.p, a.bytes, a.what);
+    if (s != MPPI_OK) {return s;}
+  }
+  for (int i = 0; i < n; ++i) {
+    mppi_handle * h = hs[i];
+    mppi_status s = check_device_costmap(h, maps[i]);
+    if (s == MPPI_OK && (maps[i].size_x >= (1u << 22) || maps[i].size_y >= (1u << 22))) {
+      s = fail(h, MPPI_E_CONFIG, "costmap side must be < 2^22 cells");
+    }
+    if (s == MPPI_OK && !template_current(h, maps[i])) {s = build_template(L, h, i, maps[i]);}
+    if (s != MPPI_OK) {return fail(L, s, "mppi_optimize_group_device: member " + std::to_string(i) + ": " + h->err);}
+  }
+  int kn = 0;
+  for (int i = 0; i < n; ++i) {
+    hs[i]->last.cm_dev = maps[i].cells;   // the job's map and the path tables' launch (batch_stream_launch)
+    kn += hs[i]->cfg.regenerate_noises ? 1 : 0;
+  }
+  const uint32_t tag = 0x80000000u | (++L->batch_tag);
+  mppi_status first = batch_stream_launch(L, hs, 0, n, 0, kn, false, tag, true, true, in);
+  if (first != MPPI_OK) {
+    for (int i = 0; i < n; ++i) {hs[i]->record_from_device = false; hs[i]->cycle_uploaded = false;}
+    return first;
+  }
+  {
+    const mppi_status s = batch_redraw(L, 0, kn);   // the set for the next step, as batch_run_group draws it
+    if (s != MPPI_OK) {first = s;}
+  }
+  std::vector<char> bad(n, 0);
+  for (int i = 0; i < n; ++i) {
+    mppi_handle * h = hs[i];
+    uint32_t status = 0;
+    mppi_status s = wait_packets(h, h->h_res + 3 * static_cast<size_t>(h->T) + 8, 1, tag, &status);
+    if (s == MPPI_OK && (status & kRecordBadPath)) {
+      bad[i] = 1;
+      h->record_from_device = false;
+      h->cycle_uploaded = false;
+      std::memset(L->jobs_sent.data() + sizeof(FusedJob) * static_cast<size_t>(i), 0, sizeof(FusedJob));   // the kernel zeroed its extents
+      s = fail(h, MPPI_E_CONFIG, "mppi_optimize_group_device: member " + std::to_string(i) +
+        ": path_size outside [1, min(MPPI_MAX_PATH_POINTS, path_stride)]");
+      if (first == MPPI_OK) {fail(L, s, h->err);}
+    } else if (s == MPPI_OK) {
+      h->angle_band_hits += status;
+      s = finish_optimize(h, outs ? &outs[i] : nullptr);
+      h->cycle_uploaded = s == MPPI_OK;
+    }
+    if (s != MPPI_OK && first == MPPI_OK) {first = s;}
+  }
+  for (int i = 0, k = 0; i < n; ++i) {
+    if (!hs[i]->cfg.regenerate_noises) {continue;}
+    if (bad[i]) {
+      const mppi_status s = restore_noise_entry(L, hs[i], k);
+      if (s != MPPI_OK && first == MPPI_OK) {first = s;}
+    }
+    ++k;
   }
   return first;
 }
@@ -2100,6 +2267,7 @@ mppi_status mppi_set_critics(mppi_handle * h, const mppi_critic_desc * critics, 
   }
   h->critics.assign(critics, critics + n);
   h->cycle_uploaded = false;
+  h->rec_gen++;
   return MPPI_OK;
 }
 
@@ -2109,6 +2277,7 @@ mppi_status mppi_set_robot(mppi_handle * h, const mppi_robot_desc * robot)
   if (robot->footprint_size < 0 || robot->footprint_size > MPPI_MAX_FOOTPRINT) {return fail(h, MPPI_E_CONFIG, "footprint_size out of range");}
   h->robot = *robot;
   h->cycle_uploaded = false;
+  h->rec_gen++;
   return MPPI_OK;
 }
 
@@ -2124,6 +2293,7 @@ mppi_status mppi_set_speed_limit(mppi_handle * h, double speed_limit, int32_t pe
     s.vx_max = b.vx_max * ratio; s.vx_min = b.vx_min * ratio; s.vy = b.vy * ratio; s.wz = b.wz * ratio;
   }
   h->cycle_uploaded = false;
+  h->rec_gen++;
   return MPPI_OK;
 }
 
@@ -2236,6 +2406,7 @@ mppi_status mppi_set_outputs(mppi_handle * h, uint32_t want_mask)
   if (!h) {return MPPI_E_CONFIG;}
   h->want_mask = want_mask;
   h->cycle_uploaded = false;
+  h->rec_gen++;
   return MPPI_OK;
 }
 
@@ -2251,6 +2422,7 @@ mppi_status mppi_set_costmap_residency(mppi_handle * h, int32_t residency)
   h->costmap_device = residency == MPPI_COSTMAP_DEVICE;
   h->cm_checked = nullptr; h->cm_checked_bytes = 0;
   h->cycle_uploaded = false;
+  h->rec_gen++;
   return MPPI_OK;
 }
 
@@ -2366,6 +2538,8 @@ mppi_status mppi_batch_bind(mppi_handle ** hs, int32_t n)
   L->arena_slice = (kParamsCapacity + 256 + cap + 255) & ~static_cast<size_t>(255);
   CUDA_TRY(L, cudaHostAlloc(&L->arena_h, L->arena_slice * n, cudaHostAllocMapped | cudaHostAllocPortable));
   CUDA_TRY(L, cudaMalloc(&L->arena_d, L->arena_slice * n));
+  CUDA_TRY(L, cudaHostAlloc(&L->tmpl_h, static_cast<size_t>(kTemplateStride) * n, cudaHostAllocDefault));
+  CUDA_TRY(L, cudaMalloc(&L->tmpl_d, static_cast<size_t>(kTemplateStride) * n));
   CUDA_TRY(L, cudaStreamCreateWithFlags(&L->copy_stream, cudaStreamNonBlocking));
   for (auto & e : L->ev_upload) {CUDA_TRY(L, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));}
   for (int i = 0; i < n; ++i) {
@@ -2381,6 +2555,7 @@ mppi_status mppi_batch_bind(mppi_handle ** hs, int32_t n)
     h->costmap_capacity = L->arena_slice - kParamsCapacity - 256;
     h->params_in_arena = true;
     h->cycle_uploaded = false;
+    h->tmpl_gen = 0;
     std::memset(h->h_res, 0, (3 * static_cast<size_t>(h->T) + 10) * sizeof(uint2));
     h->batch_leader = L;
     if (h != L) {h->own_stream = h->stream; h->stream = L->stream;}
@@ -2400,12 +2575,19 @@ mppi_status mppi_batch_bind(mppi_handle ** hs, int32_t n)
     noise_jobs.push_back(j);
     L->noise_items.push_back(static_cast<long long>(h->B) * ((h->T + 3) / 4));
   }
+  std::vector<int> noise_index(n, -1);
+  for (int i = 0, k = 0; i < n; ++i) {
+    if (hs[i]->cfg.regenerate_noises) {noise_index[i] = k++;}
+  }
+  CUDA_TRY(L, cudaMalloc(&L->d_noise_index, sizeof(int) * static_cast<size_t>(n)));
+  CUDA_TRY(L, cudaMemcpyAsync(L->d_noise_index, noise_index.data(), sizeof(int) * static_cast<size_t>(n), cudaMemcpyHostToDevice, L->stream));
   if (!noise_jobs.empty()) {
     const size_t bytes = sizeof(NoiseJob) * noise_jobs.size();
     CUDA_TRY(L, cudaMalloc(&L->d_noise_jobs, bytes));
     CUDA_TRY(L, cudaMemcpyAsync(L->d_noise_jobs, noise_jobs.data(), bytes, cudaMemcpyHostToDevice, L->stream));
-    CUDA_TRY(L, cudaStreamSynchronize(L->stream));
   }
+  CUDA_TRY(L, cudaStreamSynchronize(L->stream));
+  L->noise_jobs_h = noise_jobs;
   return MPPI_OK;
 }
 
@@ -2490,6 +2672,34 @@ mppi_status mppi_batch_span_ms(mppi_handle ** hs, int32_t n, float * ms_out)
   return MPPI_OK;
 }
 
+mppi_status mppi_optimize_group_device(mppi_handle ** hs, int32_t n, const mppi_group_inputs * in, const mppi_costmap * maps,
+  mppi_cycle_out * outs)
+{
+  if (!hs || n < 1 || !hs[0] || !in || !maps) {return MPPI_E_CONFIG;}
+  if (!batch_is_group(hs, n)) {
+    return fail(hs[0], MPPI_E_CONFIG, "mppi_optimize_group_device: hs must be exactly a bound group, in bind order");
+  }
+  return group_device_run(hs, n, in, maps, outs);
+}
+
+mppi_status mppi_debug_get_record(mppi_handle * h, void * out, uint64_t capacity, uint64_t * record_bytes, uint64_t * angle_band_hits)
+{
+  if (!h || (capacity > 0 && !out)) {return MPPI_E_CONFIG;}
+  CUDA_TRY(h, cudaSetDevice(h->device));
+  CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+  DevParams p;
+  CUDA_TRY(h, cudaMemcpy(&p, h->d_params, sizeof(p), cudaMemcpyDeviceToHost));
+  size_t bytes = sizeof(DevParams);
+  if (p.N >= 1 && p.N <= MPPI_MAX_PATH_POINTS) {
+    const size_t N = p.N, n16 = ((N + 15) / 16) * 16;
+    bytes += sizeof(float) * 4 * N + 2 * n16 + sizeof(uint16_t) * N;
+  }
+  if (capacity > 0) {CUDA_TRY(h, cudaMemcpy(out, h->d_params, std::min<size_t>(capacity, kParamsCapacity), cudaMemcpyDeviceToHost));}
+  if (record_bytes) {*record_bytes = bytes;}
+  if (angle_band_hits) {*angle_band_hits = h->angle_band_hits;}
+  return MPPI_OK;
+}
+
 mppi_status mppi_get_trajectories(mppi_handle * h, float * x, float * y, float * yaw)
 {
   if (!h || !x || !y || !yaw) {return MPPI_E_CONFIG;}
@@ -2510,6 +2720,7 @@ mppi_status mppi_set_visualization(mppi_handle * h, int32_t trajectory_step, int
   CUDA_TRY(h, cudaStreamSynchronize(h->stream));
   drop_graphs(h);
   h->vis_b_step = trajectory_step; h->vis_t_step = time_step; h->vis_valid = false;
+  h->rec_gen++;
   if (trajectory_step > 0) {
     const size_t nb = (h->B + trajectory_step - 1) / trajectory_step, nt = (h->T + time_step - 1) / time_step;
     if (2 * nb * nt > h->vis_capacity) {

@@ -17,6 +17,8 @@
 #include <stddef.h>
 #include <stdint.h>
 
+#include <cmath>
+
 #include "../../include/mppi_b200.h"
 #include "../../include/mppi_det_math.h"
 
@@ -167,6 +169,51 @@ __host__ __device__ inline int path_follow_index(int f, int offset, int N, const
   return fidx > 0 ? fidx : 0;
 }
 constexpr int kHotFloats = kHotBytes / 4;
+
+// ---- the per-cycle goal gates, one definition for build_params (host inputs) and record_batch_kernel (device inputs).
+//      IEEE mul / add only, never contracted (the host pass is built with -ffp-contract=off), so both sides decide alike.
+#if defined(__CUDA_ARCH__)
+#define MPPI_DADD(a, b) __dadd_rn((a), (b))
+#else
+#define MPPI_DADD(a, b) ((a) + (b))
+#endif
+// utils::withinPositionGoalTolerance(float, ...) utils.hpp:233-249 (std::pow(d, 2) is d * d, exactly)
+__host__ __device__ inline bool within_tolerance(float pose_tolerance, double rx, double ry, double gx, double gy)
+{
+  const double dx = gx - rx, dy = gy - ry;
+  const double dist_sq = MPPI_DADD(MPPI_DMUL(dx, dx), MPPI_DMUL(dy, dy));
+  const float pose_tolerance_sq = MPPI_FMUL(pose_tolerance, pose_tolerance);
+  return dist_sq < pose_tolerance_sq;
+}
+// utils::withinPositionGoalTolerance(GoalChecker*, ...) utils.hpp:201-224
+__host__ __device__ inline bool within_checker_tolerance(double tol, double rx, double ry, double gx, double gy)
+{
+  if (tol >= 0.0) {
+    const double dx = rx - gx, dy = ry - gy;
+    if (MPPI_DADD(MPPI_DMUL(dx, dx), MPPI_DMUL(dy, dy)) < MPPI_DMUL(tol, tol)) {return true;}
+  }
+  return false;
+}
+// PathAngle's gate for the path point (gx, gy) with forward_preference (path_angle_critic.cpp:79-83): the angle A in
+// [0, pi] between the heading (cos ch, sin sh) and the direction to the point is below max (cos max = ct) iff
+// cos A > ct.  Decided from a dot product wherever that is further than 1e-5 from the threshold (atan2f, the float roundings
+// of the reference and the rounding of A to float move cos A by < 1e-6): 1 open, 0 closed, -1 undecided (the caller
+// evaluates posePointAngle itself).
+__host__ __device__ inline int path_angle_fast_gate(float gx, float gy, float pose_xf, float pose_yf, double ch, double sh, double ct)
+{
+  const double dxj = static_cast<double>(MPPI_FSUB(gx, pose_xf)), dyj = static_cast<double>(MPPI_FSUB(gy, pose_yf));
+  const double dd = MPPI_DADD(MPPI_DMUL(dxj, dxj), MPPI_DMUL(dyj, dyj));
+  if (dd > 1.0e-12) {
+#if defined(__CUDA_ARCH__)
+    const double c = __ddiv_rn(MPPI_DADD(MPPI_DMUL(dxj, ch), MPPI_DMUL(dyj, sh)), __dsqrt_rn(dd));
+#else
+    const double c = (dxj * ch + dyj * sh) / std::sqrt(dd);
+#endif
+    if (c < ct - 1.0e-5) {return 1;}
+    if (c > ct + 1.0e-5) {return 0;}
+  }
+  return -1;
+}
 
 // cooperative copy of the hot part of the record into shared memory (16-byte vectors, coalesced)
 __device__ __forceinline__ void load_hot_params(float * s_hot, const DevParams * __restrict__ P, int tid, int nthreads)

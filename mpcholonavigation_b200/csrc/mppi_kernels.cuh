@@ -3574,4 +3574,223 @@ __global__ void __launch_bounds__(kTablesThreads) path_tables_batch_kernel(const
   path_tables_body(const_cast<DevParams *>(jobs[blockIdx.y].Pg));
 }
 
+// ---------------------------------------------------------------------------------------------------
+// Cycle records of a robot group built on the device from inputs in device memory (mppi_optimize_group_device).
+// The host builds each member's TEMPLATE once per configuration change: a record made by build_params itself (constraints,
+// gamma terms, critic table, footprint, ObstaclesCritic LUTs, map geometry and circumscribed cost) followed by the
+// thresholds below.  Per cycle, record_batch_kernel copies the template into the member's slice of the group arena and
+// completes everything build_params derives from the cycle inputs, with build_params' arithmetic: the pose and speed
+// fields, the path tail (x, y, yaw, the arc-length prefix D as a sequential fp32 sum), closest_path_pt, the path spacing
+// bounds, the goal gates (within_tolerance & co, mppi_device.cuh), PathAngle's gate per index and the fields derived from
+// the gates.  path_tables_batch_kernel runs right behind it and makes the costmap-dependent tables.
+// ---------------------------------------------------------------------------------------------------
+struct RecordGates
+{
+  double angle_cos_max;                      // cos(max_angle_to_furthest), host libm (PathAngle's fast test)
+  float goal_thr, goal_angle_thr, forward_thr, follow_thr, align_thr, legacy_thr, angle_thr;   // threshold_to_consider
+  float cost_near, obst_near;                // near_goal_distance of CostCritic / ObstaclesCritic
+  float angle_max;                           // max_angle_to_furthest
+  int goal_en, goal_angle_en, forward_en, twirl_en, follow_en, align_en, legacy_en, angle_en;   // in the list and enabled
+  int has_cost, has_obst;                    // in the list
+  int angle_fast;                            // the fast test applies (forward_preference, 1e-3 < max < 3.1)
+  int want_traj;                             // MPPI_WANT_TRAJECTORIES
+};
+constexpr int kTemplateStride = ((static_cast<int>(sizeof(DevParams) + sizeof(RecordGates)) + 15) / 16) * 16;
+static_assert(sizeof(DevParams) % 8 == 0, "the template is copied in 8-byte words");
+
+constexpr int kRecordThreads = 256;
+// value of a member's status packet (host_res[3T + 8]): the PathAngle band hits of the cycle, or this bit for a path_size
+// outside [1, min(MPPI_MAX_PATH_POINTS, path_stride)] (the member's launches are then cancelled, nothing of it changes)
+constexpr unsigned kRecordBadPath = 0x80000000u;
+
+// posePointAngle (utils.hpp:417-434) with the device's atan2f: used only inside PathAngle's undecided band
+__device__ __noinline__ float pose_point_angle_dev(float pose_xf, float pose_yf, float pose_yawf, float gx, float gy, bool forward_preference)
+{
+  const float yaw = atan2f(__fsub_rn(gy, pose_yf), __fsub_rn(gx, pose_xf));
+  const double a = fabs(normalize_angle_d(__dsub_rn(static_cast<double>(pose_yawf), static_cast<double>(yaw))));
+  if (forward_preference) {return static_cast<float>(a);}
+  const double back = normalize_angle_d(__dadd_rn(static_cast<double>(pose_yawf), 3.14159265358979323846));
+  return static_cast<float>(fmin(a, fabs(normalize_angle_d(__dsub_rn(back, static_cast<double>(yaw))))));
+}
+
+// noise_jobs / noise_index: the group's regenerate_noises table and each member's entry in it (-1: none)
+__global__ void __launch_bounds__(kRecordThreads) record_batch_kernel(FusedJob * __restrict__ jobs, const char * __restrict__ templates,
+  mppi_group_inputs in, int row0, unsigned tag, NoiseJob * __restrict__ noise_jobs, const int * __restrict__ noise_index)
+{
+  __shared__ float s_seg[MPPI_MAX_PATH_POINTS];          // fp32 length of segment i - 1 -> i (D)
+  __shared__ double s_segd[MPPI_MAX_PATH_POINTS];        // fp64 length of segment j -> j + 1 (path spacing)
+  __shared__ uint8_t s_gate[MPPI_MAX_PATH_POINTS];       // PathAngle gate per candidate target index
+  __shared__ unsigned long long s_closest, s_hmax;
+  __shared__ unsigned s_band, s_open;
+  __shared__ double s_len;
+  FusedJob & job = jobs[blockIdx.y];
+  DevParams * P = const_cast<DevParams *>(job.Pg);
+  const int row = row0 + static_cast<int>(blockIdx.y), tid = threadIdx.x;
+  const DevParams * tp = reinterpret_cast<const DevParams *>(templates + static_cast<size_t>(row) * kTemplateStride);
+  const RecordGates & g = *reinterpret_cast<const RecordGates *>(tp + 1);
+  const int N = in.path_size[row];
+  if (N < 1 || N > MPPI_MAX_PATH_POINTS || N > in.path_stride) {
+    if (tid == 0) {
+      // cancel the member's launches (their blocks return at once) and its noise redraws (no items; the host restores the
+      // entry and the epoch), keep the path tables away from its stale record
+      job.rollout_blocks = 0; job.cost_blocks = 0; job.ws_chunks = 0; job.merge_blocks = 0;
+      if (noise_index[row] >= 0) {noise_jobs[noise_index[row]].B = 0;}
+      P->cm_dev = nullptr;
+      st_packet(job.host_res + 3 * tp->T + 8, kRecordBadPath, tag);
+    }
+    return;
+  }
+  {
+    const unsigned long long * src = reinterpret_cast<const unsigned long long *>(tp);
+    unsigned long long * dst = reinterpret_cast<unsigned long long *>(P);
+    for (int i = tid; i < static_cast<int>(sizeof(DevParams) / 8); i += kRecordThreads) {dst[i] = src[i];}
+  }
+  if (tid == 0) {s_closest = (static_cast<unsigned long long>(__float_as_uint(3.402823466e+38f)) << 32); s_hmax = 0ull; s_band = 0u; s_open = 0u;}
+  const double * st = in.state + 8 * static_cast<size_t>(row);
+  const double rx = st[0], ry = st[1], ryaw = st[2], gx = st[6], gy = st[7];
+  const float * px = in.path + static_cast<size_t>(row) * 3 * in.path_stride;
+  const float * py = px + in.path_stride, * pyaw = py + in.path_stride;
+  const float yaw0 = static_cast<float>(ryaw);
+  float sin0, cos0;
+  mppi_det_sincosf(yaw0, &sin0, &cos0);
+  const float svx = static_cast<float>(st[3]), svy = static_cast<float>(st[4]);
+  // trajectory 0's first pose (build_params: the rollout's own arithmetic)
+  float x00, y00;
+  {
+    const bool hol = tp->holonomic != 0;
+    const float vx0 = svx, vy0 = hol ? svy : 0.0f;
+    float dx = __fmul_rn(vx0, cos0), dy = __fmul_rn(vx0, sin0);
+    if (hol) {dx = __fsub_rn(dx, __fmul_rn(vy0, sin0)); dy = __fadd_rn(dy, __fmul_rn(vy0, cos0));}
+    x00 = static_cast<float>(__dadd_rn(rx, static_cast<double>(__fmul_rn(dx, tp->dt))));
+    y00 = static_cast<float>(__dadd_rn(ry, static_cast<double>(__fmul_rn(dy, tp->dt))));
+  }
+  const bool angle_on = g.angle_en && !within_tolerance(g.angle_thr, rx, ry, gx, gy);
+  const float pose_xf = static_cast<float>(rx), pose_yf = static_cast<float>(ry);
+  double sh = 0.0, ch = 1.0;
+  if (angle_on && g.angle_fast) {sincos(static_cast<double>(yaw0), &sh, &ch);}
+  const int n16 = ((N + 15) / 16) * 16;
+  float * tail = reinterpret_cast<float *>(P + 1);
+  uint8_t * valid = reinterpret_cast<uint8_t *>(tail + 4 * N);
+  uint8_t * flags = valid + n16;
+  __syncthreads();   // the template is in place, the shared accumulators are set
+  for (int i = tid; i < 2 * n16 + 2 * N; i += kRecordThreads) {valid[i] = 0;}
+  const int open_from = max(0, min(tp->angle_offset, N - 1));
+  unsigned long long best = ~0ull, hmax = 0ull;
+  unsigned band = 0u, open_any = 0u;
+  for (int j = tid; j < N; j += kRecordThreads) {
+    const float xj = px[j], yj = py[j];
+    tail[j] = xj; tail[N + j] = yj; tail[2 * N + j] = pyaw[j];
+    if (j > 0) {
+      const float dx = __fsub_rn(xj, px[j - 1]), dy = __fsub_rn(yj, py[j - 1]);
+      s_seg[j] = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
+    }
+    if (j + 1 < N) {
+      const double sx = __dsub_rn(static_cast<double>(px[j + 1]), static_cast<double>(xj));
+      const double sy = __dsub_rn(static_cast<double>(py[j + 1]), static_cast<double>(yj));
+      const double seg = __dsqrt_rn(__dadd_rn(__dmul_rn(sx, sx), __dmul_rn(sy, sy)));
+      s_segd[j] = seg;
+      if (seg >= 0.0) {hmax = max(hmax, static_cast<unsigned long long>(__double_as_longlong(seg)));}   // NaN is skipped, as std::max does
+    }
+    {
+      const float dx = __fsub_rn(xj, x00), dy = __fsub_rn(yj, y00);
+      const float d = __fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy));
+      if (d < 3.402823466e+38f) {best = min(best, (static_cast<unsigned long long>(__float_as_uint(d)) << 32) | static_cast<unsigned>(j));}
+    }
+    bool open = false;
+    if (angle_on) {
+      int decided = g.angle_fast ? path_angle_fast_gate(xj, yj, pose_xf, pose_yf, ch, sh, g.angle_cos_max) : -1;
+      if (decided < 0) {
+        // the point under the robot is no band decision: atan2f(+0, +0) = +0 on either side
+        band += (__fsub_rn(xj, pose_xf) != 0.0f || __fsub_rn(yj, pose_yf) != 0.0f) ? 1u : 0u;
+        decided = pose_point_angle_dev(pose_xf, pose_yf, yaw0, xj, yj, tp->angle_forward_pref != 0) < g.angle_max ? 0 : 1;
+      }
+      open = decided == 1;
+    }
+    s_gate[j] = open ? 1 : 0;
+    if (open && j >= open_from) {open_any = 1u;}
+  }
+  if (best != ~0ull) {atomicMin(&s_closest, best);}
+  if (hmax != 0ull) {atomicMax(&s_hmax, hmax);}
+  if (band) {atomicAdd(&s_band, band);}
+  if (open_any) {s_open = 1u;}
+  __syncthreads();
+  if (tid == 0) {
+    // arc-length prefix (path_align_critic.cpp:83-90): a sequential fp32 sum in index order, as build_params makes it
+    float * D = tail + 3 * N;
+    float acc = 0.0f;
+    D[0] = 0.0f;
+    for (int i = 1; i < N; ++i) {acc = __fadd_rn(acc, s_seg[i]); D[i] = acc;}
+  } else if (tid == 32) {
+    double len = 0.0;
+    for (int j = 0; j + 1 < N; ++j) {len = __dadd_rn(len, s_segd[j]);}
+    s_len = len;
+  }
+  for (int f = tid; f < N; f += kRecordThreads) {
+    if (s_gate[min(f + tp->angle_offset, N - 1)]) {flags[f] = 4u;}
+  }
+  __syncthreads();
+  if (tid != 0) {return;}
+  DevParams & p = *P;
+  p.pose_x = rx; p.pose_y = ry;
+  p.yaw0 = yaw0; p.sin0 = sin0; p.cos0 = cos0;
+  p.speed_vx = svx; p.speed_vy = svy; p.speed_wz = static_cast<float>(st[5]);
+  p.goal_x = gx; p.goal_y = gy;
+  p.N = N;
+  p.goal_yaw = pyaw[N - 1];
+  p.off_path_x = 0; p.off_path_y = N; p.off_path_yaw = 2 * N; p.off_path_D = 3 * N;
+  p.cm_dev = job.cm;
+  p.closest_path_pt = s_closest == (static_cast<unsigned long long>(__float_as_uint(3.402823466e+38f)) << 32) ? 0 :
+    static_cast<int>(s_closest & 0xFFFFFFFFull);
+  {
+    const double hm = __longlong_as_double(static_cast<long long>(s_hmax)), len = s_len;
+    p.path_hmax_inv = (hm > 0.0 && isfinite(hm)) ? static_cast<float>(__ddiv_rn(1.0, __dmul_rn(hm, 1.00001))) : 0.0f;
+    p.path_hmean_inv = (len > 0.0 && isfinite(len)) ? static_cast<float>(__ddiv_rn(static_cast<double>(N - 1), len)) : 0.0f;
+  }
+  // the gates (build_params, in its order)
+  if (g.has_cost) {p.cost_near_goal = within_tolerance(g.cost_near, rx, ry, gx, gy) ? 1 : 0;}
+  if (g.has_obst) {p.obst_near_goal = within_tolerance(g.obst_near, rx, ry, gx, gy) ? 1 : 0;}
+  p.goal.on = g.goal_en && within_tolerance(g.goal_thr, rx, ry, gx, gy);
+  p.goal_angle.on = g.goal_angle_en && within_tolerance(g.goal_angle_thr, rx, ry, gx, gy);
+  p.forward.on = g.forward_en && !within_tolerance(g.forward_thr, rx, ry, gx, gy);
+  p.twirl.on = g.twirl_en && !within_checker_tolerance(in.goal_checker_xy_tolerance[row], rx, ry, gx, gy);
+  p.follow.on = g.follow_en && N >= 2 && !within_tolerance(g.follow_thr, rx, ry, gx, gy);
+  p.align.on = g.align_en && !within_tolerance(g.align_thr, rx, ry, gx, gy);
+  p.legacy.on = g.legacy_en && !within_tolerance(g.legacy_thr, rx, ry, gx, gy);
+  p.angle.on = angle_on;
+  if (p.align.on || p.legacy.on) {
+    p.sample_step = p.align.on ? p.align_step : p.legacy_step;
+    p.n_samples = (p.T + p.sample_step - 1) / p.sample_step;
+    p.sample_yaw = (p.align.on && p.align_use_yaw) || (p.legacy.on && p.legacy_use_yaw);
+  } else {
+    p.sample_step = 0; p.n_samples = 0; p.sample_yaw = 0;
+  }
+  p.obstacle_q[0] = p.obstacle_q[1] = -1;
+  p.first_path_q = -1;
+  int nob = 0;
+  for (int q = 0; q < p.n_critics; ++q) {
+    const int kind = p.kind_of[q];
+    const bool obstacle_like = (kind == MPPI_CRITIC_COST && p.cost.on) || (kind == MPPI_CRITIC_OBSTACLES && p.obst.on);
+    if (obstacle_like && nob < 2) {p.obstacle_q[nob++] = q;}
+    const bool path_like = (kind == MPPI_CRITIC_PATH_FOLLOW && p.follow.on) || (kind == MPPI_CRITIC_PATH_ANGLE && p.angle.on) ||
+      (kind == MPPI_CRITIC_PATH_ALIGN && p.align.on) || (kind == MPPI_CRITIC_PATH_ALIGN_LEGACY && p.legacy.on);
+    if (path_like && p.first_path_q < 0) {p.first_path_q = q;}
+    int on = 0;
+    switch (kind) {
+      case MPPI_CRITIC_PATH_FOLLOW: on = p.follow.on ? 2 : 0; break;
+      case MPPI_CRITIC_PATH_ALIGN: on = p.align.on ? 3 : 0; break;
+      case MPPI_CRITIC_PATH_ALIGN_LEGACY: on = p.legacy.on ? 4 : 0; break;
+      case MPPI_CRITIC_PATH_ANGLE: on = p.angle.on ? 5 : 0; break;
+      case MPPI_CRITIC_GOAL: on = p.goal.on; break;
+      case MPPI_CRITIC_GOAL_ANGLE: on = p.goal_angle.on; break;
+      case MPPI_CRITIC_PREFER_FORWARD: on = p.forward.on; break;
+      case MPPI_CRITIC_TWIRLING: on = p.twirl.on; break;
+      default: on = p.src_base[q]; break;   // not gated per cycle: the template's
+    }
+    p.src_base[q] = static_cast<unsigned char>(on);
+  }
+  p.spill_traj = (g.want_traj || s_open) ? 1 : 0;
+  __threadfence_system();
+  st_packet(job.host_res + 3 * p.T + 8, s_band, tag);
+}
+
 }  // namespace mppi

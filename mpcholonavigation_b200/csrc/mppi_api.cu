@@ -1514,7 +1514,7 @@ mppi_status fetch_time_major(mppi_handle * h, const V * d_src, V * host_dst)
 {
   mppi_status s = ensure_tmp(h);
   if (s != MPPI_OK) {return s;}
-  const dim3 grid((h->B + 31) / 32, (h->T + 31) / 32), block(32, 8);
+  const dim3 grid = transpose_grid(h->T, h->B), block(32, 8);
   transpose_tb_to_bt_kernel<V><<<grid, block, 0, h->stream>>>(d_src, reinterpret_cast<V *>(h->d_tmp), h->T, h->B);
   CUDA_TRY(h, cudaGetLastError());
   CUDA_TRY(h, cudaMemcpyAsync(host_dst, h->d_tmp, static_cast<size_t>(h->B) * h->T * sizeof(V), cudaMemcpyDeviceToHost, h->stream));
@@ -1635,7 +1635,7 @@ mppi_status to_stream_layout(mppi_handle * h)
   mppi_status s = ensure_tmp(h);
   if (s != MPPI_OK) {return s;}
   const size_t plane = static_cast<size_t>(h->B) * h->T * sizeof(float);
-  const dim3 grid((h->T + 31) / 32, (h->B + 31) / 32), block(32, 8);
+  const dim3 grid = transpose_grid(h->B, h->T), block(32, 8);
   for (int i = 0; i < 3; ++i) {
     CUDA_TRY(h, cudaMemcpyAsync(h->d_tmp, h->d_noise[i], plane, cudaMemcpyDeviceToDevice, h->stream));
     transpose_tb_to_bt_kernel<float><<<grid, block, 0, h->stream>>>(h->d_tmp, h->d_noise[i], h->B, h->T);
@@ -2324,7 +2324,7 @@ mppi_status mppi_set_noise(mppi_handle * h, const float * vx, const float * vy, 
     } else {
       // caller's layout is [B][T]; the stream layout keeps [T][B]
       CUDA_TRY(h, cudaMemcpyAsync(h->d_tmp, src[i], plane, cudaMemcpyHostToDevice, h->stream));
-      const dim3 grid((h->T + 31) / 32, (h->B + 31) / 32), block(32, 8);
+      const dim3 grid = transpose_grid(h->B, h->T), block(32, 8);
       transpose_tb_to_bt_kernel<float><<<grid, block, 0, h->stream>>>(h->d_tmp, h->d_noise[i], h->B, h->T);
       CUDA_TRY(h, cudaGetLastError());
     }
@@ -2742,7 +2742,7 @@ mppi_status mppi_get_visualization(mppi_handle * h, float * x, float * y)
   const int nb = (h->B + h->vis_b_step - 1) / h->vis_b_step, nt = (h->T + h->vis_t_step - 1) / h->vis_t_step;
   mppi_status s = ensure_tmp(h);
   if (s != MPPI_OK) {return s;}
-  const dim3 grid((nb + 31) / 32, (nt + 31) / 32), block(32, 8);
+  const dim3 grid = transpose_grid(nt, nb), block(32, 8);
   float * dst[2] = {x, y};
   for (int k = 0; k < 2; ++k) {
     transpose_tb_to_bt_kernel<float><<<grid, block, 0, h->stream>>>(h->d_vis + static_cast<size_t>(k) * nt * nb, h->d_tmp, nt, nb);

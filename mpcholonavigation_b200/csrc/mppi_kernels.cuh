@@ -3361,21 +3361,33 @@ __global__ void __launch_bounds__(kUpdThreads) merge_exchange_finalize_kernel(
 // ---------------------------------------------------------------------------------------------------
 // small utility kernels
 // ---------------------------------------------------------------------------------------------------
-// time-major [T][B] -> row-major [B][T] (getGeneratedTrajectories / cell indices for the host)
+// time-major [T][B] -> row-major [B][T] (getGeneratedTrajectories / cell indices for the host; with the roles of T
+// and B exchanged, [B][T] -> [T][B] for the noise of the stream layout).  The blocks of y stride over T: grid.y is capped
+// at 65535, and a noise transpose puts the batch size there (transpose_grid).
 template<typename V>
 __global__ void transpose_tb_to_bt_kernel(const V * __restrict__ src, V * __restrict__ dst, int T, int B)
 {
   __shared__ V tile[32][33];
-  const int b0 = blockIdx.x * 32, t0 = blockIdx.y * 32;
-  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-    const int t = t0 + i, b = b0 + threadIdx.x;
-    if (t < T && b < B) {tile[i][threadIdx.x] = src[static_cast<size_t>(t) * B + b];}
+  const int b0 = blockIdx.x * 32;
+  for (int t0 = blockIdx.y * 32; t0 < T; t0 += gridDim.y * 32) {
+    for (int i = threadIdx.y; i < 32; i += blockDim.y) {
+      const int t = t0 + i, b = b0 + threadIdx.x;
+      if (t < T && b < B) {tile[i][threadIdx.x] = src[static_cast<size_t>(t) * B + b];}
+    }
+    __syncthreads();
+    for (int i = threadIdx.y; i < 32; i += blockDim.y) {
+      const int b = b0 + i, t = t0 + threadIdx.x;
+      if (t < T && b < B) {dst[static_cast<size_t>(b) * T + t] = tile[threadIdx.x][i];}
+    }
+    __syncthreads();
   }
-  __syncthreads();
-  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-    const int b = b0 + i, t = t0 + threadIdx.x;
-    if (t < T && b < B) {dst[static_cast<size_t>(b) * T + t] = tile[threadIdx.x][i];}
-  }
+}
+
+// grid of transpose_tb_to_bt_kernel for a [T][B] source: B on x, T on y up to the 65535 blocks y allows
+inline dim3 transpose_grid(int T, int B)
+{
+  const int ty = (T + 31) / 32;
+  return dim3((B + 31) / 32, ty < 65535 ? ty : 65535);
 }
 
 // Optimizer::shiftControlSequence (optimizer.cpp:206-225): roll by -1, last = second to last
